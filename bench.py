@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: clips/sec (10 s, 16 kHz) of logmel + CRNN inference (BASELINE.json `metric`).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]           # B200 arm (this repo's kernels)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # B200 arm (this repo's kernels)
   python bench.py --impl reference [--steps K] [--warmup W]     # reference algorithm on the host CPU
 
 A step = one pass of the whole hot path (waveform -> log-mel -> Cnn9 -> bi-GRU -> frame-attention pooling)
@@ -25,6 +25,7 @@ SR, N_FFT, HOP, FMIN, FMAX = 16000, 512, 160, 25, 7000
 CLIP_SAMPLES = 160000
 CONV_GFLOP_TC = 26.031 - 0.0738  # tensor-core conv layers per clip (SURVEY.md 8d minus conv_block1.conv1)
 METRIC = "clips/sec (10 s, 16 kHz) logmel+CRNN inference"
+DUMP_BYTES = 64 * 10 ** 6  # what --dump-outputs writes at most, .npy headers included
 
 
 def config_index():
@@ -119,6 +120,29 @@ class ClockSampler:
                 "samples": len(sm), "window": "device-resident + end-to-end timed regions"}
 
 
+def dump_outputs(out, directory, seed=0):
+    """Write every tensor of one step's output dict as `directory/<name>.npy` in float32.  When they exceed DUMP_BYTES
+    together, each keeps the same seeded sample of clips (rows of the batch dimension, in ascending order) and the
+    sampled indices are written as `directory/sampled_clips.npy` (float64).  Returns the names written."""
+    import numpy as np
+    import torch
+    out = {k: v.float() for k, v in out.items() if v is not None}
+    n = next(iter(out.values())).shape[0]
+    per_clip = sum(v[0].numel() * 4 for v in out.values()) + 8
+    keep = min(n, (DUMP_BYTES - 4096) // per_clip)  # 4096: room for the .npy headers
+    arrays = {}
+    if keep < n:
+        idx = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        sel = torch.from_numpy(idx)
+        out = {k: v.index_select(0, sel.to(v.device)) for k, v in out.items()}
+        arrays["sampled_clips"] = idx.astype(np.float64)
+    arrays.update({k: v.cpu().numpy() for k, v in out.items()})
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+    return sorted(arrays)
+
+
 def reference_modules_available():
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import ref_import
@@ -198,7 +222,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, args.steps)
+    steps = args.steps
     warmup = max(0, args.warmup)
     batch = args.ref_batch
     cb = cpu_reference_throughput(steps, warmup, batch, args.ref_device, args.ref_autocast, args.ref_channels_last)
@@ -519,7 +543,7 @@ def run_b200(args):
     capi.load()
 
     B = args.batch
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     sd = synth.synthetic_state_dict(MODEL_TYPE, SR)
     pm = engine.PackedModel(sd, MODEL_TYPE, N_FFT, HOP, dev, precision=args.precision)
     wave_host = synth.synthetic_waveform(B, CLIP_SAMPLES, seed=1234, rank=rank).pin_memory()
@@ -551,11 +575,17 @@ def run_b200(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ctx.barrier()
     e0.record()
-    for i in range(steps):
+    for i in range(steps - 1):
         step_device(warmup + i)
-    gather.finish()
+    last = step_device(warmup + steps - 1)  # earlier steps drop their outputs at once, the last one's are kept
+    done = gather.finish()  # push: the last step completes here
+    if done is not None:
+        last = done
     e1.record()
     ctx.barrier()
+    # written after the clock samples close (below); region 2 leaves the gather buffers these may alias untouched
+    dump = last if args.dump_outputs and rank == 0 else None
+    del last, done
     elapsed_ms = e0.elapsed_time(e1)
     launches = capi.launches()
     conv_ms = sum(a.elapsed_time(b) for a, b, _ in pm.conv_events)
@@ -583,6 +613,9 @@ def run_b200(args):
     if rank == 0:
         sampler.mark_end()
         clocks = sampler.stop()
+    if dump is not None:
+        dump_outputs(dump, args.dump_outputs)
+    del dump
 
     # ---------------- the other BASELINE configs: short runs outside the headline regions ----------------
     peaks = load_peaks()
@@ -685,7 +718,14 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the short runs of BASELINE configs 3 / 4 / 5")
     ap.add_argument("--gather", default="push", choices=["push", "peer", "nccl", "none"],
                     help="N > 1: how rank 0 gets every rank's outputs (see class Gatherer)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB: a seeded "
+                         "sample of clips when larger, see dump_outputs); the inputs are the same in every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm (--impl b200)")
     args.ref_autocast = {"bf16": "bfloat16", "fp16": "float16"}.get(args.ref_autocast, args.ref_autocast)
     globals()["MODEL_TYPE"] = args.model_type
     if args.impl == "reference":
