@@ -163,6 +163,45 @@ int sed_window_merge_avg(const float* frames, int n_windows, int frames_per_wind
 int sed_events(const float* frames, int n_clips, int n_frames, int classes, const double* high, const double* low,
                const int* n_smooth, const int* n_salt, int max_events, int* events, int* counts, void* stream);
 
+/* ---- Live streaming: audio that is still arriving, many streams per batch ----------------------------------------
+ * The rolling window of pytorch/predict.py:297-349 run incrementally: each stream (slot) owns a mirrored audio ring,
+ * a merge accumulator ring and per-class event state, all in caller-allocated device memory; the caller keeps the
+ * counters and runs, per push, sed_live_ingest -> the model on the ready windows (sed_frontend_logmel reads them in
+ * place through its clip_offset table) -> sed_live_merge -> sed_live_events.  sed_b200.LiveStreamer is the driver.
+ *
+ * Table of sed_live_merge / sed_live_events: [n_entries, SED_LIVE_TABLE_COLS] i32, one row per stream with work:
+ *   slot, k0 (windows merged before), m (windows in this push, rows row0 .. row0+m-1 of the model output), row0,
+ *   lo (frames returned before), n_final (frames final after this push), out_row (row of frame lo in `out`),
+ *   ev_off / ev_cap (events of class c go to events[ev_off + c*ev_cap ..], at most ev_cap), closing (0 / 1). */
+#define SED_LIVE_TABLE_COLS 10
+#define SED_LIVE_EVENT_STATE_INTS 19 /* ints of event state per (slot, class) */
+
+/* Write chunks into their slots' rings.  Replaces the growing `audio_full` slices of pytorch/predict.py:297-305.
+ *   src: packed chunks (dtype 0 = f32, 1 = int16 PCM); table [n_entries, 4] i64 = (slot, offset in src or -1 for
+ *   zeros, length <= max_len, absolute position of the first sample in the stream); arena [n_slots, 2*ring_samples]
+ *   of src's type: sample p of a slot is stored at p mod ring_samples and at p mod ring_samples + ring_samples. */
+int sed_live_ingest(const void* src, int dtype, const long* table, int n_entries, long max_len, long ring_samples,
+                    void* arena, void* stream);
+
+/* Incremental merge + avg_merge of the windows of one push.  Replaces merge / avg_merge utils/utilities.py:405-446
+ * as driven window by window by pytorch/predict.py:323-349, bit for bit: the first window covering a frame sets it,
+ * later windows add in ascending order, final frames are divided by avg_merge's divisor.
+ *   window_frames [rows, frames_per_window, classes] f32 (model output of the push); acc [n_slots, ring_frames,
+ *   classes] f32; out [rows_out, classes] f32 receives frames lo .. n_final-1 of each entry at out_row;
+ *   max_span >= (k0+m-1)*overlap_interval + frames_per_window - lo of every entry with m > 0 (and n_final - lo). */
+int sed_live_merge(const float* window_frames, const int* table, int n_entries, int max_span, int frames_per_window,
+                   int classes, int overlap_interval, int sample_duration, int ring_frames, float* acc, float* out,
+                   void* stream);
+
+/* Resumable activity_detection utils/vad.py:11-199 on the frames sed_live_merge finalized (`frames` = its `out`):
+ * events are reported as soon as no later frame can change them, close flushes the rest (quirks as sed_events).
+ *   state [n_slots, classes, SED_LIVE_EVENT_STATE_INTS] i32 (reset when lo == 0); high/low/n_smooth/n_salt as
+ *   sed_events (low may be NULL); events i32 pairs (bgn, fin) at the table's ev_off / ev_cap; counts
+ *   [n_entries, classes] i32 (may exceed ev_cap: only ev_cap are stored). */
+int sed_live_events(const float* frames, const int* table, int n_entries, int classes, const double* high,
+                    const double* low, const int* n_smooth, const int* n_salt, void* state, int* events, int* counts,
+                    void* stream);
+
 /* ---- Peer-memory result buffers (multi-GPU gather without a collective on the data path) -------------------------
  * The reference gathers replica outputs on GPU 0 inside torch.nn.DataParallel (pytorch/main_strong.py:541,
  * pytorch/predict.py:239).  Here the destination rank owns ONE buffer for the results of all ranks; every other rank

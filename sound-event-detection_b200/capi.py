@@ -14,6 +14,7 @@ HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "sed_b200.h")
 SED_DTYPE_F16 = 0
 SED_DTYPE_BF16 = 1
 CONV_STORE, CONV_POOL, CONV_FREQMEAN = 0, 1, 2
+LIVE_TABLE_COLS, LIVE_EVENT_STATE_INTS = 10, 19  # SED_LIVE_TABLE_COLS / SED_LIVE_EVENT_STATE_INTS
 ERR_NAMES = {1: "SED_ERR_BAD_SHAPE", 2: "SED_ERR_UNSUPPORTED", 3: "SED_ERR_CUDA", 4: "SED_ERR_NULL",
              5: "SED_ERR_DRIVER"}
 
@@ -30,6 +31,9 @@ SIGNATURES = {
     "sed_frontend_logmel": ([_p, _i, _i, _i, _l, _p, _l, _i, _i, _p, _p, _p, _p, _p, _p, _i, _f, _f, _i, _p, _p, _p, _p], _i),
     "sed_events": ([_p, _i, _i, _i, _p, _p, _p, _p, _i, _p, _p, _p], _i),
     "sed_window_merge_avg": ([_p, _i, _i, _i, _i, _i, _i, _p, _p], _i),
+    "sed_live_ingest": ([_p, _i, _p, _i, _l, _l, _p, _p], _i),
+    "sed_live_merge": ([_p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p], _i),
+    "sed_live_events": ([_p, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p], _i),
     "sed_spectrogram_f32": ([_p, _i, _i, _i, _i, _p, _p, _p, _p], _i),
     "sed_logmel_rows_f32": ([_p, _l, _i, _p, _p, _p, _p, _i, _f, _f, _i, _p, _p], _i),
     "sed_conv_first_f32": ([_p, _i, _i, _i, _p, _p, _p, _p, _i, _p], _i),

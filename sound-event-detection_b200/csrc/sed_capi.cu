@@ -85,6 +85,29 @@ int sed_events(const float* frames, int n_clips, int n_frames, int classes, cons
                             as_stream(stream));
 }
 
+int sed_live_ingest(const void* src, int dtype, const long* table, int n_entries, long max_len, long ring_samples,
+                    void* arena, void* stream) {
+  SED_REQUIRE(src); SED_REQUIRE(table); SED_REQUIRE(arena);
+  return sed::live_ingest_launch(src, dtype, table, n_entries, max_len, ring_samples, arena, as_stream(stream));
+}
+
+int sed_live_merge(const float* window_frames, const int* table, int n_entries, int max_span, int frames_per_window,
+                   int classes, int overlap_interval, int sample_duration, int ring_frames, float* acc, float* out,
+                   void* stream) {
+  SED_REQUIRE(window_frames); SED_REQUIRE(table); SED_REQUIRE(acc); SED_REQUIRE(out);
+  return sed::live_merge_launch(window_frames, table, n_entries, max_span, frames_per_window, classes, overlap_interval,
+                                sample_duration, ring_frames, acc, out, as_stream(stream));
+}
+
+int sed_live_events(const float* frames, const int* table, int n_entries, int classes, const double* high,
+                    const double* low, const int* n_smooth, const int* n_salt, void* state, int* events, int* counts,
+                    void* stream) {
+  SED_REQUIRE(frames); SED_REQUIRE(table); SED_REQUIRE(high); SED_REQUIRE(n_smooth); SED_REQUIRE(n_salt);
+  SED_REQUIRE(state); SED_REQUIRE(events); SED_REQUIRE(counts);
+  return sed::live_events_launch(frames, table, n_entries, classes, high, low, n_smooth, n_salt, state, events, counts,
+                                 as_stream(stream));
+}
+
 int sed_logmel_rows_f32(const float* spec, long rows, int F, const int* mel_lo, const int* mel_len,
                         const int* mel_off, const float* mel_val, int n_mels, float amin, float db_offset,
                         int is_log, float* out, void* stream) {

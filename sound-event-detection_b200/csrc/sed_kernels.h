@@ -59,6 +59,15 @@ int events_launch(const float* frames, int n_clips, int n_frames, int classes, c
                   const int* n_smooth, const int* n_salt, int max_events, int* events, int* counts,
                   cudaStream_t stream);
 
+int live_ingest_launch(const void* src, int dtype, const long* table, int n_entries, long max_len, long ring_samples,
+                       void* arena, cudaStream_t stream);
+int live_merge_launch(const float* win, const int* table, int n_entries, int max_span, int frames_per_window,
+                      int classes, int overlap_interval, int sample_duration, int ring_frames, float* acc, float* out,
+                      cudaStream_t stream);
+int live_events_launch(const float* frames, const int* table, int n_entries, int classes, const double* high,
+                       const double* low, const int* n_smooth, const int* n_salt, void* state, int* events, int* counts,
+                       cudaStream_t stream);
+
 int mha_core_launch(const float* qkv, int B, int T, long rs_t, long rs_b, void* out16, int dtype, cudaStream_t stream);
 
 int mha_tc_launch(const void* qkv16, const void* qk_lo16, int B, int T, long Bp, void* ctx16, int dtype,

@@ -289,6 +289,23 @@ def logmel_rows_forward(plan, spec):
     return out
 
 
+def event_params(high, low, n_smooth, n_salt, classes, device):
+    """Per-class thresholds (sequences or scalars) -> the device arrays of sed_events / sed_live_events:
+    high / low float64 (low may be None), n_smooth / n_salt int32."""
+    def per_class(v, dtype):
+        if v is None:
+            return None
+        t = torch.as_tensor(np.asarray(v, dtype=np.float64 if dtype == torch.float64 else np.int64))
+        if t.dim() == 0:
+            t = t.repeat(classes)
+        if t.numel() != classes:
+            raise ValueError("expected %d per-class values, got %d" % (classes, t.numel()))
+        return t.to(dtype).contiguous().to(device)
+
+    return (per_class(high, torch.float64), per_class(low, torch.float64), per_class(n_smooth, torch.int32),
+            per_class(n_salt, torch.int32))
+
+
 @_on_device_of(0)
 def extract_events(frames, high, low, n_smooth, n_salt, max_events=64):
     """frames [n_clips, n_frames, classes] f32 cuda; per-class thresholds (sequences or scalars).
@@ -298,19 +315,7 @@ def extract_events(frames, high, low, n_smooth, n_salt, max_events=64):
     frames = frames.contiguous()
     n_clips, n_frames, classes = frames.shape
     dev = frames.device
-
-    def per_class(v, dtype):
-        if v is None:
-            return None
-        t = torch.as_tensor(np.asarray(v, dtype=np.float64 if dtype == torch.float64 else np.int64))
-        if t.dim() == 0:
-            t = t.repeat(classes)
-        if t.numel() != classes:
-            raise ValueError("expected %d per-class values, got %d" % (classes, t.numel()))
-        return t.to(dtype).contiguous().to(dev)
-
-    hi, lo = per_class(high, torch.float64), per_class(low, torch.float64)
-    ns, nsalt = per_class(n_smooth, torch.int32), per_class(n_salt, torch.int32)
+    hi, lo, ns, nsalt = event_params(high, low, n_smooth, n_salt, classes, dev)
     while True:
         events = torch.zeros((n_clips, classes, max_events, 2), dtype=torch.int32, device=dev)
         counts = torch.zeros((n_clips, classes), dtype=torch.int32, device=dev)
@@ -323,6 +328,36 @@ def extract_events(frames, high, low, n_smooth, n_salt, max_events=64):
         if most <= max_events:
             return events, counts
         max_events = most  # rare: more events than the buffer holds -> rerun once with the exact capacity
+
+
+@_on_device_of(0)
+def live_ingest(src, table, n_entries, max_len, ring_samples, arena):
+    """sed_live_ingest: chunks of `src` (packed, arena's dtype) -> their slots' mirrored rings in `arena`;
+    table = int64 CUDA tensor [>= n_entries, 4] of (slot, offset in src or -1 for zeros, length, stream position)."""
+    _call("sed_live_ingest", capi.ptr(src), _wave_dtype_code(arena), capi.ptr(table), int(n_entries), int(max_len),
+          int(ring_samples), capi.ptr(arena), capi.current_stream(arena.device))
+    capi._count()
+
+
+@_on_device_of(0)
+def live_merge(window_frames, table, n_entries, max_span, overlap_interval, sample_duration, acc, out):
+    """sed_live_merge: window_frames [rows, fpw, classes] of one push -> per-slot accumulators acc [slots, ring,
+    classes]; frames that became final -> out rows (table: int32 CUDA tensor [>= n_entries, LIVE_TABLE_COLS])."""
+    _, fpw, classes = window_frames.shape
+    _call("sed_live_merge", capi.ptr(window_frames), capi.ptr(table), int(n_entries), int(max_span), int(fpw),
+          int(classes), int(overlap_interval), int(sample_duration), int(acc.shape[1]), capi.ptr(acc), capi.ptr(out),
+          capi.current_stream(acc.device))
+    capi._count()
+
+
+@_on_device_of(0)
+def live_events(frames, table, n_entries, params, state, events, counts):
+    """sed_live_events over the frames sed_live_merge finalized; params = event_params(...) on the device."""
+    hi, lo, ns, nsalt = params
+    _call("sed_live_events", capi.ptr(frames), capi.ptr(table), int(n_entries), int(frames.shape[-1]), capi.ptr(hi),
+          capi.ptr(lo), capi.ptr(ns), capi.ptr(nsalt), capi.ptr(state), capi.ptr(events), capi.ptr(counts),
+          capi.current_stream(frames.device))
+    capi._count()
 
 
 def blocks_to_rows(xb, n, T):

@@ -6,9 +6,10 @@ the framewise outputs are overlap-added (`merge`) and block-averaged (`avg_merge
 Here the windows become the batch dimension -- the front-end kernel reads them in place from the recording with a
 1-second clip stride -- and merge/avg_merge run as one device kernel, bug-compatible with the numpy code.
 """
+import numpy as np
 import torch
 
-from . import engine
+from . import capi, engine
 
 
 def window_starts(audio_duration, sample_duration, overlap=True):
@@ -208,6 +209,284 @@ class HostStreamer:
             for j, (f, _) in enumerate(members):
                 merged[f] = host_out[j:j + 1]
         return merged
+
+
+# predict.py:252-257: the event parameters when no thresholds file is loaded
+DEFAULT_SED_PARAMS = {"sed_high_threshold": 0.5, "sed_low_threshold": 0.3, "n_smooth": 10, "n_salt": 10}
+
+LIVE_TICK_SECONDS = 2  # audio one internal tick takes per stream; larger pushes are split into several ticks
+
+
+def live_final_frames(windows_run, frames_per_window, overlap_interval, sample_duration):
+    """Frames of a stream's merged output that are final once `windows_run` windows (numpy int array) have been merged:
+    no later window covers them (f < windows_run * oi), and their avg_merge block has the same divisor for every total
+    length the stream can still reach (>= (windows_run - 1) * oi + fpw).  0 before the first window."""
+    oi, fpw = int(overlap_interval), int(frames_per_window)
+    k = np.asarray(windows_run, dtype=np.int64) - 1
+    tmin = k * oi + fpw
+    interval = int(sample_duration) * 100 - oi
+    b = np.minimum(tmin - oi, np.maximum(interval, tmin - interval))
+    lb = np.maximum(oi, -(-b // oi) * oi)
+    return np.where(k >= 0, np.minimum((k + 1) * oi, lb), 0)
+
+
+class LiveStreamer:
+    """Live detection on many streams at once: audio is pushed as it arrives, every window that becomes ready in any
+    stream runs in ONE batch, and each push returns the frames and events that have become final.
+
+    Equivalent, stream by stream, to the offline path on the concatenation `rec` of everything pushed up to `close`:
+      * frames: the concatenation of all returned `frames` equals predict_framewise(model, rec, ...)[0] bit for bit;
+      * events: label by label, the concatenation of all returned `events` equals frame_prediction_to_event_prediction
+        on that merged tensor, in the same order.
+    Timeliness:
+      * window k runs in the push after which the stream holds (k + sample_duration) * sample_rate samples; window 0
+        also runs, zero padded, at close if it never ran (window_starts' rule);
+      * a frame is returned once no later window covers it and its avg_merge block can no longer become a tail block;
+        for the shipped presets (frames_per_window 500 / 496, overlap interval <= 100) that is (k + 1) * oi frames after
+        the push that ran window k.  The tail blocks, whose divisor depends on the final length, come at close;
+      * with a low threshold that is not above the high threshold, an event with offset frame F is returned no later
+        than the push that finalizes frame F + n_smooth + 1 when frames F .. F + n_smooth + 1 are all below the low
+        threshold;
+      * without a low threshold the reference's last pair has no +1 on its offset (find_bgn_fin_pairs), so an event
+        stays open until the next run above the high threshold starts, or until close.
+
+    Per slot, the device holds a mirrored audio ring (windows are read in place by the front-end through its offset
+    table), a merge accumulator ring and the event state machine; the host holds the counters (samples, windows run,
+    frames returned) from which it builds each push's tables without a device round trip.  One device per streamer:
+    on several GPUs run one streamer per GPU."""
+
+    def __init__(self, model, sample_rate, sample_duration=5, overlap_value=1, max_streams=4096, dtype=torch.int16,
+                 sed_params=None, device=None, labels=None):
+        if dtype not in (torch.int16, torch.float32):
+            raise ValueError("dtype must be torch.int16 or torch.float32")
+        if isinstance(model, engine.PackedModel):
+            self.packed, self.micro_batch, self.variant = model, engine.DEFAULT_MICRO_BATCH, 4
+        else:
+            if model.training:
+                raise RuntimeError("inference only -- call .eval()")
+            if device is None:
+                device = next(model.parameters()).device
+            device = torch.device(device)
+            if device.type != "cuda":
+                raise RuntimeError("model is on %s; the B200 path has no CPU fallback" % (device,))
+            if device.index is None:
+                device = torch.device("cuda", torch.cuda.current_device())
+            self.packed = model._packed_for(device)
+            self.micro_batch, self.variant = model.micro_batch, model.conv_variant
+        self.device = self.packed.device
+        self.sr, self.dur, self.dtype = int(sample_rate), int(sample_duration), dtype
+        self.oi = int(100 * overlap_value)
+        self.W = self.sr * self.dur
+        self.fpw = self.packed.frames_for((self.W // self.packed.front.hop + 1) // 8)
+        self.classes = int(self.packed.classes)
+        self.labels = LABELS if labels is None else labels
+        self.max_streams = int(max_streams)
+        self.slack = LIVE_TICK_SECONDS * self.sr
+        self.ring = self.W + self.slack  # a multiple of sr: every window start is sr-aligned in the ring
+        self.ring_frames = (LIVE_TICK_SECONDS - 1) * self.oi + max(self.fpw, 100 * self.dur) + self.oi
+        p = DEFAULT_SED_PARAMS if sed_params is None else sed_params
+        with torch.cuda.device(self.device):
+            self.arena = torch.zeros(self.max_streams * 2 * self.ring, dtype=dtype, device=self.device)
+            self.acc = torch.empty((self.max_streams, self.ring_frames, self.classes), dtype=torch.float32,
+                                   device=self.device)
+            self.ev_state = torch.zeros(self.max_streams * self.classes * capi.LIVE_EVENT_STATE_INTS,
+                                        dtype=torch.int32, device=self.device)
+            self.ev_params = engine.event_params(p["sed_high_threshold"], p.get("sed_low_threshold"), p["n_smooth"],
+                                                 p["n_salt"], self.classes, self.device)
+        self.n_samples = np.zeros(self.max_streams, np.int64)
+        self.windows_run = np.zeros(self.max_streams, np.int64)
+        self.frames_out = np.zeros(self.max_streams, np.int64)
+        self.is_open = np.zeros(self.max_streams, bool)
+        self.names = [None] * self.max_streams
+        self._host = None  # pinned staging (grown on demand, reused)
+        self._dev = None
+
+    # ---- slots ----
+    def open(self, name=None):
+        """Start a stream; returns its slot id (the lowest free one: slots are reused after close)."""
+        free = np.flatnonzero(~self.is_open)
+        if free.size == 0:
+            raise RuntimeError("all %d streams are open" % self.max_streams)
+        sid = int(free[0])
+        self.is_open[sid] = True
+        self.n_samples[sid] = self.windows_run[sid] = self.frames_out[sid] = 0
+        self.names[sid] = name if name is not None else "stream-%d" % sid
+        return sid
+
+    def _check_sid(self, sid):
+        if not isinstance(sid, (int, np.integer)) or not 0 <= sid < self.max_streams or not self.is_open[sid]:
+            raise ValueError("stream %r is not open" % (sid,))
+        return int(sid)
+
+    def push(self, items):
+        """items: iterable of (sid, chunk), chunk a 1-D CPU (pinned preferred) or CUDA tensor of the streamer's dtype,
+        any length (several chunks of one stream are taken in order).  Returns {sid: {"first_frame", "frames",
+        "events"}} for every stream of the push: the newly final rows of its merged output (CPU float32
+        [n, classes], starting at frame `first_frame`) and its newly decided events."""
+        chunks = {}
+        for sid, chunk in items:
+            sid = self._check_sid(sid)
+            if not torch.is_tensor(chunk) or chunk.dtype != self.dtype:
+                raise TypeError("chunk for stream %d must be a %s tensor" % (sid, self.dtype))
+            if chunk.dim() != 1:
+                raise ValueError("chunk for stream %d must be 1-D, got shape %s" % (sid, tuple(chunk.shape)))
+            chunks.setdefault(sid, []).append(chunk)
+        sids = np.fromiter(chunks.keys(), np.int64, len(chunks))
+        parts = [c[0] if len(c) == 1 else torch.cat([t.to(self.device) for t in c] if any(t.is_cuda for t in c) else c)
+                 for c in chunks.values()]
+        return self._run(sids, parts, closing=False)
+
+    def close(self, sid):
+        """End a stream: runs window 0 (zero padded) if it never ran, returns the remaining frames (the tail blocks)
+        and events, in push()'s format for this one stream, and frees the slot."""
+        sid = self._check_sid(sid)
+        res = self._run(np.array([sid], np.int64), [torch.empty(0, dtype=self.dtype)], closing=True)[sid]
+        self.is_open[sid] = False
+        return res
+
+    # ---- one push ----
+    def _ready(self, n):
+        return np.where(n >= self.W, n // self.sr - self.dur + 1, 0)
+
+    def _run(self, sids, parts, closing):
+        S, sr, W, C, oi, fpw, ncls = len(sids), self.sr, self.W, self.ring, self.oi, self.fpw, self.classes
+        lens = np.fromiter((t.numel() for t in parts), np.int64, S)
+        on_dev = np.fromiter((t.is_cuda for t in parts), bool, S)
+        # audio layout in the staging buffer: host chunks first (one H2D copy), then device chunks
+        order = np.concatenate([np.flatnonzero(~on_dev), np.flatnonzero(on_dev)])
+        src = np.zeros(S, np.int64)
+        src[order] = np.concatenate([[0], np.cumsum(lens[order])[:-1]]) if S else []
+        n_host = int(lens[~on_dev].sum())
+        n_audio = int(lens.sum())
+        n_ticks = max(1, int(-(-lens.max() // self.slack)) if S else 1)
+
+        n0, k_run, f_ret = self.n_samples[sids].copy(), self.windows_run[sids].copy(), self.frames_out[sids].copy()
+        offsets, ticks, ev_total, rows_per_stream = [], [], 0, np.zeros(S, np.int64)
+        for t in range(n_ticks):
+            piece = np.clip(lens - t * self.slack, 0, self.slack)
+            ing = np.stack([sids, src + t * self.slack, piece, n0], 1)[piece > 0]
+            n1 = n0 + piece
+            ready = self._ready(n1)
+            last = closing and t == n_ticks - 1
+            if last:
+                zero = ready == 0  # window 0 runs at close, reading zeros past the end of the stream
+                ready = np.maximum(ready, 1)
+                fill = np.stack([sids, np.full(S, -1), W - n1, n1], 1)[zero & (n1 < W)]
+                ing = np.concatenate([ing, fill])
+            m = ready - k_run
+            total = (ready - 1) * oi + fpw
+            n_final = total if last else live_final_frames(ready, fpw, oi, self.dur)
+            sel = np.flatnonzero((m > 0) | last)
+            e = len(sel)
+            tab = np.zeros((e, capi.LIVE_TABLE_COLS), np.int64)
+            tab[:, 0], tab[:, 1], tab[:, 2] = sids[sel], k_run[sel], m[sel]
+            tab[:, 3] = np.concatenate([[0], np.cumsum(m[sel])[:-1]]) if e else []
+            tab[:, 4], tab[:, 5] = f_ret[sel], n_final[sel]
+            tab[:, 6] = rows_per_stream[sel]  # relative to the stream's block: rebased below
+            new = n_final[sel] - f_ret[sel]
+            cap = (new + 1) // 2 + 4  # see the output bound of live_events_kernel's state machine
+            tab[:, 7] = ev_total + np.concatenate([[0], np.cumsum(cap * ncls)[:-1]]) if e else []
+            tab[:, 8], tab[:, 9] = cap, int(last)
+            ev_total += int((cap * ncls).sum())
+            win = np.repeat(np.arange(e), m[sel])
+            k = np.arange(win.size) - np.repeat(tab[:, 3], m[sel]) + np.repeat(k_run[sel], m[sel])
+            offsets.append(sids[sel][win] * 2 * C + (k * sr) % C)
+            hi = np.where(m[sel] > 0, total[sel], n_final[sel])
+            ticks.append((ing, tab, sel, int(win.size), int((hi - f_ret[sel]).max()) if e else 0))
+            rows_per_stream[sel] += new
+            n0, k_run, f_ret = n1, np.maximum(k_run, ready), np.where((m > 0) | last, n_final, f_ret)
+        base = np.concatenate([[0], np.cumsum(rows_per_stream)[:-1]]) if S else np.zeros(0, np.int64)
+        for ing, tab, sel, _, _ in ticks:
+            tab[:, 6] += base[sel]
+        n_rows = int(rows_per_stream.sum())
+        n_entries = sum(len(tk[1]) for tk in ticks)
+
+        # one pinned staging buffer, one host->device copy: audio, then the tables of every tick
+        esz = 2 if self.dtype == torch.int16 else 4
+        a16 = lambda b: (b + 15) // 16 * 16
+        blobs = []
+        for ing, tab, _, _, _ in ticks:
+            blobs += [ing.astype(np.int64), tab.astype(np.int32)]
+        blobs += [np.concatenate(offsets).astype(np.int64)]
+        pos, at = [], a16(n_audio * esz)
+        for b in blobs:
+            pos.append(at)
+            at = a16(at + b.nbytes)
+        host, dev = self._staging(at)
+        if n_host:
+            hv = host[:n_host * esz].view(self.dtype)
+            torch.cat([parts[i] for i in np.flatnonzero(~on_dev)], out=hv)
+        for b, p in zip(blobs, pos):
+            host[p:p + b.nbytes].copy_(torch.from_numpy(b.view(np.uint8).reshape(-1)))
+        out_words = n_rows * ncls + 2 * ev_total + n_entries * ncls
+        with torch.cuda.device(self.device), torch.no_grad():
+            dev[:at].copy_(host[:at], non_blocking=True)
+            if n_audio > n_host:
+                torch.cat([parts[i].to(self.device) for i in np.flatnonzero(on_dev)],
+                          out=dev[n_host * esz:n_audio * esz].view(self.dtype))
+            audio = dev[:max(n_audio, 1) * esz].view(self.dtype)
+            view = lambda j, dt: dev[pos[j]:pos[j] + blobs[j].nbytes].view(dt)
+            out = torch.empty(max(out_words, 1), dtype=torch.int32, device=self.device)
+            frames = out[:n_rows * ncls].view(torch.float32).view(n_rows, ncls)
+            events = out[n_rows * ncls:n_rows * ncls + 2 * ev_total]
+            counts_all = out[n_rows * ncls + 2 * ev_total:]
+            off_all, e0, w0 = view(len(blobs) - 1, torch.int64), 0, 0
+            for j, (ing, tab, sel, n_win, span) in enumerate(ticks):
+                if len(ing):
+                    engine.live_ingest(audio, view(2 * j, torch.int64), len(ing), int(ing[:, 2].max()), C, self.arena)
+                if not len(tab):
+                    continue
+                if n_win:
+                    wf = self.packed.forward_windows(self.arena, W, 0, n_win, micro_batch=self.micro_batch,
+                                                     variant=self.variant, offsets=off_all[w0:w0 + n_win])
+                    wf = wf["framewise_output"].contiguous()
+                    w0 += n_win
+                else:
+                    wf = torch.empty((1, fpw, ncls), dtype=torch.float32, device=self.device)
+                t32 = view(2 * j + 1, torch.int32)
+                engine.live_merge(wf, t32, len(tab), span, oi, self.dur, self.acc, frames)
+                engine.live_events(frames, t32, len(tab), self.ev_params, self.ev_state, events,
+                                   counts_all[e0 * ncls:(e0 + len(tab)) * ncls])
+                e0 += len(tab)
+            res_host = self._result_buffer(out_words)
+            res_host[:out_words].copy_(out[:out_words], non_blocking=True)
+            torch.cuda.current_stream(self.device).synchronize()
+        res = res_host[:out_words].clone()
+
+        self.n_samples[sids], self.windows_run[sids], self.frames_out[sids] = n0, k_run, f_ret
+        fr = res[:n_rows * ncls].view(torch.float32).view(n_rows, ncls)
+        ev = res[n_rows * ncls:n_rows * ncls + 2 * ev_total].numpy()
+        cnt = res[n_rows * ncls + 2 * ev_total:].numpy().reshape(n_entries, ncls)
+        tab_all = np.concatenate([tk[1] for tk in ticks]) if n_entries else np.zeros((0, capi.LIVE_TABLE_COLS), np.int64)
+        if (cnt > tab_all[:, 8:9]).any():
+            raise RuntimeError("live event buffer overflow (%d > %d)" % (cnt.max(), tab_all[:, 8].max()))
+        first = self.frames_out[sids] - rows_per_stream
+        out_res = {}
+        for j, sid in enumerate(sids.tolist()):
+            out_res[sid] = {"first_frame": int(first[j]), "frames": fr[base[j]:base[j] + rows_per_stream[j]],
+                            "events": []}
+        # events in the reference's order within a push: class, then time (ticks are in time order)
+        for e, c in sorted(zip(*np.nonzero(cnt)), key=lambda ec: (int(tab_all[ec[0], 0]), ec[1], ec[0])):
+            sid = int(tab_all[e, 0])
+            name = self.names[sid]
+            p0 = int(tab_all[e, 7]) + int(c) * int(tab_all[e, 8])
+            for q in range(int(cnt[e, c])):
+                out_res[sid]["events"].append({"filename": name, "onset": ev[2 * (p0 + q)] / 100.0,
+                                               "offset": ev[2 * (p0 + q) + 1] / 100.0,
+                                               "event_label": self.labels[c]})
+        return out_res
+
+    def _staging(self, nbytes):
+        if self._host is None or self._host.numel() < nbytes:
+            size = max(nbytes, 1 << 20) * 5 // 4
+            self._host = torch.empty(size, dtype=torch.uint8).pin_memory()
+            self._dev = torch.empty(size, dtype=torch.uint8, device=self.device)
+        return self._host, self._dev
+
+    def _result_buffer(self, words):
+        if getattr(self, "_res", None) is None or self._res.numel() < words:
+            self._res = torch.empty(max(words, 1 << 18) * 5 // 4, dtype=torch.int32).pin_memory()
+        return self._res
 
 
 def overlap_window_counts(audio_durations, sample_duration, overlap_value):
