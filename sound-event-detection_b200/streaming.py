@@ -12,31 +12,77 @@ import torch
 from . import capi, engine
 
 
-def window_starts(audio_duration, sample_duration, overlap=True):
-    """Start times (s) of the windows the reference runs: predict.py:279-281, 297, 334-339."""
+def _resolve(model, device):
+    """(packed model, micro_batch, conv variant) that run `model` on `device`.  An engine.PackedModel runs where it was
+    packed (`device` is not used); a drop-in model is packed for `device` (a bare 'cuda' is the current device)."""
+    if isinstance(model, engine.PackedModel):
+        return model, engine.DEFAULT_MICRO_BATCH, 4
+    if model.training:
+        raise RuntimeError("inference only -- call .eval()")
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise RuntimeError("%s is not a CUDA device; the B200 path has no CPU fallback" % (device,))
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    return model._packed_for(device), model.micro_batch, model.conv_variant
+
+
+def _window_starts(duration, sample_duration, stride):
+    """The reference's window loop: a window starts at 0 and every `stride` while `end <= duration`, end updated after
+    each window.  The start accumulates `stride` (float accumulation for a float stride, as the reference does)."""
     starts = []
     start, end = 0, 0
-    while end <= audio_duration:
+    while end <= duration:
         starts.append(start)
-        start += 1 if overlap else sample_duration
+        start += stride
         end = start + sample_duration
     return starts
+
+
+def window_starts(audio_duration, sample_duration, overlap=True):
+    """Start times (s) of the windows the reference runs: predict.py:279-281, 297, 334-339."""
+    return _window_starts(audio_duration, sample_duration, 1 if overlap else sample_duration)
+
+
+def _layout(lengths, sample_rate, sample_duration):
+    """Recordings of `lengths` samples laid out one after another in one flat buffer, each zero padded up to the end
+    of its last window (the reference zero-pads the last window, predict.py:302-305).  Returns the window counts, the
+    segment lengths and the host list of window start offsets into the buffer."""
+    sr, window_samples = int(sample_rate), int(sample_rate * sample_duration)
+    counts, seg_len, offsets, base = [], [], [], 0
+    for n in lengths:
+        starts = window_starts(n / float(sample_rate), sample_duration, overlap=True)
+        counts.append(len(starts))
+        need = max(n, starts[-1] * sr + window_samples)
+        seg_len.append((need + 7) // 8 * 8)  # keep every segment 16-byte aligned for the cp.async staging
+        offsets.extend(base + k * sr for k in range(len(starts)))
+        base += seg_len[-1]
+    return counts, seg_len, offsets
+
+
+def _merge_groups(frames, counts, overlap_interval, sample_duration):
+    """Merge + avg_merge per recording: `frames` holds the windows of every recording in order, recording f has
+    counts[f] of them.  Recordings with the same number of windows are merged by one launch; yields (member indices,
+    merged [n_members, total_frames, classes]) per window count, in ascending order."""
+    groups, first = {}, 0
+    for f, nw in enumerate(counts):
+        groups.setdefault(nw, []).append((f, first))
+        first += nw
+    for nw, members in sorted(groups.items()):
+        if all(members[i + 1][1] == members[i][1] + nw for i in range(len(members) - 1)):
+            group = frames[members[0][1]:members[0][1] + nw * len(members)]  # contiguous rows: a view
+        else:
+            rows = torch.tensor([fst + k for _, fst in members for k in range(nw)], dtype=torch.int64).to(frames.device)
+            group = frames.index_select(0, rows)
+        group = group.view(len(members), nw, frames.shape[1], frames.shape[2])
+        yield [f for f, _ in members], engine.window_merge_avg(group, int(overlap_interval), int(sample_duration))
 
 
 def predict_framewise(model, recording, sample_rate, sample_duration=5, overlap_value=1, return_windows=False):
     """model: a sed_b200 drop-in model in eval mode (or an engine.PackedModel); recording: 1-D float32 / int16
     waveform on the model's CUDA device.  Returns merged framewise probabilities [1, total_frames, 25]
     (what `merged` holds after predict.py:349)."""
-    if isinstance(model, engine.PackedModel):
-        packed = model
-        micro_batch, variant = engine.DEFAULT_MICRO_BATCH, 4
-    else:
-        if model.training:
-            raise RuntimeError("inference only -- call .eval()")
-        if not recording.is_cuda:
-            raise RuntimeError("recording is on %s; the B200 path has no CPU fallback" % (recording.device,))
-        packed = model._packed_for(recording.device)
-        micro_batch, variant = model.micro_batch, model.conv_variant
+    packed, micro_batch, variant = _resolve(model, recording.device)
     audio_duration = recording.numel() / float(sample_rate)
     starts = window_starts(audio_duration, sample_duration, overlap=True)
     n_windows = len(starts)
@@ -44,7 +90,7 @@ def predict_framewise(model, recording, sample_rate, sample_duration=5, overlap_
     with torch.no_grad():
         out = packed.forward_windows(recording, window_samples, int(sample_rate), n_windows, micro_batch=micro_batch,
                                      variant=variant)
-        merged = engine.window_merge_avg(out["framewise_output"], int(100 * overlap_value), int(sample_duration))
+        _, merged = next(_merge_groups(out["framewise_output"], [n_windows], int(100 * overlap_value), sample_duration))
     if return_windows:
         return merged, out
     return merged
@@ -57,45 +103,23 @@ def predict_framewise_many(model, recordings, sample_rate, sample_duration=5, ov
     predict.py:302-305), the windows of all recordings are read in place through an offset table, and recordings with
     the same number of windows are merged by one launch.  Returns a list of [1, total_frames, classes] tensors equal,
     bit for bit, to calling predict_framewise per recording."""
-    if isinstance(model, engine.PackedModel):
-        packed, micro_batch, variant = model, engine.DEFAULT_MICRO_BATCH, 4
-    else:
-        if model.training:
-            raise RuntimeError("inference only -- call .eval()")
-        packed = model._packed_for(recordings[0].device)
-        micro_batch, variant = model.micro_batch, model.conv_variant
+    packed, micro_batch, variant = _resolve(model, recordings[0].device)
     dev, dtype = recordings[0].device, recordings[0].dtype
     if any(r.dim() != 1 or r.device != dev or r.dtype != dtype for r in recordings):
         raise ValueError("recordings must be 1-D tensors of one dtype on one CUDA device")
     window_samples = int(sample_rate * sample_duration)
-    counts, seg_len = [], []
-    for r in recordings:
-        starts = window_starts(r.numel() / float(sample_rate), sample_duration, overlap=True)
-        counts.append(len(starts))
-        need = max(r.numel(), starts[-1] * int(sample_rate) + window_samples)
-        seg_len.append((need + 7) // 8 * 8)  # keep every segment 16-byte aligned for the cp.async staging
+    counts, seg_len, offsets = _layout([r.numel() for r in recordings], sample_rate, sample_duration)
     flat = torch.zeros(sum(seg_len), dtype=dtype, device=dev)
-    offsets, base = [], 0
-    for r, nw, sl in zip(recordings, counts, seg_len):
+    base = 0
+    for r, sl in zip(recordings, seg_len):
         flat[base:base + r.numel()].copy_(r)
-        offsets.extend(base + k * int(sample_rate) for k in range(nw))
         base += sl
     offsets = torch.tensor(offsets, dtype=torch.int64, device=dev)
     with torch.no_grad():
         out = packed.forward_windows(flat, window_samples, 0, int(offsets.numel()), micro_batch=micro_batch,
                                      variant=variant, offsets=offsets)
-        frames = out["framewise_output"]
         merged = [None] * len(recordings)
-        firsts, first = [], 0
-        for nw in counts:
-            firsts.append(first)
-            first += nw
-        oi = int(100 * overlap_value)
-        for nw in sorted(set(counts)):
-            idx = [f for f in range(len(recordings)) if counts[f] == nw]
-            rows = torch.tensor([firsts[f] + k for f in idx for k in range(nw)], dtype=torch.int64, device=dev)
-            group = frames.index_select(0, rows).view(len(idx), nw, frames.shape[1], frames.shape[2])
-            m = engine.window_merge_avg(group, oi, int(sample_duration))
+        for idx, m in _merge_groups(out["framewise_output"], counts, int(100 * overlap_value), sample_duration):
             for j, f in enumerate(idx):
                 merged[f] = m[j:j + 1]
     return merged
@@ -111,33 +135,20 @@ class HostStreamer:
 
     def __init__(self, model, sample_rate, sample_duration=5, overlap_value=1):
         self.model, self.sr, self.dur, self.ov = model, int(sample_rate), int(sample_duration), overlap_value
-        self.packed = model if isinstance(model, engine.PackedModel) else None
         self.slots = [dict(), dict()]
         self.calls = 0
         self.pending = []
         self.copy_stream = None
 
-    def _packed(self, device):
-        if self.packed is not None:
-            return self.packed, engine.DEFAULT_MICRO_BATCH, 4
-        if self.model.training:
-            raise RuntimeError("inference only -- call .eval()")
-        return self.model._packed_for(device), self.model.micro_batch, self.model.conv_variant
-
     def submit(self, recordings, device):
         """recordings: list of 1-D CPU tensors (float32 or int16 PCM, one dtype).  Queues the call; returns a ticket."""
         device = torch.device(device)
-        packed, micro_batch, variant = self._packed(device)
+        packed, micro_batch, variant = _resolve(self.model, device)
         dtype = recordings[0].dtype
         if any(r.dim() != 1 or r.is_cuda or r.dtype != dtype for r in recordings) or dtype not in (torch.float32, torch.int16):
             raise ValueError("recordings must be 1-D float32 or int16 CPU tensors of one dtype")
         window_samples = self.sr * self.dur
-        counts, seg_len = [], []
-        for r in recordings:
-            starts = window_starts(r.numel() / float(self.sr), self.dur, overlap=True)
-            counts.append(len(starts))
-            need = max(r.numel(), starts[-1] * self.sr + window_samples)
-            seg_len.append((need + 7) // 8 * 8)
+        counts, seg_len, offs = _layout([r.numel() for r in recordings], self.sr, self.dur)
         total = sum(seg_len)
         slot = self.slots[self.calls % 2]
         if "done" in slot:
@@ -152,10 +163,6 @@ class HostStreamer:
                 slot["off_dev"] = torch.empty(sum(counts), dtype=torch.int64, device=device)
                 slot["key"] = key
                 slot["out"] = {}
-            base, offs = 0, []
-            for nw, sl in zip(counts, seg_len):
-                offs.extend(base + k * self.sr for k in range(nw))
-                base += sl
             slot["off_host"].copy_(torch.tensor(offs, dtype=torch.int64))
             slot["src"] = list(recordings)  # keeps pinned sources alive until their asynchronous copies have run
             compute = torch.cuda.current_stream(device)
@@ -174,20 +181,8 @@ class HostStreamer:
             with torch.no_grad():
                 out = packed.forward_windows(slot["dev"], window_samples, 0, len(offs), micro_batch=micro_batch,
                                              variant=variant, offsets=slot["off_dev"])
-                frames = out["framewise_output"]
-                oi = int(100 * self.ov)
-                groups, first = {}, 0
-                for f, nw in enumerate(counts):
-                    groups.setdefault(nw, []).append((f, first))
-                    first += nw
                 results = []
-                for nw, members in sorted(groups.items()):
-                    if all(members[i + 1][1] == members[i][1] + nw for i in range(len(members) - 1)):
-                        group = frames[members[0][1]:members[0][1] + nw * len(members)]  # contiguous rows: a view
-                    else:
-                        rows = torch.tensor([fst + k for _, fst in members for k in range(nw)], dtype=torch.int64).to(device)
-                        group = frames.index_select(0, rows)
-                    merged = engine.window_merge_avg(group.view(len(members), nw, frames.shape[1], frames.shape[2]), oi, self.dur)
+                for members, merged in _merge_groups(out["framewise_output"], counts, int(100 * self.ov), self.dur):
                     host_out = slot["out"].get(tuple(merged.shape))
                     if host_out is None:
                         host_out = slot["out"][tuple(merged.shape)] = torch.empty(merged.shape, dtype=torch.float32).pin_memory()
@@ -206,7 +201,7 @@ class HostStreamer:
         slot["done"].synchronize()
         merged = [None] * n
         for members, host_out in results:
-            for j, (f, _) in enumerate(members):
+            for j, f in enumerate(members):
                 merged[f] = host_out[j:j + 1]
         return merged
 
@@ -228,6 +223,67 @@ def live_final_frames(windows_run, frames_per_window, overlap_interval, sample_d
     b = np.minimum(tmin - oi, np.maximum(interval, tmin - interval))
     lb = np.maximum(oi, -(-b // oi) * oi)
     return np.where(k >= 0, np.minimum((k + 1) * oi, lb), 0)
+
+
+def _plan_live_push(sids, n_samples, windows_run, frames_out, lens, src, closing, sr, sample_duration, W, ring, oi, fpw,
+                    classes, slack):
+    """The tables of one LiveStreamer push, built from the host counters alone (numpy only, no device round trip).
+
+    sids, n_samples, windows_run, frames_out: the streams of the push and their counters before it; lens, src: each
+    stream's chunk length and its first sample in the staged audio; closing: the push closes its (one) stream.
+    Geometry: W samples per window, `ring` samples of mirrored audio ring per stream, oi / fpw frames of window stride /
+    window, `slack` samples per stream and tick (larger chunks are split into several ticks).  Returns
+      * ticks: per tick (ingest table, merge/event table, positions of its streams in `sids`, windows run, merge span
+        in frames);
+      * offsets: every window's start in the audio arena, ticks in order;
+      * rows_per_stream, base: rows of the push's output frames per stream and the first of them;
+      * n_rows, n_entries, ev_total: output rows, table entries and event slots of the push;
+      * (n_samples, windows_run, frames_out) after the push.
+    Every window a tick runs is resident in its stream's ring, no tick spans more frames than the merge accumulator
+    holds, and each entry's event capacity bounds what live_events_kernel writes for it."""
+    S = len(sids)
+    n_ticks = max(1, int(-(-lens.max() // slack)) if S else 1)
+    n0, k_run, f_ret = n_samples, windows_run, frames_out
+    offsets, ticks, ev_total, rows_per_stream = [], [], 0, np.zeros(S, np.int64)
+    for t in range(n_ticks):
+        piece = np.clip(lens - t * slack, 0, slack)
+        ing = np.stack([sids, src + t * slack, piece, n0], 1)[piece > 0]
+        n1 = n0 + piece
+        ready = np.where(n1 >= W, n1 // sr - sample_duration + 1, 0)
+        last = closing and t == n_ticks - 1
+        if last:
+            zero = ready == 0  # window 0 runs at close, reading zeros past the end of the stream
+            ready = np.maximum(ready, 1)
+            fill = np.stack([sids, np.full(S, -1), W - n1, n1], 1)[zero & (n1 < W)]
+            ing = np.concatenate([ing, fill])
+        m = ready - k_run
+        total = (ready - 1) * oi + fpw
+        n_final = total if last else live_final_frames(ready, fpw, oi, sample_duration)
+        sel = np.flatnonzero((m > 0) | last)
+        e = len(sel)
+        tab = np.zeros((e, capi.LIVE_TABLE_COLS), np.int64)
+        tab[:, 0], tab[:, 1], tab[:, 2] = sids[sel], k_run[sel], m[sel]
+        tab[:, 3] = np.concatenate([[0], np.cumsum(m[sel])[:-1]]) if e else []
+        tab[:, 4], tab[:, 5] = f_ret[sel], n_final[sel]
+        tab[:, 6] = rows_per_stream[sel]  # relative to the stream's block: rebased below
+        new = n_final[sel] - f_ret[sel]
+        cap = (new + 1) // 2 + 4  # see the output bound of live_events_kernel's state machine
+        tab[:, 7] = ev_total + np.concatenate([[0], np.cumsum(cap * classes)[:-1]]) if e else []
+        tab[:, 8], tab[:, 9] = cap, int(last)
+        ev_total += int((cap * classes).sum())
+        win = np.repeat(np.arange(e), m[sel])
+        k = np.arange(win.size) - np.repeat(tab[:, 3], m[sel]) + np.repeat(k_run[sel], m[sel])
+        offsets.append(sids[sel][win] * 2 * ring + (k * sr) % ring)
+        hi = np.where(m[sel] > 0, total[sel], n_final[sel])
+        ticks.append((ing, tab, sel, int(win.size), int((hi - f_ret[sel]).max()) if e else 0))
+        rows_per_stream[sel] += new
+        n0, k_run, f_ret = n1, np.maximum(k_run, ready), np.where((m > 0) | last, n_final, f_ret)
+    base = np.concatenate([[0], np.cumsum(rows_per_stream)[:-1]]) if S else np.zeros(0, np.int64)
+    for ing, tab, sel, _, _ in ticks:
+        tab[:, 6] += base[sel]
+    n_rows = int(rows_per_stream.sum())
+    n_entries = sum(len(tk[1]) for tk in ticks)
+    return ticks, np.concatenate(offsets), rows_per_stream, base, n_rows, n_entries, ev_total, (n0, k_run, f_ret)
 
 
 class LiveStreamer:
@@ -259,20 +315,9 @@ class LiveStreamer:
                  sed_params=None, device=None, labels=None):
         if dtype not in (torch.int16, torch.float32):
             raise ValueError("dtype must be torch.int16 or torch.float32")
-        if isinstance(model, engine.PackedModel):
-            self.packed, self.micro_batch, self.variant = model, engine.DEFAULT_MICRO_BATCH, 4
-        else:
-            if model.training:
-                raise RuntimeError("inference only -- call .eval()")
-            if device is None:
-                device = next(model.parameters()).device
-            device = torch.device(device)
-            if device.type != "cuda":
-                raise RuntimeError("model is on %s; the B200 path has no CPU fallback" % (device,))
-            if device.index is None:
-                device = torch.device("cuda", torch.cuda.current_device())
-            self.packed = model._packed_for(device)
-            self.micro_batch, self.variant = model.micro_batch, model.conv_variant
+        if device is None and not isinstance(model, engine.PackedModel):
+            device = next(model.parameters()).device
+        self.packed, self.micro_batch, self.variant = _resolve(model, device)
         self.device = self.packed.device
         self.sr, self.dur, self.dtype = int(sample_rate), int(sample_duration), dtype
         self.oi = int(100 * overlap_value)
@@ -345,11 +390,8 @@ class LiveStreamer:
         return res
 
     # ---- one push ----
-    def _ready(self, n):
-        return np.where(n >= self.W, n // self.sr - self.dur + 1, 0)
-
     def _run(self, sids, parts, closing):
-        S, sr, W, C, oi, fpw, ncls = len(sids), self.sr, self.W, self.ring, self.oi, self.fpw, self.classes
+        S, W, C, oi, fpw, ncls = len(sids), self.W, self.ring, self.oi, self.fpw, self.classes
         lens = np.fromiter((t.numel() for t in parts), np.int64, S)
         on_dev = np.fromiter((t.is_cuda for t in parts), bool, S)
         # audio layout in the staging buffer: host chunks first (one H2D copy), then device chunks
@@ -358,48 +400,9 @@ class LiveStreamer:
         src[order] = np.concatenate([[0], np.cumsum(lens[order])[:-1]]) if S else []
         n_host = int(lens[~on_dev].sum())
         n_audio = int(lens.sum())
-        n_ticks = max(1, int(-(-lens.max() // self.slack)) if S else 1)
-
-        n0, k_run, f_ret = self.n_samples[sids].copy(), self.windows_run[sids].copy(), self.frames_out[sids].copy()
-        offsets, ticks, ev_total, rows_per_stream = [], [], 0, np.zeros(S, np.int64)
-        for t in range(n_ticks):
-            piece = np.clip(lens - t * self.slack, 0, self.slack)
-            ing = np.stack([sids, src + t * self.slack, piece, n0], 1)[piece > 0]
-            n1 = n0 + piece
-            ready = self._ready(n1)
-            last = closing and t == n_ticks - 1
-            if last:
-                zero = ready == 0  # window 0 runs at close, reading zeros past the end of the stream
-                ready = np.maximum(ready, 1)
-                fill = np.stack([sids, np.full(S, -1), W - n1, n1], 1)[zero & (n1 < W)]
-                ing = np.concatenate([ing, fill])
-            m = ready - k_run
-            total = (ready - 1) * oi + fpw
-            n_final = total if last else live_final_frames(ready, fpw, oi, self.dur)
-            sel = np.flatnonzero((m > 0) | last)
-            e = len(sel)
-            tab = np.zeros((e, capi.LIVE_TABLE_COLS), np.int64)
-            tab[:, 0], tab[:, 1], tab[:, 2] = sids[sel], k_run[sel], m[sel]
-            tab[:, 3] = np.concatenate([[0], np.cumsum(m[sel])[:-1]]) if e else []
-            tab[:, 4], tab[:, 5] = f_ret[sel], n_final[sel]
-            tab[:, 6] = rows_per_stream[sel]  # relative to the stream's block: rebased below
-            new = n_final[sel] - f_ret[sel]
-            cap = (new + 1) // 2 + 4  # see the output bound of live_events_kernel's state machine
-            tab[:, 7] = ev_total + np.concatenate([[0], np.cumsum(cap * ncls)[:-1]]) if e else []
-            tab[:, 8], tab[:, 9] = cap, int(last)
-            ev_total += int((cap * ncls).sum())
-            win = np.repeat(np.arange(e), m[sel])
-            k = np.arange(win.size) - np.repeat(tab[:, 3], m[sel]) + np.repeat(k_run[sel], m[sel])
-            offsets.append(sids[sel][win] * 2 * C + (k * sr) % C)
-            hi = np.where(m[sel] > 0, total[sel], n_final[sel])
-            ticks.append((ing, tab, sel, int(win.size), int((hi - f_ret[sel]).max()) if e else 0))
-            rows_per_stream[sel] += new
-            n0, k_run, f_ret = n1, np.maximum(k_run, ready), np.where((m > 0) | last, n_final, f_ret)
-        base = np.concatenate([[0], np.cumsum(rows_per_stream)[:-1]]) if S else np.zeros(0, np.int64)
-        for ing, tab, sel, _, _ in ticks:
-            tab[:, 6] += base[sel]
-        n_rows = int(rows_per_stream.sum())
-        n_entries = sum(len(tk[1]) for tk in ticks)
+        ticks, offsets, rows_per_stream, base, n_rows, n_entries, ev_total, counters = _plan_live_push(
+            sids, self.n_samples[sids], self.windows_run[sids], self.frames_out[sids], lens, src, closing, self.sr,
+            self.dur, W, C, oi, fpw, ncls, self.slack)
 
         # one pinned staging buffer, one host->device copy: audio, then the tables of every tick
         esz = 2 if self.dtype == torch.int16 else 4
@@ -407,7 +410,7 @@ class LiveStreamer:
         blobs = []
         for ing, tab, _, _, _ in ticks:
             blobs += [ing.astype(np.int64), tab.astype(np.int32)]
-        blobs += [np.concatenate(offsets).astype(np.int64)]
+        blobs += [offsets.astype(np.int64)]
         pos, at = [], a16(n_audio * esz)
         for b in blobs:
             pos.append(at)
@@ -453,7 +456,7 @@ class LiveStreamer:
             torch.cuda.current_stream(self.device).synchronize()
         res = res_host[:out_words].clone()
 
-        self.n_samples[sids], self.windows_run[sids], self.frames_out[sids] = n0, k_run, f_ret
+        self.n_samples[sids], self.windows_run[sids], self.frames_out[sids] = counters
         fr = res[:n_rows * ncls].view(torch.float32).view(n_rows, ncls)
         ev = res[n_rows * ncls:n_rows * ncls + 2 * ev_total].numpy()
         cnt = res[n_rows * ncls + 2 * ev_total:].numpy().reshape(n_entries, ncls)
@@ -493,15 +496,7 @@ def overlap_window_counts(audio_durations, sample_duration, overlap_value):
     """Windows the loop of main_strong.py:786-834 runs per file: start k*overlap_value for k = 0 and every k with
     k*overlap_value + sample_duration <= audio_duration (the `while end <= audio_duration` rule, end updated after
     each window)."""
-    counts = []
-    for d in audio_durations:
-        n, start, end = 0, 0.0, 0.0
-        while end <= d:
-            n += 1
-            start += overlap_value
-            end = start + sample_duration
-        counts.append(n)
-    return counts
+    return [len(_window_starts(d, sample_duration, overlap_value)) for d in audio_durations]
 
 
 def predict_framewise_overlap(model, clips, sample_rate, sample_duration, overlap_value, audio_durations=None):
@@ -512,15 +507,7 @@ def predict_framewise_overlap(model, clips, sample_rate, sample_duration, overla
     10.0 each) -- they decide how many windows a file gets.  All windows of all files run as ONE batch (the front-end
     reads them in place through an offset table), each file's windows are overlap-added and block-averaged on the
     device.  Returns a list of per-file tensors [1, total_frames, classes] (what `merged` holds after :835)."""
-    if isinstance(model, engine.PackedModel):
-        packed, micro_batch, variant = model, engine.DEFAULT_MICRO_BATCH, 4
-    else:
-        if model.training:
-            raise RuntimeError("inference only -- call .eval()")
-        if not clips.is_cuda:
-            raise RuntimeError("clips are on %s; the B200 path has no CPU fallback" % (clips.device,))
-        packed = model._packed_for(clips.device)
-        micro_batch, variant = model.micro_batch, model.conv_variant
+    packed, micro_batch, variant = _resolve(model, clips.device)
     if clips.dim() != 2:
         raise ValueError("clips must be (n_files, samples)")
     n_files, L = clips.shape
@@ -541,19 +528,8 @@ def predict_framewise_overlap(model, clips, sample_rate, sample_duration, overla
     with torch.no_grad():
         out = packed.forward_windows(flat, window_samples, 0, len(starts), micro_batch=micro_batch, variant=variant,
                                      offsets=offsets)
-        frames = out["framewise_output"]
         merged = [None] * n_files
-        oi = int(100 * overlap_value)
-        first = 0
-        firsts = []
-        for nw in counts:
-            firsts.append(first)
-            first += nw
-        for nw in sorted(set(counts)):  # files with the same number of windows are merged by one launch
-            idx = [f for f in range(n_files) if counts[f] == nw]
-            rows = torch.tensor([firsts[f] + k for f in idx for k in range(nw)], dtype=torch.int64, device=clips.device)
-            group = frames.index_select(0, rows).view(len(idx), nw, frames.shape[1], frames.shape[2])
-            m = engine.window_merge_avg(group, oi, int(sample_duration))
+        for idx, m in _merge_groups(out["framewise_output"], counts, int(100 * overlap_value), sample_duration):
             for j, f in enumerate(idx):
                 merged[f] = m[j:j + 1]
     return merged

@@ -5,7 +5,7 @@ import pytest
 import torch
 
 from conftest import synthetic_sd
-from sed_b200 import models, stft, synth
+from sed_b200 import models, stft, streaming, synth
 
 
 @pytest.mark.parametrize("mt", synth.MODEL_TYPES)
@@ -58,11 +58,24 @@ def test_checkpoint_roundtrip_reference_format(mt, tmp_path):
 
 def test_refuses_training_mode_and_cpu_inputs():
     model = models.Cnn_9layers_Gru_FrameAtt(16000, 512, 160, 64, 25, 7000, 25, "logmel")
+    wave, clips = torch.zeros(16000), torch.zeros(2, 160000)
+    streaming_entries = [lambda: streaming.predict_framewise(model, wave, 16000),
+                         lambda: streaming.predict_framewise_many(model, [wave, wave], 16000),
+                         lambda: streaming.predict_framewise_overlap(model, clips, 16000, 5, 1),
+                         lambda: streaming.HostStreamer(model, 16000).submit([wave], "cpu"),
+                         lambda: streaming.LiveStreamer(model, 16000),
+                         lambda: streaming.LiveStreamer(model, 16000, device="cpu")]
     with pytest.raises(RuntimeError, match="inference only"):
         model(torch.zeros(1, 16000))
+    for entry in streaming_entries:
+        with pytest.raises(RuntimeError, match="inference only"):
+            entry()
     model.eval()
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         model(torch.zeros(1, 16000))
+    for entry in streaming_entries:
+        with pytest.raises(RuntimeError, match="no CPU fallback"):
+            entry()
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         stft.Spectrogram(n_fft=512, hop_length=160)(torch.zeros(1, 16000))
     with pytest.raises(RuntimeError, match="no CPU fallback"):

@@ -1,6 +1,7 @@
 """CPU model of the live (incremental) streaming path: the per-slot merge accumulator with its finality rule, and the
 resumable event state machine of csrc/sed_stream.cu (live_merge_kernel / live_events_kernel), restated in numpy and
-checked against the pinned oracle (stream_oracle.merge_windows / activity_detection) under random arrival patterns."""
+checked against the pinned oracle (stream_oracle.merge_windows / activity_detection) under random arrival patterns;
+and streaming.LiveStreamer's push planner itself, checked against the bounds these kernels rely on."""
 import json
 import os
 
@@ -320,3 +321,114 @@ def test_streaming_events_with_shipped_thresholds():
                 for chunk in (1, 37, len(x)):
                     _check(x, hi[c], None if lo is None else lo[c],
                            ns[c] if np.ndim(ns) else ns, salt[c] if np.ndim(salt) else salt, chunk)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# the push planner of streaming.LiveStreamer: ring residency, accumulator span, frame and event bookkeeping
+# ---------------------------------------------------------------------------------------------------------------
+def _check_plan(plan, sids, before, lens, src, closing, geometry):
+    """Checks one planned push against the stream counters `before` = (samples, windows run, frames returned) and
+    returns the counters after it, as the kernels would leave them."""
+    from sed_b200 import streaming
+    sr, dur, W, ring, oi, fpw, classes, slack = geometry
+    span_max = ring_frames(fpw, oi, dur, streaming.LIVE_TICK_SECONDS)
+    ticks, offsets, rows_per_stream, base, n_rows, n_entries, ev_total, after = plan
+    n, k_run, f_ret = (v.copy() for v in before)
+    taken, rows = np.zeros(len(sids), np.int64), np.zeros(len(sids), np.int64)
+    pos = {int(s): j for j, s in enumerate(sids)}
+    w0 = ev = entries = 0
+    for t, (ing, tab, sel, n_win, span) in enumerate(ticks):
+        last = closing and t == len(ticks) - 1
+        fill = {}
+        for sid, at, piece, n0 in ing.tolist():
+            j = pos[sid]
+            if at < 0:  # zero fill of the closing window 0 of a stream shorter than one window
+                assert last and k_run[j] == 0 and n0 == n[j] < W and piece == W - n0, (t, sid)
+                fill[j] = True
+                continue
+            assert at == src[j] + taken[j] and n0 == n[j] and 0 < piece, (t, sid)
+            taken[j] += piece
+            n[j] += piece
+        ready = np.where(n >= W, n // sr - dur + 1, 0)
+        if last:
+            ready = np.maximum(ready, 1)
+        assert sorted(sel.tolist()) == sorted(set(np.flatnonzero(ready > k_run).tolist()) |
+                                              (set(range(len(sids))) if last else set()))
+        tick_span = tick_windows = 0
+        for sid, k0, m, w_rel, f0, f1, row, ev0, cap, is_last in tab.tolist():
+            j = pos[sid]
+            assert k0 == k_run[j] and k0 + m == ready[j] and is_last == int(last) and w_rel == tick_windows
+            tick_windows += m
+            n1 = int(n[j])
+            for i, k in enumerate(range(k0, k0 + m)):
+                assert offsets[w0 + w_rel + i] == sid * 2 * ring + (k * sr) % ring
+                assert k * sr >= n1 - ring, ("window leaves the ring", sid, k, n1)
+                assert k * sr + W <= n1 or (last and k == 0 and fill.get(j)), ("window not ready", sid, k, n1)
+            # frames: continue where the stream stopped; final_frames after a push, the whole merged length at close
+            assert f0 == f_ret[j]
+            assert f1 == ((k0 + m - 1) * oi + fpw if last else final_frames(k0 + m, fpw, oi, dur))
+            assert row == base[j] + rows[j]
+            rows[j] += f1 - f0
+            hi = (k0 + m - 1) * oi + fpw if m else f1
+            tick_span = max(tick_span, hi - f0)
+            assert cap == event_capacity(f1 - f0) and ev0 == ev
+            ev += cap * classes
+            k_run[j], f_ret[j] = k0 + m, f1
+        assert span == tick_span and span <= span_max, (t, span, span_max)
+        assert n_win == tick_windows
+        w0 += n_win
+        entries += len(tab)
+    assert list(taken) == list(lens)
+    assert (w0, ev, entries, n_rows) == (len(offsets), ev_total, n_entries, int(rows.sum()))
+    assert list(rows) == list(rows_per_stream) and list(base) == list(np.cumsum(rows) - rows)
+    for got, want in zip(after, (n, k_run, f_ret)):
+        assert list(got) == list(want)
+    return n, k_run, f_ret
+
+
+PLAN_GEOMETRIES = [(16000, 500, 100, 5), (16000, 496, 100, 5), (32000, 500, 100, 5), (8000, 496, 100, 5),
+                   (16000, 500, 50, 6), (16000, 496, 50, 6), (8000, 600, 100, 5), (8000, 600, 50, 6)]
+
+
+@pytest.mark.parametrize("sr,fpw,oi,dur", PLAN_GEOMETRIES)
+def test_live_push_planner_keeps_windows_in_ring_and_frames_complete(sr, fpw, oi, dur):
+    """The real planner driven by random pushes of several streams (chunks of 0 and 1 samples, odd sizes, several
+    ticks, a stream that closes before one window): every window it runs is ready and resident in its stream's
+    audio ring, no tick spans more frames than the accumulator ring, entries finalize frames contiguously and with
+    the finality rule above, their event capacity is event_capacity, and at close a stream has returned the whole
+    offline merged length."""
+    from sed_b200 import streaming
+    classes = 3
+    slack = streaming.LIVE_TICK_SECONDS * sr
+    W, ring = sr * dur, sr * dur + slack
+    geometry = (sr, dur, W, ring, oi, fpw, classes, slack)
+    rng = np.random.RandomState(sr + fpw + oi + dur)
+    for trial in range(4):
+        total = [0, 1, W // 2 + 3, W - 1, W, W + sr - 1, 9 * sr + 123, 31 * sr + 7]
+        sid_of = rng.permutation(12)[:len(total)]  # slot ids: not the stream order, not contiguous
+        n = np.zeros(12, np.int64)
+        k_run, f_ret = n.copy(), n.copy()
+        fed = [0] * len(total)
+        sizes = [0, 1, 777, sr - 1, sr, 2 * sr, 2 * sr + 5, 5 * sr + 3]
+        open_ = list(range(len(total)))
+        while open_:
+            push = [i for i in open_ if rng.rand() < 0.8]
+            lens = np.array([min(int(rng.choice(sizes)), total[i] - fed[i]) for i in push], np.int64)
+            sids = sid_of[push].astype(np.int64)
+            order = rng.permutation(len(push))  # any disjoint layout of the chunks in the staged audio
+            src = np.zeros(len(push), np.int64)
+            src[order] = np.concatenate([[0], np.cumsum(lens[order])[:-1]]) if len(push) else []
+            before = (n[sids], k_run[sids], f_ret[sids])
+            plan = streaming._plan_live_push(sids, *before, lens, src, False, *geometry)
+            n[sids], k_run[sids], f_ret[sids] = _check_plan(plan, sids, before, lens, src, False, geometry)
+            for i, ln in zip(push, lens):
+                fed[i] += int(ln)
+            for i in [i for i in open_ if fed[i] == total[i] and rng.rand() < 0.5]:
+                sids = sid_of[[i]].astype(np.int64)
+                before = (n[sids], k_run[sids], f_ret[sids])
+                zero = np.zeros(1, np.int64)
+                plan = streaming._plan_live_push(sids, *before, zero, zero, True, *geometry)
+                n[sids], k_run[sids], f_ret[sids] = _check_plan(plan, sids, before, zero, zero, True, geometry)
+                nw = len(stream_oracle.window_starts(total[i] / float(sr), dur))
+                assert k_run[sid_of[i]] == nw and f_ret[sid_of[i]] == (nw - 1) * oi + fpw, (trial, i)
+                open_.remove(i)
