@@ -202,6 +202,38 @@ int sed_live_events(const float* frames, const int* table, int n_entries, int cl
                     const double* low, const int* n_smooth, const int* n_salt, void* state, int* events, int* counts,
                     void* stream);
 
+/* ---- Sample-rate conversion and downmix ---------------------------------------------------------------------------
+ * Replaces librosa.load(path, sr=sample_rate, mono=True) of pytorch/predict.py:288-295 for decoded audio: the
+ * channels are averaged (numpy's x.astype(float32).mean(axis=1), int16 PCM as q / 32767), then
+ *   y[j] = sum_i x[i] * taps[j*down + half - i*up]   (0 <= j < ceil(n_in*up/down); x[i] = 0 outside [0, n_in))
+ * is summed over ascending i in float32 FMAs -- scipy.signal.resample_poly(x, up, down, window=h) with taps = up*h.
+ * Both device entries take the taps sed_resample_filter returns (n_taps = 2*half + 1 floats on the device; any
+ * odd-length filter works), int16 (dtype 1) or float32 (dtype 0) frames of 1 <= channels <= 8 interleaved samples. */
+
+/* HOST helper: the polyphase filter for in_rate -> out_rate (both 1 .. 384000).  up = out_rate/g, down = in_rate/g
+ * (g = gcd), half = 64*max(up, down), *n_taps = 2*half + 1; taps_or_NULL (host, *n_taps floats) receives
+ * float32(up * h), h = scipy.signal.firwin(n_taps, 0.9475937167399596 / max(up, down), window=('kaiser',
+ * 14.769656459379492)) computed in float64 (resampy's kaiser_best design).  Call with NULL for the sizes first.
+ * SED_ERR_UNSUPPORTED when max(up, down) > 4096. */
+int sed_resample_filter(int in_rate, int out_rate, int* up, int* down, int* n_taps, float* taps_or_NULL);
+
+/* Many recordings in one launch.  table [n_rows, 4] i64 = (first frame in src, n_in frames, first sample in dst,
+ * n_out samples); max_out >= every n_out.  dst f32: only the n_out samples of each row are written. */
+int sed_resample(const void* src, int dtype, int channels, const long* table, int n_rows, long max_out,
+                 const float* taps, int up, int down, int half, float* dst, void* stream);
+
+/* Live ingest with resampling: computes model-rate samples of live streams into the mirrored rings of
+ * sed_live_ingest (arena f32 [n_slots, 2*ring_samples]).  table [n_entries, 6] i64 = (slot, first output j0, outputs
+ * (<= max_len), first frame of the stream's chunk in src or -1 to write zeros, n_prev = input frames before this
+ * push, n_end = input frames after it).  Input i reads the chunk for n_prev <= i < n_end, the slot's history
+ * hist[slot*history_len + i mod history_len] (f32) for 0 <= i < n_prev, and zero otherwise: an output must only need
+ * i >= n_prev - history_len.  After the outputs, history_table [n_history, 4] i64 = (slot, first frame of the chunk
+ * in src, n_prev, frames) stores the last min(frames, history_len) downmixed inputs of each chunk into its history:
+ * pass it with the last call of a push (n_history = 0 otherwise; table may be NULL when n_entries = 0). */
+int sed_live_resample(const void* src, int dtype, int channels, const long* table, int n_entries, long max_len,
+                      const float* taps, int up, int down, int half, long ring_samples, float* arena, float* hist,
+                      int history_len, const long* history_table, int n_history, void* stream);
+
 /* ---- Peer-memory result buffers (multi-GPU gather without a collective on the data path) -------------------------
  * The reference gathers replica outputs on GPU 0 inside torch.nn.DataParallel (pytorch/main_strong.py:541,
  * pytorch/predict.py:239).  Here the destination rank owns ONE buffer for the results of all ranks; every other rank

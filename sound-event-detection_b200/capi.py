@@ -34,6 +34,9 @@ SIGNATURES = {
     "sed_live_ingest": ([_p, _i, _p, _i, _l, _l, _p, _p], _i),
     "sed_live_merge": ([_p, _p, _i, _i, _i, _i, _i, _i, _i, _p, _p, _p], _i),
     "sed_live_events": ([_p, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p], _i),
+    "sed_resample_filter": ([_i, _i, _p, _p, _p, _p], _i),
+    "sed_resample": ([_p, _i, _i, _p, _i, _l, _p, _i, _i, _i, _p, _p], _i),
+    "sed_live_resample": ([_p, _i, _i, _p, _i, _l, _p, _i, _i, _i, _l, _p, _p, _i, _p, _i, _p], _i),
     "sed_spectrogram_f32": ([_p, _i, _i, _i, _i, _p, _p, _p, _p], _i),
     "sed_logmel_rows_f32": ([_p, _l, _i, _p, _p, _p, _p, _i, _f, _f, _i, _p, _p], _i),
     "sed_conv_first_f32": ([_p, _i, _i, _i, _p, _p, _p, _p, _i, _p], _i),

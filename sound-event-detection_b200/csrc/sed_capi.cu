@@ -108,6 +108,28 @@ int sed_live_events(const float* frames, const int* table, int n_entries, int cl
                                  as_stream(stream));
 }
 
+int sed_resample_filter(int in_rate, int out_rate, int* up, int* down, int* n_taps, float* taps_or_NULL) {
+  SED_REQUIRE(up); SED_REQUIRE(down); SED_REQUIRE(n_taps);
+  return sed::resample_filter_host(in_rate, out_rate, up, down, n_taps, taps_or_NULL);
+}
+
+int sed_resample(const void* src, int dtype, int channels, const long* table, int n_rows, long max_out,
+                 const float* taps, int up, int down, int half, float* dst, void* stream) {
+  SED_REQUIRE(src); SED_REQUIRE(table); SED_REQUIRE(taps); SED_REQUIRE(dst);
+  return sed::resample_launch(src, dtype, channels, table, n_rows, max_out, taps, up, down, half, dst,
+                              as_stream(stream));
+}
+
+int sed_live_resample(const void* src, int dtype, int channels, const long* table, int n_entries, long max_len,
+                      const float* taps, int up, int down, int half, long ring_samples, float* arena, float* hist,
+                      int history_len, const long* history_table, int n_history, void* stream) {
+  SED_REQUIRE(src); SED_REQUIRE(taps); SED_REQUIRE(arena); SED_REQUIRE(hist);
+  if (n_entries > 0) SED_REQUIRE(table);  // a push's last call may only update the history
+  if (n_history > 0) SED_REQUIRE(history_table);
+  return sed::live_resample_launch(src, dtype, channels, table, n_entries, max_len, taps, up, down, half, ring_samples,
+                                   arena, hist, history_len, history_table, n_history, as_stream(stream));
+}
+
 int sed_logmel_rows_f32(const float* spec, long rows, int F, const int* mel_lo, const int* mel_len,
                         const int* mel_off, const float* mel_val, int n_mels, float amin, float db_offset,
                         int is_log, float* out, void* stream) {

@@ -306,6 +306,20 @@ SED_DEVICE_INLINE void umma_commit_2sm(uint64_t* bar, uint16_t cta_mask) {
       : "memory");
 }
 
+// ------------------------------------------------------------------ input samples
+// int16 PCM input follows the reference's HDF5 path: x = q / 32767 (utils/utilities.py:78-79).  The three-operation
+// sequence below (multiply by the rounded reciprocal, exact residual, correction) returns the correctly rounded
+// float32 quotient for every int16 q (checked exhaustively on the host) -- the value numpy's
+// (q / 32767.).astype(float32) produces.  Used by the front-end and by the resampler's downmix.
+SED_DEVICE_INLINE float load_sample(const float* p) { return *p; }
+SED_DEVICE_INLINE float load_sample(const short* p) {
+  const float q = static_cast<float>(*p);
+  constexpr float kInv = 1.0f / 32767.0f;
+  const float r = q * kInv;
+  const float e = fmaf(-r, 32767.0f, q);
+  return fmaf(e, kInv, r);
+}
+
 // ------------------------------------------------------------------ 16-bit element traits
 template <typename T>
 struct Elem16;

@@ -258,18 +258,7 @@ struct PassTw {
   }
 };
 
-// int16 PCM input follows the reference's HDF5 path: x = q / 32767 (utils/utilities.py:78-79).  The three-operation
-// sequence below (multiply by the rounded reciprocal, exact residual, correction) returns the correctly rounded
-// float32 quotient for every int16 q (checked exhaustively on the host) -- the value numpy's
-// (q / 32767.).astype(float32) produces.
-__device__ __forceinline__ float load_sample(const float* p) { return *p; }
-__device__ __forceinline__ float load_sample(const short* p) {
-  const float q = static_cast<float>(*p);
-  constexpr float kInv = 1.0f / 32767.0f;
-  const float r = q * kInv;
-  const float e = fmaf(-r, 32767.0f, q);
-  return fmaf(e, kInv, r);
-}
+// load_sample (int16 PCM as q / 32767, correctly rounded) lives in sed_common.cuh: sed_resample.cu shares it.
 __device__ __forceinline__ float load_sample_global(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float load_sample_global(const short* p) { return static_cast<float>(__ldg(p)); }
 __device__ __forceinline__ void store_raw(float* p, float v) { *p = v; }

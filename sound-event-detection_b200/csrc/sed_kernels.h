@@ -68,6 +68,14 @@ int live_events_launch(const float* frames, const int* table, int n_entries, int
                        const double* low, const int* n_smooth, const int* n_salt, void* state, int* events, int* counts,
                        cudaStream_t stream);
 
+// sed_resample.cu: sample-rate conversion + downmix
+int resample_launch(const void* src, int dtype, int channels, const long* table, int n_rows, long max_out,
+                    const float* taps, int up, int down, int half, float* dst, cudaStream_t stream);
+int live_resample_launch(const void* src, int dtype, int channels, const long* table, int n_entries, long max_len,
+                         const float* taps, int up, int down, int half, long ring_samples, float* arena, float* hist,
+                         int history_len, const long* history_table, int n_history, cudaStream_t stream);
+int resample_filter_host(int in_rate, int out_rate, int* up, int* down, int* n_taps, float* taps);
+
 int mha_core_launch(const float* qkv, int B, int T, long rs_t, long rs_b, void* out16, int dtype, cudaStream_t stream);
 
 int mha_tc_launch(const void* qkv16, const void* qk_lo16, int B, int T, long Bp, void* ctx16, int dtype,

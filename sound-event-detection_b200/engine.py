@@ -11,6 +11,7 @@ batch of 1024 is one launch group with a 14.5 GB activation workspace); the temp
 the batch.
 """
 import collections
+import ctypes
 import functools
 import math
 import threading
@@ -358,6 +359,83 @@ def live_events(frames, table, n_entries, params, state, events, counts):
           capi.ptr(lo), capi.ptr(ns), capi.ptr(nsalt), capi.ptr(state), capi.ptr(events), capi.ptr(counts),
           capi.current_stream(frames.device))
     capi._count()
+
+
+def resample_filter(input_rate, output_rate):
+    """sed_resample_filter (host helper): (up, down, half, float32 taps) of the polyphase filter input_rate ->
+    output_rate.  ValueError for a rate pair it refuses (rates outside 1 .. 384000, max(up, down) > 4096)."""
+    lib = capi.load()
+    up, down, n = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
+    args = (int(input_rate), int(output_rate), ctypes.byref(up), ctypes.byref(down), ctypes.byref(n))
+    rc = lib.sed_resample_filter(*args, None)
+    if rc == 0:
+        taps = np.zeros(n.value, np.float32)
+        rc = lib.sed_resample_filter(*args, taps.ctypes.data_as(ctypes.c_void_p))
+    if rc != 0:
+        raise ValueError("cannot resample %s Hz -> %s Hz: %s" % (input_rate, output_rate,
+                                                                 lib.sed_last_error_string().decode("utf-8", "replace")))
+    return up.value, down.value, (n.value - 1) // 2, taps
+
+
+class ResamplePlan:
+    """The filter input_rate -> output_rate on one device.  Equal rates keep librosa.load's behaviour (no resampling,
+    downmix only): the one-tap filter [1.0], for which y[j] = x[j] exactly."""
+
+    def __init__(self, input_rate, output_rate, device):
+        self.input_rate, self.output_rate = int(input_rate), int(output_rate)
+        if self.input_rate == self.output_rate and 0 < self.input_rate <= 384000:
+            self.up = self.down = 1
+            self.half, taps = 0, np.ones(1, np.float32)
+        else:
+            self.up, self.down, self.half, taps = resample_filter(input_rate, output_rate)
+        self.n_taps = 2 * self.half + 1
+        self.taps = torch.from_numpy(taps).to(device)
+
+    def n_out(self, n_in):
+        """Output samples of a whole recording of n_in input samples: ceil(n_in * up / down)."""
+        return -(-np.asarray(n_in, np.int64) * self.up // self.down)
+
+    def n_out_live(self, n_in):
+        """Outputs whose whole filter support lies in the first n_in input samples (before a stream's end)."""
+        n_in = np.asarray(n_in, np.int64)
+        return np.maximum(0, ((n_in - 1) * self.up - self.half) // self.down + 1)
+
+    def history_len(self):
+        """Input samples a live stream keeps from earlier pushes (DESIGN.md K7 derives the bound)."""
+        return -(-(self.n_taps - 1 + self.down) // self.up) + 1
+
+
+_RESAMPLE_PLANS = {}
+
+
+def resample_plan(input_rate, output_rate, device):
+    key = (int(input_rate), int(output_rate), torch.device(device))
+    if key not in _RESAMPLE_PLANS:
+        _RESAMPLE_PLANS[key] = ResamplePlan(input_rate, output_rate, device)
+    return _RESAMPLE_PLANS[key]
+
+
+@_on_device_of(0)
+def resample(src, channels, table, n_rows, max_out, plan, dst):
+    """sed_resample: the recordings of `src` (interleaved frames of `channels` samples, float32 or int16) -> float32
+    `dst`; table = int64 CUDA tensor [>= n_rows, 4] of (first frame in src, n_in, first sample in dst, n_out)."""
+    _call("sed_resample", capi.ptr(src), _wave_dtype_code(src), int(channels), capi.ptr(table), int(n_rows),
+          int(max_out), capi.ptr(plan.taps), plan.up, plan.down, plan.half, capi.ptr(dst),
+          capi.current_stream(src.device))
+    capi._count()
+
+
+@_on_device_of(0)
+def live_resample(src, channels, table, n_entries, max_len, plan, ring_samples, arena, hist, history_len, history_table,
+                  n_history):
+    """sed_live_resample: one tick of live ingest with resampling (table: int64 [>= n_entries, 6]); with n_history > 0
+    the push's chunks then go into the slots' history rings hist [slots, history_len] (history_table: int64
+    [>= n_history, 4])."""
+    _call("sed_live_resample", capi.ptr(src), _wave_dtype_code(src), int(channels), capi.ptr(table), int(n_entries),
+          int(max_len), capi.ptr(plan.taps), plan.up, plan.down, plan.half, int(ring_samples), capi.ptr(arena),
+          capi.ptr(hist), int(history_len), capi.ptr(history_table),
+          int(n_history), capi.current_stream(arena.device))
+    capi._count((1 if n_entries and max_len else 0) + (1 if n_history else 0))
 
 
 def blocks_to_rows(xb, n, T):

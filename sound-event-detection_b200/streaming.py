@@ -125,30 +125,89 @@ def predict_framewise_many(model, recordings, sample_rate, sample_duration=5, ov
     return merged
 
 
+def _check_channels(channels):
+    if not isinstance(channels, (int, np.integer)) or not 1 <= channels <= 8:
+        raise ValueError("channels must be an int in 1 .. 8, got %r" % (channels,))
+    return int(channels)
+
+
+def _frames(rec, channels, what):
+    """Frames of a [n] (mono) or [n, channels] recording or chunk; ValueError for any other shape."""
+    if rec.dim() == 2 and rec.shape[1] == channels or rec.dim() == 1 and channels == 1:
+        return int(rec.shape[0])
+    raise ValueError("%s must be [n, %d]%s, got shape %s" % (what, channels, " or [n]" if channels == 1 else "",
+                                                             tuple(rec.shape)))
+
+
+def resample(recordings, input_rate, sample_rate, channels=1):
+    """librosa.load(path, sr=sample_rate, mono=True) (pytorch/predict.py:288-295) for decoded audio on the device:
+    `recordings` is a list of CUDA tensors of one dtype (float32, or int16 PCM read as q / 32767), each [n] or
+    [n, channels] at `input_rate`.  The channels are averaged, then the polyphase filter of engine.resample_filter
+    resamples to `sample_rate`, every recording in ONE launch.  Returns 1-D float32 CUDA tensors of
+    ceil(n * up / down) samples.  Equal rates only downmix (librosa does not resample then)."""
+    channels = _check_channels(channels)
+    if not recordings:
+        raise ValueError("no recordings")
+    dev, dtype = recordings[0].device, recordings[0].dtype
+    if dtype not in (torch.float32, torch.int16) or dev.type != "cuda":
+        raise ValueError("recordings must be float32 or int16 CUDA tensors, got %s on %s" % (dtype, dev))
+    if any(r.dtype != dtype or r.device != dev for r in recordings):
+        raise ValueError("recordings must be tensors of one dtype on one CUDA device")
+    n_in = np.array([_frames(r, channels, "recording") for r in recordings], np.int64)
+    plan = engine.resample_plan(input_rate, sample_rate, dev)
+    n_out = plan.n_out(n_in)
+    table = np.stack([np.cumsum(n_in) - n_in, n_in, np.cumsum(n_out) - n_out, n_out], 1)
+    src = torch.cat([r.reshape(-1) for r in recordings])
+    dst = torch.empty(max(int(n_out.sum()), 1), dtype=torch.float32, device=dev)
+    with torch.no_grad():
+        engine.resample(src if src.numel() else dst, channels, torch.from_numpy(table).to(dev), len(recordings),
+                        int(n_out.max()), plan, dst)
+    return list(dst[:int(n_out.sum())].split(n_out.tolist()))
+
+
 class HostStreamer:
     """predict_framewise_many for recordings that live in HOST memory, end to end: every recording of a call is copied
     by DMA from the caller's (pinned) buffer straight to its place in one flat device buffer (zero padded up to the end
     of its last window by a device memset; nothing is repacked on the host), the window offset table is built on the
     host, and the merged frames of all recordings come back with one device->host copy per window-count group.  Two staging slots alternate, so the copy in of call k+1 can be queued while call k
     computes (`submit` returns at once, `result` blocks for the oldest call).  Replaces the per-file, per-window loop of
-    pytorch/predict.py:264-349, which reads each window back to the host before it runs the next one."""
+    pytorch/predict.py:264-349, which reads each window back to the host before it runs the next one.
 
-    def __init__(self, model, sample_rate, sample_duration=5, overlap_value=1):
+    With `input_rate` (Hz) other than `sample_rate`, or `channels` > 1, recordings are [n] or [n, channels] at
+    `input_rate`: they are copied as they are into a device staging buffer and sed_resample downmixes and resamples
+    all of them in one launch straight into the padded layout -- equal, bit for bit, to
+    predict_framewise_many(model, resample(recordings on the device, input_rate, sample_rate, channels))."""
+
+    def __init__(self, model, sample_rate, sample_duration=5, overlap_value=1, input_rate=None, channels=1):
         self.model, self.sr, self.dur, self.ov = model, int(sample_rate), int(sample_duration), overlap_value
+        self.channels = _check_channels(channels)
+        self.input_rate = self.sr if input_rate is None else int(input_rate)
+        self.resampling = self.input_rate != self.sr or self.channels != 1
+        if self.resampling and self.input_rate != self.sr:
+            engine.resample_filter(self.input_rate, self.sr)  # ValueError now for a rate pair the filter refuses
         self.slots = [dict(), dict()]
         self.calls = 0
         self.pending = []
         self.copy_stream = None
 
     def submit(self, recordings, device):
-        """recordings: list of 1-D CPU tensors (float32 or int16 PCM, one dtype).  Queues the call; returns a ticket."""
+        """recordings: list of CPU tensors (float32 or int16 PCM, one dtype), 1-D at sample_rate -- or, when
+        resampling, [n] / [n, channels] at input_rate.  Queues the call; returns a ticket."""
         device = torch.device(device)
         packed, micro_batch, variant = _resolve(self.model, device)
         dtype = recordings[0].dtype
-        if any(r.dim() != 1 or r.is_cuda or r.dtype != dtype for r in recordings) or dtype not in (torch.float32, torch.int16):
+        if self.resampling:
+            if any(r.is_cuda or r.dtype != dtype for r in recordings) or dtype not in (torch.float32, torch.int16):
+                raise ValueError("recordings must be float32 or int16 CPU tensors of one dtype")
+            n_in = np.array([_frames(r, self.channels, "recording") for r in recordings], np.int64)
+            plan = engine.resample_plan(self.input_rate, self.sr, device)
+            lengths = plan.n_out(n_in).tolist()
+        elif any(r.dim() != 1 or r.is_cuda or r.dtype != dtype for r in recordings) or dtype not in (torch.float32, torch.int16):
             raise ValueError("recordings must be 1-D float32 or int16 CPU tensors of one dtype")
+        else:
+            lengths = [r.numel() for r in recordings]
         window_samples = self.sr * self.dur
-        counts, seg_len, offs = _layout([r.numel() for r in recordings], self.sr, self.dur)
+        counts, seg_len, offs = _layout(lengths, self.sr, self.dur)
         total = sum(seg_len)
         slot = self.slots[self.calls % 2]
         if "done" in slot:
@@ -156,29 +215,39 @@ class HostStreamer:
         with torch.cuda.device(device):
             if self.copy_stream is None:
                 self.copy_stream = torch.cuda.Stream(device)
-            key = (total, dtype, len(recordings))
-            if slot.get("key") != key:
-                slot["dev"] = torch.empty(total, dtype=dtype, device=device)
-                slot["off_host"] = torch.zeros(sum(counts), dtype=torch.int64).pin_memory()
-                slot["off_dev"] = torch.empty(sum(counts), dtype=torch.int64, device=device)
-                slot["key"] = key
-                slot["out"] = {}
-            slot["off_host"].copy_(torch.tensor(offs, dtype=torch.int64))
-            slot["src"] = list(recordings)  # keeps pinned sources alive until their asynchronous copies have run
             compute = torch.cuda.current_stream(device)
             cs = self.copy_stream  # the slot's previous call has finished (host-synchronised above): copy at once,
             with torch.cuda.stream(cs):  # under the kernels of the call queued before this one
-                # the DMA engine does the layout: every recording goes straight from the caller's (pinned) buffer to its
-                # place in the flat device buffer -- no host-side repacking; the zero padding is a device memset
-                base = 0
-                for r, sl in zip(recordings, seg_len):
-                    slot["dev"][base:base + r.numel()].copy_(r, non_blocking=True)
-                    if r.numel() < sl:
-                        slot["dev"][base + r.numel():base + sl].zero_()
-                    base += sl
+                key = (total, dtype, len(recordings))
+                if slot.get("key") != key:
+                    # allocated on the copy stream, which writes them while the compute stream may still run the
+                    # previous call: memory that call's temporaries free on the compute stream is never handed out here
+                    slot["dev"] = torch.empty(total, dtype=torch.float32 if self.resampling else dtype, device=device)
+                    slot["off_host"] = torch.zeros(sum(counts), dtype=torch.int64).pin_memory()
+                    slot["off_dev"] = torch.empty(sum(counts), dtype=torch.int64, device=device)
+                    for t in (slot["dev"], slot["off_dev"]):
+                        t.record_stream(compute)
+                    slot["key"] = key
+                    slot["out"] = {}
+                slot["off_host"].copy_(torch.tensor(offs, dtype=torch.int64))
+                slot["src"] = list(recordings)  # keeps pinned sources alive until their asynchronous copies have run
+                if self.resampling:
+                    self._stage_raw(slot, recordings, n_in, lengths, seg_len, device, compute)
+                else:
+                    # the DMA engine does the layout: every recording goes straight from the caller's (pinned) buffer to
+                    # its place in the flat device buffer -- no host-side repacking; the zero padding is a device memset
+                    base = 0
+                    for r, sl in zip(recordings, seg_len):
+                        slot["dev"][base:base + r.numel()].copy_(r, non_blocking=True)
+                        if r.numel() < sl:
+                            slot["dev"][base + r.numel():base + sl].zero_()
+                        base += sl
                 slot["off_dev"].copy_(slot["off_host"], non_blocking=True)
             compute.wait_stream(cs)
             with torch.no_grad():
+                if self.resampling:
+                    engine.resample(slot["raw"], self.channels, slot["rs_dev"], len(recordings), max(lengths), plan,
+                                    slot["dev"])
                 out = packed.forward_windows(slot["dev"], window_samples, 0, len(offs), micro_batch=micro_batch,
                                              variant=variant, offsets=slot["off_dev"])
                 results = []
@@ -193,6 +262,29 @@ class HostStreamer:
         self.calls += 1
         self.pending.append((slot, results, len(recordings)))
         return self.calls - 1
+
+    def _stage_raw(self, slot, recordings, n_in, n_out, seg_len, device, compute):
+        """Copy stream, resampling call: the raw recordings go as they are into one device staging buffer (DMA from
+        the caller's pinned buffers), each recording's padding past its n_out resampled samples is zeroed, and the
+        sed_resample table (raw frame offset, n_in, padded-layout offset, n_out) goes up."""
+        C, dtype = self.channels, recordings[0].dtype
+        total_in = int(n_in.sum()) * C
+        if slot.get("raw") is None or slot["raw"].numel() < total_in or slot["raw"].dtype != dtype:
+            slot["raw"] = torch.empty(max(total_in, 1), dtype=dtype, device=device)
+            slot["raw"].record_stream(compute)
+        seg = np.array(seg_len, np.int64)
+        n_out = np.array(n_out, np.int64)
+        table = np.stack([np.cumsum(n_in) - n_in, n_in, np.cumsum(seg) - seg, n_out], 1)
+        slot["rs_host"] = torch.from_numpy(table).pin_memory()
+        slot["rs_dev"] = slot["rs_host"].to(device, non_blocking=True)
+        slot["rs_dev"].record_stream(compute)
+        base = 0
+        for r, n in zip(recordings, n_in.tolist()):
+            slot["raw"][base:base + n * C].copy_(r.reshape(-1), non_blocking=True)
+            base += n * C
+        for b, n, sl in zip(table[:, 2].tolist(), n_out.tolist(), seg_len):
+            if n < sl:
+                slot["dev"][b + n:b + sl].zero_()
 
     def result(self):
         """Merged frames of the oldest queued call: list of [1, total_frames, classes] CPU tensors, one per recording
@@ -286,6 +378,28 @@ def _plan_live_push(sids, n_samples, windows_run, frames_out, lens, src, closing
     return ticks, np.concatenate(offsets), rows_per_stream, base, n_rows, n_entries, ev_total, (n0, k_run, f_ret)
 
 
+def _plan_live_resample(rs, sids, n_in, n_samples, windows_run, frames_out, lens, src, closing, *geometry):
+    """_plan_live_push for streams that arrive at another rate: `lens` / `src` are input frames and `n_in` the input
+    frames before the push; `rs` is the engine.ResamplePlan.  The planner itself runs unchanged on model-rate counts --
+    before close, the outputs whose whole filter support has arrived (rs.n_out_live); at close, the whole resampled
+    length -- and each of its ingest rows becomes a sed_live_resample row (slot, j0, outputs, chunk frame or -1, n_prev,
+    n_end).  Returns (the planner's result with the rows replaced, history table, input frames after the push)."""
+    n_end = n_in + lens
+    n_out = rs.n_out(n_end) if closing else rs.n_out_live(n_end)
+    out_lens = n_out - n_samples
+    out_src = np.cumsum(out_lens) - out_lens
+    plan = _plan_live_push(sids, n_samples, windows_run, frames_out, out_lens, out_src, closing, *geometry)
+    at = {int(s): j for j, s in enumerate(sids)}
+    ticks = []
+    for ing, tab, sel, n_win, span in plan[0]:
+        j = np.array([at[int(s)] for s in ing[:, 0]], np.int64)
+        rows = np.stack([ing[:, 0], ing[:, 3], ing[:, 2], np.where(ing[:, 1] >= 0, src[j], -1), n_in[j], n_end[j]], 1)
+        ticks.append((rows.reshape(-1, 6), tab, sel, n_win, span))
+    fed = lens > 0
+    hist = np.stack([sids, src, n_in, lens], 1)[fed]
+    return (ticks,) + plan[1:], hist, n_end
+
+
 class LiveStreamer:
     """Live detection on many streams at once: audio is pushed as it arrives, every window that becomes ready in any
     stream runs in ONE batch, and each push returns the frames and events that have become final.
@@ -294,9 +408,15 @@ class LiveStreamer:
       * frames: the concatenation of all returned `frames` equals predict_framewise(model, rec, ...)[0] bit for bit;
       * events: label by label, the concatenation of all returned `events` equals frame_prediction_to_event_prediction
         on that merged tensor, in the same order.
+    With `input_rate` other than `sample_rate`, or `channels` > 1, chunks are [n] or [n, channels] at input_rate
+    (`dtype` is their dtype) and `rec` is resample(everything pushed, input_rate, sample_rate, channels): each push
+    resamples on the device the model-rate samples whose whole filter support has arrived, reading earlier input from
+    a per-slot history ring (sed_live_resample), into a float32 arena.
     Timeliness:
       * window k runs in the push after which the stream holds (k + sample_duration) * sample_rate samples; window 0
-        also runs, zero padded, at close if it never ran (window_starts' rule);
+        also runs, zero padded, at close if it never ran (window_starts' rule).  When resampling, a model-rate sample
+        is held once the filter's look-ahead has arrived too: half / up input samples more (half = 64 * max(up, down)),
+        4 ms of input when downsampling 44.1 or 48 kHz, 8 ms for 8 kHz -> 16 kHz; the last samples come at close;
       * a frame is returned once no later window covers it and its avg_merge block can no longer become a tail block;
         for the shipped presets (frames_per_window 500 / 496, overlap interval <= 100) that is (k + 1) * oi frames after
         the push that ran window k.  The tail blocks, whose divisor depends on the final length, come at close;
@@ -312,9 +432,14 @@ class LiveStreamer:
     on several GPUs run one streamer per GPU."""
 
     def __init__(self, model, sample_rate, sample_duration=5, overlap_value=1, max_streams=4096, dtype=torch.int16,
-                 sed_params=None, device=None, labels=None):
+                 sed_params=None, device=None, labels=None, input_rate=None, channels=1):
         if dtype not in (torch.int16, torch.float32):
             raise ValueError("dtype must be torch.int16 or torch.float32")
+        self.channels = _check_channels(channels)
+        self.input_rate = int(sample_rate) if input_rate is None else int(input_rate)
+        self.resampling = self.input_rate != int(sample_rate) or self.channels != 1
+        if self.resampling and self.input_rate != int(sample_rate):
+            engine.resample_filter(self.input_rate, sample_rate)  # ValueError for a rate pair the filter refuses
         if device is None and not isinstance(model, engine.PackedModel):
             device = next(model.parameters()).device
         self.packed, self.micro_batch, self.variant = _resolve(model, device)
@@ -331,14 +456,20 @@ class LiveStreamer:
         self.ring_frames = (LIVE_TICK_SECONDS - 1) * self.oi + max(self.fpw, 100 * self.dur) + self.oi
         p = DEFAULT_SED_PARAMS if sed_params is None else sed_params
         with torch.cuda.device(self.device):
-            self.arena = torch.zeros(self.max_streams * 2 * self.ring, dtype=dtype, device=self.device)
+            self.arena = torch.zeros(self.max_streams * 2 * self.ring, dtype=torch.float32 if self.resampling else dtype,
+                                     device=self.device)
+            if self.resampling:
+                self.rs = engine.resample_plan(self.input_rate, self.sr, self.device)
+                self.H = self.rs.history_len()
+                self.hist = torch.zeros(self.max_streams * self.H, dtype=torch.float32, device=self.device)
             self.acc = torch.empty((self.max_streams, self.ring_frames, self.classes), dtype=torch.float32,
                                    device=self.device)
             self.ev_state = torch.zeros(self.max_streams * self.classes * capi.LIVE_EVENT_STATE_INTS,
                                         dtype=torch.int32, device=self.device)
             self.ev_params = engine.event_params(p["sed_high_threshold"], p.get("sed_low_threshold"), p["n_smooth"],
                                                  p["n_salt"], self.classes, self.device)
-        self.n_samples = np.zeros(self.max_streams, np.int64)
+        self.n_samples = np.zeros(self.max_streams, np.int64)  # at sample_rate
+        self.n_in = np.zeros(self.max_streams, np.int64)       # at input_rate (frames)
         self.windows_run = np.zeros(self.max_streams, np.int64)
         self.frames_out = np.zeros(self.max_streams, np.int64)
         self.is_open = np.zeros(self.max_streams, bool)
@@ -354,7 +485,7 @@ class LiveStreamer:
             raise RuntimeError("all %d streams are open" % self.max_streams)
         sid = int(free[0])
         self.is_open[sid] = True
-        self.n_samples[sid] = self.windows_run[sid] = self.frames_out[sid] = 0
+        self.n_samples[sid] = self.n_in[sid] = self.windows_run[sid] = self.frames_out[sid] = 0
         self.names[sid] = name if name is not None else "stream-%d" % sid
         return sid
 
@@ -365,15 +496,18 @@ class LiveStreamer:
 
     def push(self, items):
         """items: iterable of (sid, chunk), chunk a 1-D CPU (pinned preferred) or CUDA tensor of the streamer's dtype,
-        any length (several chunks of one stream are taken in order).  Returns {sid: {"first_frame", "frames",
-        "events"}} for every stream of the push: the newly final rows of its merged output (CPU float32
+        any length (several chunks of one stream are taken in order); [n] or [n, channels] when resampling.  Returns
+        {sid: {"first_frame", "frames", "events"}} for every stream of the push: the newly final rows of its merged output (CPU float32
         [n, classes], starting at frame `first_frame`) and its newly decided events."""
         chunks = {}
         for sid, chunk in items:
             sid = self._check_sid(sid)
             if not torch.is_tensor(chunk) or chunk.dtype != self.dtype:
                 raise TypeError("chunk for stream %d must be a %s tensor" % (sid, self.dtype))
-            if chunk.dim() != 1:
+            if self.resampling:
+                _frames(chunk, self.channels, "chunk for stream %d" % sid)
+                chunk = chunk.reshape(-1)  # interleaved frames
+            elif chunk.dim() != 1:
                 raise ValueError("chunk for stream %d must be 1-D, got shape %s" % (sid, tuple(chunk.shape)))
             chunks.setdefault(sid, []).append(chunk)
         sids = np.fromiter(chunks.keys(), np.int64, len(chunks))
@@ -392,7 +526,7 @@ class LiveStreamer:
     # ---- one push ----
     def _run(self, sids, parts, closing):
         S, W, C, oi, fpw, ncls = len(sids), self.W, self.ring, self.oi, self.fpw, self.classes
-        lens = np.fromiter((t.numel() for t in parts), np.int64, S)
+        lens = np.fromiter((t.numel() for t in parts), np.int64, S)  # samples (frames x channels when resampling)
         on_dev = np.fromiter((t.is_cuda for t in parts), bool, S)
         # audio layout in the staging buffer: host chunks first (one H2D copy), then device chunks
         order = np.concatenate([np.flatnonzero(~on_dev), np.flatnonzero(on_dev)])
@@ -400,9 +534,15 @@ class LiveStreamer:
         src[order] = np.concatenate([[0], np.cumsum(lens[order])[:-1]]) if S else []
         n_host = int(lens[~on_dev].sum())
         n_audio = int(lens.sum())
-        ticks, offsets, rows_per_stream, base, n_rows, n_entries, ev_total, counters = _plan_live_push(
-            sids, self.n_samples[sids], self.windows_run[sids], self.frames_out[sids], lens, src, closing, self.sr,
-            self.dur, W, C, oi, fpw, ncls, self.slack)
+        before = (self.n_samples[sids], self.windows_run[sids], self.frames_out[sids])
+        geometry = (closing, self.sr, self.dur, W, C, oi, fpw, ncls, self.slack)
+        if self.resampling:
+            ch = self.channels
+            plan, hist_tab, n_in_after = _plan_live_resample(self.rs, sids, self.n_in[sids], *before, lens // ch,
+                                                             src // ch, *geometry)
+        else:
+            plan = _plan_live_push(sids, *before, lens, src, *geometry)
+        ticks, offsets, rows_per_stream, base, n_rows, n_entries, ev_total, counters = plan
 
         # one pinned staging buffer, one host->device copy: audio, then the tables of every tick
         esz = 2 if self.dtype == torch.int16 else 4
@@ -411,6 +551,9 @@ class LiveStreamer:
         for ing, tab, _, _, _ in ticks:
             blobs += [ing.astype(np.int64), tab.astype(np.int32)]
         blobs += [offsets.astype(np.int64)]
+        i_off = len(blobs) - 1
+        if self.resampling:
+            blobs += [hist_tab.astype(np.int64)]
         pos, at = [], a16(n_audio * esz)
         for b in blobs:
             pos.append(at)
@@ -433,9 +576,15 @@ class LiveStreamer:
             frames = out[:n_rows * ncls].view(torch.float32).view(n_rows, ncls)
             events = out[n_rows * ncls:n_rows * ncls + 2 * ev_total]
             counts_all = out[n_rows * ncls + 2 * ev_total:]
-            off_all, e0, w0 = view(len(blobs) - 1, torch.int64), 0, 0
+            off_all, e0, w0 = view(i_off, torch.int64), 0, 0
             for j, (ing, tab, sel, n_win, span) in enumerate(ticks):
-                if len(ing):
+                if self.resampling:
+                    n_hist = len(hist_tab) if j == len(ticks) - 1 else 0  # history: after the push's last reads
+                    if len(ing) or n_hist:
+                        engine.live_resample(audio, self.channels, view(2 * j, torch.int64), len(ing),
+                                             int(ing[:, 2].max()) if len(ing) else 0, self.rs, C, self.arena,
+                                             self.hist, self.H, view(i_off + 1, torch.int64), n_hist)
+                elif len(ing):
                     engine.live_ingest(audio, view(2 * j, torch.int64), len(ing), int(ing[:, 2].max()), C, self.arena)
                 if not len(tab):
                     continue
@@ -457,6 +606,8 @@ class LiveStreamer:
         res = res_host[:out_words].clone()
 
         self.n_samples[sids], self.windows_run[sids], self.frames_out[sids] = counters
+        if self.resampling:
+            self.n_in[sids] = n_in_after
         fr = res[:n_rows * ncls].view(torch.float32).view(n_rows, ncls)
         ev = res[n_rows * ncls:n_rows * ncls + 2 * ev_total].numpy()
         cnt = res[n_rows * ncls + 2 * ev_total:].numpy().reshape(n_entries, ncls)
