@@ -49,14 +49,16 @@ const char* sed_last_error_string(void);
  *   window [n_fft] f32 (row 0 of the loaded conv_real kernel); twiddle [n_fft][2] f32 = exp(-2 pi i k / n_fft);
  *   banded mel matrix: for mel bin m the non-zero weights melW[mel_lo[m] .. mel_lo[m]+mel_len[m]) are stored at
  *   mel_val[mel_off[m] ..]; db_offset = 10*log10(max(amin, ref)); bn_scale/bn_shift [n_mels] or NULL;
- *   out [B, T, n_mels] f32 with T = L / hop + 1.  n_fft in {256, 512, 1024}. */
+ *   out [B, T, n_mels] f32 with T = L / hop + 1.  n_fft in {256, 512, 1024}.  The hop is bounded by the staging
+ *   buffers in shared memory (64 mel bands, float32 input: 1793 / 1642 / 1805 samples); a larger hop returns
+ *   SED_ERR_UNSUPPORTED with the limit in sed_last_error_string() and launches nothing. */
 int sed_frontend_logmel(const void* wave, int wave_dtype, int B, int L, long clip_stride, const long* clip_offset,
                         long total_len, int n_fft, int hop, const float* window, const float* twiddle, const int* mel_lo, const int* mel_len,
                         const int* mel_off, const float* mel_val, int n_mels, float amin, float db_offset, int is_log,
                         const float* bn_scale, const float* bn_shift, float* out, void* stream);
 
 /* Power spectrogram only.  Replaces Spectrogram.forward pytorch/stft.py:651-670 (power == 2).
- *   out [B, T, n_fft/2+1] f32 (the reference's [B,1,T,F] layout). */
+ *   out [B, T, n_fft/2+1] f32 (the reference's [B,1,T,F] layout).  Hop bound as for sed_frontend_logmel. */
 int sed_spectrogram_f32(const float* wave, int B, int L, int n_fft, int hop, const float* window,
                         const float* twiddle, float* out, void* stream);
 

@@ -48,8 +48,16 @@ int sed_frontend_logmel(const void* wave, int wave_dtype, int B, int L, long cli
   if (rc == SED_ERR_BAD_SHAPE)
     sed::set_error("sed_frontend_logmel: bad shape B=%d L=%d stride=%ld total=%ld n_fft=%d hop=%d", B, L, clip_stride,
                    total_len, n_fft, hop);
-  if (rc == SED_ERR_UNSUPPORTED)
-    sed::set_error("sed_frontend_logmel: n_fft=%d (256/512/1024) or wave_dtype=%d (0/1) unsupported", n_fft, wave_dtype);
+  if (rc == SED_ERR_UNSUPPORTED) {
+    const int max_hop = sed::frontend_max_hop(n_fft, wave_dtype, n_mels);
+    if (max_hop > 0 && hop > max_hop)
+      sed::set_error("sed_frontend_logmel: hop=%d too large: the staging buffers of a work item do not fit in shared "
+                     "memory (n_fft=%d, %s input, %d mel bands: hop <= %d)", hop, n_fft,
+                     wave_dtype == 1 ? "int16" : "float32", n_mels, max_hop);
+    else
+      sed::set_error("sed_frontend_logmel: n_fft=%d (256/512/1024) or wave_dtype=%d (0/1) unsupported", n_fft,
+                     wave_dtype);
+  }
   if (rc == SED_ERR_CUDA) sed::set_error("sed_frontend_logmel: %s", cudaGetErrorString(cudaGetLastError()));
   return rc;
 }
@@ -65,7 +73,14 @@ int sed_spectrogram_f32(const float* wave, int B, int L, int n_fft, int hop, con
   a.out = out; a.mode = 1;
   int rc = sed::frontend_launch(a, as_stream(stream));
   if (rc == SED_ERR_BAD_SHAPE) sed::set_error("sed_spectrogram_f32: bad shape B=%d L=%d n_fft=%d hop=%d", B, L, n_fft, hop);
-  if (rc == SED_ERR_UNSUPPORTED) sed::set_error("sed_spectrogram_f32: n_fft=%d unsupported (256/512/1024)", n_fft);
+  if (rc == SED_ERR_UNSUPPORTED) {
+    const int max_hop = sed::frontend_max_hop(n_fft, 0, 0);
+    if (max_hop > 0 && hop > max_hop)
+      sed::set_error("sed_spectrogram_f32: hop=%d too large: the staging buffers of a work item do not fit in shared "
+                     "memory (n_fft=%d: hop <= %d)", hop, n_fft, max_hop);
+    else
+      sed::set_error("sed_spectrogram_f32: n_fft=%d unsupported (256/512/1024)", n_fft);
+  }
   if (rc == SED_ERR_CUDA) sed::set_error("sed_spectrogram_f32: %s", cudaGetErrorString(cudaGetLastError()));
   return rc;
 }

@@ -335,6 +335,31 @@ __device__ __forceinline__ void fft_pass(float2 (&v)[N / R / 32][R], uint32_t ld
   if (!LAST) __syncwarp();
 }
 
+// A frame pair shares one complex FFT, and so its float32 rounding error: both spectra carry an error of the order of
+// eps * sqrt(N (E_a + E_b)), E = windowed energy of a frame.  A frame far quieter than its partner (the frame before an
+// onset after digital silence) reads its partner's error as signal: bands near its own level miss the log-mel
+// tolerance, and silent bands are not exactly 10 log10(amin).  When one frame's energy is below kSoloShare of its
+// partner's, that frame is transformed a second time with a zero partner (read from s_zero, n_fft zero samples behind
+// the staging buffers), at its own error scale, and that result replaces its output.
+// The energies are the sums of the power bins k < N/2 the split has computed (Parseval; the quiet frame's sum is its
+// energy plus the coupling error, far below kSoloShare of its partner's).  Where every lane's partial sums already meet
+// the share both ways, so do the totals: one vote skips the reduction for almost every pair.  The decision depends on
+// the pair's samples alone and is uniform over the LANES lanes of the transform (the vote covers the warp; an xor
+// butterfly leaves the same sums in every lane), so batch invariance and int16 == float32 hold; on real audio the
+// second transform is rare.  kSoloShare comes from the onset probe of tests/test_gpu_frontend_configs.py.
+// Returns 0 (no second transform), 1 (frame a alone) or 2 (frame b alone).
+constexpr float kSoloShare = 0x1p-20f;
+template <int LANES>
+__device__ __forceinline__ int solo_frame(float ea, float eb) {
+  if (!__any_sync(0xffffffffu, ea < kSoloShare * eb || eb < kSoloShare * ea)) return 0;
+#pragma unroll
+  for (int d = LANES / 2; d > 0; d >>= 1) {
+    ea += __shfl_xor_sync(0xffffffffu, ea, d);
+    eb += __shfl_xor_sync(0xffffffffu, eb, d);
+  }
+  return (ea < kSoloShare * eb) ? 1 : (eb < kSoloShare * ea) ? 2 : 0;
+}
+
 // byte address of pidx(j0(lane)) for the stores of a pass (see fft_pass); buf_addr is 128-byte aligned
 template <int R, int Ns>
 __device__ __forceinline__ uint32_t pass_store_base(uint32_t buf_addr, int lane) {
@@ -527,6 +552,7 @@ frontend_kernel(const TIn* __restrict__ wave, long clip_stride, const long* __re
   float2* s_bn = reinterpret_cast<float2*>(s_band + ((n_mels + 1) & ~1));  // [n_mels] bn0 (scale, shift)
   TIn* s_stage0 = reinterpret_cast<TIn*>(sp + frontend_fixed_smem<NFFT>(n_mels));  // 16-byte aligned (bulk copy)
   TIn* s_stage1 = reinterpret_cast<TIn*>(reinterpret_cast<uint8_t*>(s_stage0) + seg_bytes);
+  TIn* s_zero = reinterpret_cast<TIn*>(reinterpret_cast<uint8_t*>(s_stage1) + seg_bytes);  // [NFFT] (solo_frame)
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int chunks = (T + FPB - 1) / FPB;
@@ -548,6 +574,7 @@ frontend_kernel(const TIn* __restrict__ wave, long clip_stride, const long* __re
   for (int i = threadIdx.x; i < NFFT; i += blockDim.x) {
     s_win[i] = window[i];
     s_tw[i] = twiddle[i];
+    s_zero[i] = TIn(0);
   }
   int nseg = -1;
   if (MODE == 0) {
@@ -601,134 +628,150 @@ frontend_kernel(const TIn* __restrict__ wave, long clip_stride, const long* __re
       if (fa >= T) break;
       const TIn* seg_a = s_seg + (2 * pair) * hop;
       const TIn* seg_b = seg_a + hop;
-
-      // ---- 2 real frames -> 1 complex FFT of size NFFT (Stockham autosort); the last pass stays in registers ----
-      {
-        float2 v0[NFFT / R0 / 32][R0];
-        fft_pass<NFFT, R0, 1, true, false, TIn>(v0, ld_base, st_base0, tw0, s_tw, seg_a, seg_b, s_win, lane);
-      }
-      {
-        float2 v1[NFFT / R1 / 32][R1];
-        fft_pass<NFFT, R1, NS1, false, false, TIn>(v1, ld_base, st_base1, tw1, s_tw, seg_a, seg_b, s_win, lane);
-      }
-      float2 X[BPL2][R2];  // X[lane + 32 i] = X[i % BPL2][i / BPL2]
-      fft_pass<NFFT, R2, NS2, false, true, TIn>(X, ld_base, 0u, tw2, s_tw, seg_a, seg_b, s_win, lane);
-
-      // ---- split the two real spectra and take the power (stft.py:663).  Bin k = lane + 32 i (i < H) needs
-      //      Z[N - k]: slot NS - 1 - i of lane 32 - lane (one shuffle per component); lane 0 pairs with itself
-      //      (slot (NS - i) % NS).  The warp has passed the barrier behind the last pass's reads, so P2 can overwrite
-      //      the buffer. ----
-#pragma unroll
-      for (int i = 0; i < H; ++i) {
-        const float2 zk = X[i % BPL2][i / BPL2];
-        const float2 up = X[(NS - 1 - i) % BPL2][(NS - 1 - i) / BPL2];
-        float2 zn = make_float2(__shfl_sync(0xffffffffu, up.x, src_lane), __shfl_sync(0xffffffffu, up.y, src_lane));
-        if (lane == 0) zn = X[((NS - i) % NS) % BPL2][((NS - i) % NS) / BPL2];
-        // A = (zk + conj(zn)) / 2, B = (zk - conj(zn)) / 2i; the halves are folded into one exact scale by 1/4
-        const float ar = zk.x + zn.x, ai = zk.y - zn.y;
-        const float br = zk.y + zn.y, bi = zn.x - zk.x;
-        // (the log-mel path keeps 4 |.|^2 and carries the 1/4 in its mel weights)
-        constexpr float kQ = (MODE == 0) ? 1.0f : 0.25f;
-        P2[lane + 32 * i] = make_float2(kQ * fmaf(ai, ai, ar * ar), kQ * fmaf(bi, bi, br * br));
-      }
-      if (lane == 0) {  // Nyquist bin N / 2 = 32 H: its own partner, so A = re, B = im
-        constexpr float kN = (MODE == 0) ? 4.0f : 1.0f;
-        const float2 z = X[H % BPL2][H / BPL2];
-        P2[NFFT / 2] = make_float2(kN * z.x * z.x, kN * z.y * z.y);
-      }
-      __syncwarp();
-
       const bool has_b = fa + 1 < T;
-      if (MODE == 1) {
-        float* o = out + (static_cast<size_t>(b) * T + fa) * F;
-        for (int k = lane; k < F; k += 32) {
-          const float2 p = P2[k];
-          o[k] = p.x;
-          if (has_b) o[F + k] = p.y;
+      // rep 0 transforms the pair and writes both frames; rep 1 (warp-uniform, rare) transforms the frame solo_frame
+      // picked with a zero partner and writes that frame again (same lanes, same addresses: the later store wins).
+      int redo = 0;
+      for (int rep = 0;; ++rep) {
+        const int solo = redo;
+
+        // ---- 2 real frames -> 1 complex FFT of size NFFT (Stockham autosort); the last pass stays in registers ----
+        {
+          float2 v0[NFFT / R0 / 32][R0];
+          fft_pass<NFFT, R0, 1, true, false, TIn>(v0, ld_base, st_base0, tw0, s_tw, solo == 2 ? s_zero : seg_a,
+                                                  solo == 1 ? s_zero : seg_b, s_win, lane);
         }
-      } else {
-        float* o = out + (static_cast<size_t>(b) * T + fa) * n_mels;
-        // ---- mel projection, one lane per segment: SEG multiply-adds per round for both frames of the pair ----
-        if (rounds == RU) {  // the presets: every round unrolled, all loads in flight, RU independent chains per frame
-          float a0[RU], b0[RU];
-          const float2* Pm[RU];
+        {
+          float2 v1[NFFT / R1 / 32][R1];
+          fft_pass<NFFT, R1, NS1, false, false, TIn>(v1, ld_base, st_base1, tw1, s_tw, seg_a, seg_b, s_win, lane);
+        }
+        float2 X[BPL2][R2];  // X[lane + 32 i] = X[i % BPL2][i / BPL2]
+        fft_pass<NFFT, R2, NS2, false, true, TIn>(X, ld_base, 0u, tw2, s_tw, seg_a, seg_b, s_win, lane);
+
+        // ---- split the two real spectra and take the power (stft.py:663).  Bin k = lane + 32 i (i < H) needs
+        //      Z[N - k]: slot NS - 1 - i of lane 32 - lane (one shuffle per component); lane 0 pairs with itself
+        //      (slot (NS - i) % NS).  The warp has passed the barrier behind the last pass's reads, so P2 can overwrite
+        //      the buffer. ----
+        float ea = 0.0f, eb = 0.0f;  // frame energies for solo_frame
 #pragma unroll
-          for (int r = 0; r < RU; ++r) {
-            Pm[r] = P2 + s_seglo[32 * r + lane];
-            a0[r] = 0.0f;
-            b0[r] = 0.0f;
-          }
-#pragma unroll
-          for (int i = 0; i < SEG; ++i) {
-#pragma unroll
-            for (int r = 0; r < RU; ++r) {
-              const float2 p = Pm[r][i];
-              const float w = s_segw[(r * SEG + i) * 32 + lane];
-              a0[r] = fmaf(p.x, w, a0[r]);
-              b0[r] = fmaf(p.y, w, b0[r]);
-            }
-          }
-#pragma unroll
-          for (int r = 0; r < RU; ++r) part[32 * r + lane] = make_float2(a0[r], b0[r]);
-        } else {
-          for (int r = 0; r < rounds; ++r) {
-            const float2* Pm = P2 + s_seglo[32 * r + lane];
-            const float* wr = s_segw + r * (SEG * 32) + lane;
-            float a0 = 0.0f, b0 = 0.0f;
-#pragma unroll
-            for (int i = 0; i < SEG; ++i) {
-              const float2 p = Pm[i];
-              const float w = wr[32 * i];
-              a0 = fmaf(p.x, w, a0);
-              b0 = fmaf(p.y, w, b0);
-            }
-            part[32 * r + lane] = make_float2(a0, b0);
-          }
+        for (int i = 0; i < H; ++i) {
+          const float2 zk = X[i % BPL2][i / BPL2];
+          const float2 up = X[(NS - 1 - i) % BPL2][(NS - 1 - i) / BPL2];
+          float2 zn = make_float2(__shfl_sync(0xffffffffu, up.x, src_lane), __shfl_sync(0xffffffffu, up.y, src_lane));
+          if (lane == 0) zn = X[((NS - i) % NS) % BPL2][((NS - i) % NS) / BPL2];
+          // A = (zk + conj(zn)) / 2, B = (zk - conj(zn)) / 2i; the halves are folded into one exact scale by 1/4
+          const float ar = zk.x + zn.x, ai = zk.y - zn.y;
+          const float br = zk.y + zn.y, bi = zn.x - zk.x;
+          // (the log-mel path keeps 4 |.|^2 and carries the 1/4 in its mel weights)
+          constexpr float kQ = (MODE == 0) ? 1.0f : 0.25f;
+          const float pa = kQ * fmaf(ai, ai, ar * ar), pb = kQ * fmaf(bi, bi, br * br);
+          P2[lane + 32 * i] = make_float2(pa, pb);
+          ea += pa;
+          eb += pb;
+        }
+        const bool wr_a = rep == 0 || solo == 1;
+        const bool wr_b = has_b && (rep == 0 || solo == 2);
+        if (lane == 0) {  // Nyquist bin N / 2 = 32 H: its own partner, so A = re, B = im
+          constexpr float kN = (MODE == 0) ? 4.0f : 1.0f;
+          const float2 z = X[H % BPL2][H / BPL2];
+          P2[NFFT / 2] = make_float2(kN * z.x * z.x, kN * z.y * z.y);
         }
         __syncwarp();
-        for (int m = lane; m < n_mels; m += 32) {
-          float ya = 0.0f, yb = 0.0f;
-          if (rounds > 0) {
-            const int first = s_band[m] & 0xffff, np = s_band[m] >> 16;
-            const float2* pm = part + first;
-            // ascending segments: the summation order is fixed.  The first NP_UNROLL are predicated (no loop for the
-            // reference's presets), wider bands continue in a loop.
+
+        if (MODE == 1) {
+          float* o = out + (static_cast<size_t>(b) * T + fa) * F;
+          for (int k = lane; k < F; k += 32) {
+            const float2 p = P2[k];
+            if (wr_a) o[k] = p.x;
+            if (wr_b) o[F + k] = p.y;
+          }
+        } else {
+          float* o = out + (static_cast<size_t>(b) * T + fa) * n_mels;
+          // ---- mel projection, one lane per segment: SEG multiply-adds per round for both frames of the pair ----
+          if (rounds == RU) {  // the presets: every round unrolled, all loads in flight, RU independent chains per frame
+            float a0[RU], b0[RU];
+            const float2* Pm[RU];
 #pragma unroll
-            for (int j = 0; j < NP_UNROLL; ++j) {
-              if (j < np) {
+            for (int r = 0; r < RU; ++r) {
+              Pm[r] = P2 + s_seglo[32 * r + lane];
+              a0[r] = 0.0f;
+              b0[r] = 0.0f;
+            }
+#pragma unroll
+            for (int i = 0; i < SEG; ++i) {
+#pragma unroll
+              for (int r = 0; r < RU; ++r) {
+                const float2 p = Pm[r][i];
+                const float w = s_segw[(r * SEG + i) * 32 + lane];
+                a0[r] = fmaf(p.x, w, a0[r]);
+                b0[r] = fmaf(p.y, w, b0[r]);
+              }
+            }
+#pragma unroll
+            for (int r = 0; r < RU; ++r) part[32 * r + lane] = make_float2(a0[r], b0[r]);
+          } else {
+            for (int r = 0; r < rounds; ++r) {
+              const float2* Pm = P2 + s_seglo[32 * r + lane];
+              const float* wr = s_segw + r * (SEG * 32) + lane;
+              float a0 = 0.0f, b0 = 0.0f;
+#pragma unroll
+              for (int i = 0; i < SEG; ++i) {
+                const float2 p = Pm[i];
+                const float w = wr[32 * i];
+                a0 = fmaf(p.x, w, a0);
+                b0 = fmaf(p.y, w, b0);
+              }
+              part[32 * r + lane] = make_float2(a0, b0);
+            }
+          }
+          __syncwarp();
+          for (int m = lane; m < n_mels; m += 32) {
+            float ya = 0.0f, yb = 0.0f;
+            if (rounds > 0) {
+              const int first = s_band[m] & 0xffff, np = s_band[m] >> 16;
+              const float2* pm = part + first;
+              // ascending segments: the summation order is fixed.  The first NP_UNROLL are predicated (no loop for the
+              // reference's presets), wider bands continue in a loop.
+#pragma unroll
+              for (int j = 0; j < NP_UNROLL; ++j) {
+                if (j < np) {
+                  const float2 t = pm[j];
+                  ya += t.x;
+                  yb += t.y;
+                }
+              }
+              for (int j = NP_UNROLL; j < np; ++j) {
                 const float2 t = pm[j];
                 ya += t.x;
                 yb += t.y;
               }
+            } else {
+              const float2* Pm = P2 + mel_lo[m];
+              const float* mv = mel_val + mel_off[m];
+              const int len = mel_len[m];
+              for (int i = 0; i < len; ++i) {
+                const float2 p = Pm[i];
+                const float w = 0.25f * __ldg(mv + i);
+                ya = fmaf(p.x, w, ya);
+                yb = fmaf(p.y, w, yb);
+              }
             }
-            for (int j = NP_UNROLL; j < np; ++j) {
-              const float2 t = pm[j];
-              ya += t.x;
-              yb += t.y;
+            if (is_log) {  // stft.py:726-727
+              ya = power_to_db(ya, amin, db_offset, db_floor);
+              yb = power_to_db(yb, amin, db_offset, db_floor);
             }
-          } else {
-            const float2* Pm = P2 + mel_lo[m];
-            const float* mv = mel_val + mel_off[m];
-            const int len = mel_len[m];
-            for (int i = 0; i < len; ++i) {
-              const float2 p = Pm[i];
-              const float w = 0.25f * __ldg(mv + i);
-              ya = fmaf(p.x, w, ya);
-              yb = fmaf(p.y, w, yb);
-            }
+            const float2 sc = s_bn[m];  // models.py:642-644 (identity when no bn0 is fused)
+            ya = fmaf(ya, sc.x, sc.y);
+            yb = fmaf(yb, sc.x, sc.y);
+            if (wr_a) o[m] = ya;
+            if (wr_b) o[n_mels + m] = yb;
           }
-          if (is_log) {  // stft.py:726-727
-            ya = power_to_db(ya, amin, db_offset, db_floor);
-            yb = power_to_db(yb, amin, db_offset, db_floor);
-          }
-          const float2 sc = s_bn[m];  // models.py:642-644 (identity when no bn0 is fused)
-          ya = fmaf(ya, sc.x, sc.y);
-          yb = fmaf(yb, sc.x, sc.y);
-          o[m] = ya;
-          if (has_b) o[n_mels + m] = yb;
         }
+        __syncwarp();
+        if (rep == 1) break;
+        redo = solo_frame<32>(ea, eb);  // after the epilogue: off the critical path of the pair
+        if (redo == 0) break;
       }
-      __syncwarp();
     }
   }
 }
@@ -804,6 +847,7 @@ frontend2_kernel(const TIn* __restrict__ wave, long clip_stride, const long* __r
   float2* s_bn = reinterpret_cast<float2*>(s_band + ((n_mels + 1) & ~1));
   TIn* s_stage0 = reinterpret_cast<TIn*>(sp + frontend_fixed_smem<NFFT>(n_mels, WARPS * BUF, TW_ELEMS));
   TIn* s_stage1 = reinterpret_cast<TIn*>(reinterpret_cast<uint8_t*>(s_stage0) + seg_bytes);
+  TIn* s_zero = reinterpret_cast<TIn*>(reinterpret_cast<uint8_t*>(s_stage1) + seg_bytes);  // [NFFT] (solo_frame)
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int chunks = (T + FPB - 1) / FPB;
@@ -822,7 +866,10 @@ frontend2_kernel(const TIn* __restrict__ wave, long clip_stride, const long* __r
   if (item < items)
     cur_bulk = stage_segment<NFFT, FPB, TIn>(s_stage0, &s_bar[0], wave, clip_stride, clip_offset, total_len, L, hop,
                                              seg_len, item, chunks, aligned != 0);
-  for (int i = threadIdx.x; i < NFFT; i += blockDim.x) s_win[i] = window[i];
+  for (int i = threadIdx.x; i < NFFT; i += blockDim.x) {
+    s_win[i] = window[i];
+    s_zero[i] = TIn(0);
+  }
   int nseg = -1;
   if (MODE == 0) {
     for (int i = threadIdx.x; i < n_mels; i += blockDim.x)
@@ -873,173 +920,193 @@ frontend2_kernel(const TIn* __restrict__ wave, long clip_stride, const long* __r
     for (int grp = warp; grp < FPB / GROUP; grp += WARPS) {
       const int fa0 = f_base + GROUP * grp;  // first frame of this warp's 2 T frames
       if (fa0 >= T) break;
-
-      // ---- pass A: per transform the RA-point DFT over n1 of the windowed frame pair, twiddle, store to row (t, k1) ----
-      {
-        float wv[RA];
+      // rep 0 transforms the T pairs and writes every frame; rep 1 (warp-uniform, rare) transforms again the frames
+      // solo_frame picked, each with a zero partner, and writes those frames again (same lanes, same addresses)
+      // (two bits per transform: 1 = frame a alone, 2 = frame b alone, 0 = no output in rep 1)
+      unsigned redo = 0;
+      for (int rep = 0;; ++rep) {
+        // ---- pass A: per transform the RA-point DFT over n1 of the windowed frame pair, twiddle, store to row (t, k1) ----
+        {
+          float wv[RA];
 #pragma unroll
-        for (int n1 = 0; n1 < RA; ++n1) wv[n1] = s_win[lane + 32 * n1];
+          for (int n1 = 0; n1 < RA; ++n1) wv[n1] = s_win[lane + 32 * n1];
 #pragma unroll
-        for (int t = 0; t < NT; ++t) {
-          const TIn* seg_a = s_seg + (GROUP * grp + 2 * t) * hop + lane;
-          const TIn* seg_b = seg_a + hop;
-          float2 v[RA];
+          for (int t = 0; t < NT; ++t) {
+            const unsigned solo = (redo >> (2 * t)) & 3u;  // 0 in rep 0
+            const TIn* seg_a = (solo == 2 ? s_zero : s_seg + (GROUP * grp + 2 * t) * hop) + lane;
+            const TIn* seg_b = solo == 1 ? s_zero + lane : s_seg + (GROUP * grp + 2 * t + 1) * hop + lane;
+            float2 v[RA];
 #pragma unroll
-          for (int n1 = 0; n1 < RA; ++n1)
-            v[n1] = make_float2(wv[n1] * load_sample(seg_a + 32 * n1), wv[n1] * load_sample(seg_b + 32 * n1));
-          butterfly<RA>(v);
+            for (int n1 = 0; n1 < RA; ++n1)
+              v[n1] = make_float2(wv[n1] * load_sample(seg_a + 32 * n1), wv[n1] * load_sample(seg_b + 32 * n1));
+            butterfly<RA>(v);
 #pragma unroll
-          for (int k1 = 0; k1 < RA; ++k1) {
-            const int row = t * RA + k1;
-            const float2 y = (k1 == 0) ? v[0] : cmul(v[k1], C2::TW_SMEM ? s_tw[(k1 - 1) * 32 + lane] : twa[k1 - 1]);
-            sts_f2((st_base ^ static_cast<uint32_t>(8 * (row & 15))) + static_cast<uint32_t>(256 * row), y);
-          }
-        }
-      }
-      __syncwarp();
-
-      // ---- pass B: 32-point DFT over n2 of this lane's row ----
-      float2 X[32];
-#pragma unroll
-      for (int n2 = 0; n2 < 32; ++n2)
-        X[n2] = lds_f2((ld_base ^ static_cast<uint32_t>(8 * (n2 & 15))) + static_cast<uint32_t>(8 * (n2 & 16)));
-      __syncwarp();  // every row has been read: the buffer can take the power spectra
-      butterfly<32>(X);
-
-      // ---- split the two real spectra and take the power (stft.py:663): bin k = k1 + RA k2, k2 < 16 ----
-#pragma unroll
-      for (int k2 = 0; k2 < 16; ++k2) {
-        const float2 zk = X[k2];
-        const float2 up = X[31 - k2];
-        float2 zn = make_float2(__shfl_sync(0xffffffffu, up.x, src_lane), __shfl_sync(0xffffffffu, up.y, src_lane));
-        if (k1b == 0) zn = X[(32 - k2) & 31];
-        const float ar = zk.x + zn.x, ai = zk.y - zn.y;
-        const float br = zk.y + zn.y, bi = zn.x - zk.x;
-        constexpr float kQ = (MODE == 0) ? 1.0f : 0.25f;  // the log-mel path carries the 1/4 in its mel weights
-        P2own[RA * k2] = make_float2(kQ * fmaf(ai, ai, ar * ar), kQ * fmaf(bi, bi, br * br));
-      }
-      if (k1b == 0) {  // Nyquist bin N / 2 = RA * 16
-        constexpr float kN = (MODE == 0) ? 4.0f : 1.0f;
-        const float2 z = X[16];
-        P2own[RA * 16] = make_float2(kN * z.x * z.x, kN * z.y * z.y);
-      }
-      __syncwarp();
-
-      if (MODE == 1) {
-#pragma unroll
-        for (int t = 0; t < NT; ++t) {
-          const int fa = fa0 + 2 * t;
-          if (fa >= T) break;
-          const float2* P2 = buf + C2::p2_base(t);
-          float* o = out + (static_cast<size_t>(b) * T + fa) * F;
-          for (int k = lane; k < F; k += 32) {
-            const float2 p = P2[k];
-            o[k] = p.x;
-            if (fa + 1 < T) o[F + k] = p.y;
-          }
-        }
-      } else {
-        // ---- mel projection, one lane per segment; seglo and weights are loaded once for the T transforms ----
-        if (rounds == RU) {
-          float a0[RU][NT], b0[RU][NT];
-          int slo[RU];
-#pragma unroll
-          for (int r = 0; r < RU; ++r) {
-            slo[r] = s_seglo[32 * r + lane];
-#pragma unroll
-            for (int t = 0; t < NT; ++t) a0[r][t] = b0[r][t] = 0.0f;
-          }
-#pragma unroll
-          for (int i = 0; i < SEG; ++i) {
-#pragma unroll
-            for (int r = 0; r < RU; ++r) {
-              const float w = s_segw[(r * SEG + i) * 32 + lane];
-#pragma unroll
-              for (int t = 0; t < NT; ++t) {
-                const float2 p = buf[C2::p2_base(t) + slo[r] + i];
-                a0[r][t] = fmaf(p.x, w, a0[r][t]);
-                b0[r][t] = fmaf(p.y, w, b0[r][t]);
-              }
+            for (int k1 = 0; k1 < RA; ++k1) {
+              const int row = t * RA + k1;
+              const float2 y = (k1 == 0) ? v[0] : cmul(v[k1], C2::TW_SMEM ? s_tw[(k1 - 1) * 32 + lane] : twa[k1 - 1]);
+              sts_f2((st_base ^ static_cast<uint32_t>(8 * (row & 15))) + static_cast<uint32_t>(256 * row), y);
             }
-          }
-#pragma unroll
-          for (int r = 0; r < RU; ++r)
-#pragma unroll
-            for (int t = 0; t < NT; ++t) buf[C2::p2_base(t) + F + 32 * r + lane] = make_float2(a0[r][t], b0[r][t]);
-        } else {
-          for (int r = 0; r < rounds; ++r) {
-            const int slo = s_seglo[32 * r + lane];
-            const float* wr = s_segw + r * (SEG * 32) + lane;
-            float a0[NT], b0[NT];
-#pragma unroll
-            for (int t = 0; t < NT; ++t) a0[t] = b0[t] = 0.0f;
-#pragma unroll
-            for (int i = 0; i < SEG; ++i) {
-              const float w = wr[32 * i];
-#pragma unroll
-              for (int t = 0; t < NT; ++t) {
-                const float2 p = buf[C2::p2_base(t) + slo + i];
-                a0[t] = fmaf(p.x, w, a0[t]);
-                b0[t] = fmaf(p.y, w, b0[t]);
-              }
-            }
-#pragma unroll
-            for (int t = 0; t < NT; ++t) buf[C2::p2_base(t) + F + 32 * r + lane] = make_float2(a0[t], b0[t]);
           }
         }
         __syncwarp();
-        for (int m = lane; m < n_mels; m += 32) {
-          int first = 0, np = 0;
-          if (rounds > 0) {
-            first = s_band[m] & 0xffff;
-            np = s_band[m] >> 16;
-          }
-          const float2 sc = s_bn[m];  // models.py:642-644 (identity when no bn0 is fused)
+
+        // ---- pass B: 32-point DFT over n2 of this lane's row ----
+        float2 X[32];
+#pragma unroll
+        for (int n2 = 0; n2 < 32; ++n2)
+          X[n2] = lds_f2((ld_base ^ static_cast<uint32_t>(8 * (n2 & 15))) + static_cast<uint32_t>(8 * (n2 & 16)));
+        __syncwarp();  // every row has been read: the buffer can take the power spectra
+        butterfly<32>(X);
+
+        // ---- split the two real spectra and take the power (stft.py:663): bin k = k1 + RA k2, k2 < 16 ----
+        float ea = 0.0f, eb = 0.0f;  // frame energies for solo_frame
+#pragma unroll
+        for (int k2 = 0; k2 < 16; ++k2) {
+          const float2 zk = X[k2];
+          const float2 up = X[31 - k2];
+          float2 zn = make_float2(__shfl_sync(0xffffffffu, up.x, src_lane), __shfl_sync(0xffffffffu, up.y, src_lane));
+          if (k1b == 0) zn = X[(32 - k2) & 31];
+          const float ar = zk.x + zn.x, ai = zk.y - zn.y;
+          const float br = zk.y + zn.y, bi = zn.x - zk.x;
+          constexpr float kQ = (MODE == 0) ? 1.0f : 0.25f;  // the log-mel path carries the 1/4 in its mel weights
+          const float pa = kQ * fmaf(ai, ai, ar * ar), pb = kQ * fmaf(bi, bi, br * br);
+          P2own[RA * k2] = make_float2(pa, pb);
+          ea += pa;
+          eb += pb;
+        }
+        if (k1b == 0) {  // Nyquist bin N / 2 = RA * 16
+          constexpr float kN = (MODE == 0) ? 4.0f : 1.0f;
+          const float2 z = X[16];
+          P2own[RA * 16] = make_float2(kN * z.x * z.x, kN * z.y * z.y);
+        }
+        __syncwarp();
+
+        if (MODE == 1) {
 #pragma unroll
           for (int t = 0; t < NT; ++t) {
             const int fa = fa0 + 2 * t;
             if (fa >= T) break;
-            float ya = 0.0f, yb = 0.0f;
-            if (rounds > 0) {
-              const float2* pm = buf + C2::p2_base(t) + F + first;
-              // ascending segments: the summation order is fixed
+            const unsigned rt = (redo >> (2 * t)) & 3u;
+            const bool wr_a = rep == 0 || rt == 1;
+            const bool wr_b = fa + 1 < T && (rep == 0 || rt == 2);
+            const float2* P2 = buf + C2::p2_base(t);
+            float* o = out + (static_cast<size_t>(b) * T + fa) * F;
+            for (int k = lane; k < F; k += 32) {
+              const float2 p = P2[k];
+              if (wr_a) o[k] = p.x;
+              if (wr_b) o[F + k] = p.y;
+            }
+          }
+        } else {
+          // ---- mel projection, one lane per segment; seglo and weights are loaded once for the T transforms ----
+          if (rounds == RU) {
+            float a0[RU][NT], b0[RU][NT];
+            int slo[RU];
 #pragma unroll
-              for (int j = 0; j < NP_UNROLL; ++j) {
-                if (j < np) {
+            for (int r = 0; r < RU; ++r) {
+              slo[r] = s_seglo[32 * r + lane];
+#pragma unroll
+              for (int t = 0; t < NT; ++t) a0[r][t] = b0[r][t] = 0.0f;
+            }
+#pragma unroll
+            for (int i = 0; i < SEG; ++i) {
+#pragma unroll
+              for (int r = 0; r < RU; ++r) {
+                const float w = s_segw[(r * SEG + i) * 32 + lane];
+#pragma unroll
+                for (int t = 0; t < NT; ++t) {
+                  const float2 p = buf[C2::p2_base(t) + slo[r] + i];
+                  a0[r][t] = fmaf(p.x, w, a0[r][t]);
+                  b0[r][t] = fmaf(p.y, w, b0[r][t]);
+                }
+              }
+            }
+#pragma unroll
+            for (int r = 0; r < RU; ++r)
+#pragma unroll
+              for (int t = 0; t < NT; ++t) buf[C2::p2_base(t) + F + 32 * r + lane] = make_float2(a0[r][t], b0[r][t]);
+          } else {
+            for (int r = 0; r < rounds; ++r) {
+              const int slo = s_seglo[32 * r + lane];
+              const float* wr = s_segw + r * (SEG * 32) + lane;
+              float a0[NT], b0[NT];
+#pragma unroll
+              for (int t = 0; t < NT; ++t) a0[t] = b0[t] = 0.0f;
+#pragma unroll
+              for (int i = 0; i < SEG; ++i) {
+                const float w = wr[32 * i];
+#pragma unroll
+                for (int t = 0; t < NT; ++t) {
+                  const float2 p = buf[C2::p2_base(t) + slo + i];
+                  a0[t] = fmaf(p.x, w, a0[t]);
+                  b0[t] = fmaf(p.y, w, b0[t]);
+                }
+              }
+#pragma unroll
+              for (int t = 0; t < NT; ++t) buf[C2::p2_base(t) + F + 32 * r + lane] = make_float2(a0[t], b0[t]);
+            }
+          }
+          __syncwarp();
+          for (int m = lane; m < n_mels; m += 32) {
+            int first = 0, np = 0;
+            if (rounds > 0) {
+              first = s_band[m] & 0xffff;
+              np = s_band[m] >> 16;
+            }
+            const float2 sc = s_bn[m];  // models.py:642-644 (identity when no bn0 is fused)
+#pragma unroll
+            for (int t = 0; t < NT; ++t) {
+              const int fa = fa0 + 2 * t;
+              if (fa >= T) break;
+              float ya = 0.0f, yb = 0.0f;
+              if (rounds > 0) {
+                const float2* pm = buf + C2::p2_base(t) + F + first;
+                // ascending segments: the summation order is fixed
+#pragma unroll
+                for (int j = 0; j < NP_UNROLL; ++j) {
+                  if (j < np) {
+                    const float2 s = pm[j];
+                    ya += s.x;
+                    yb += s.y;
+                  }
+                }
+                for (int j = NP_UNROLL; j < np; ++j) {
                   const float2 s = pm[j];
                   ya += s.x;
                   yb += s.y;
                 }
+              } else {
+                const float2* Pm = buf + C2::p2_base(t) + mel_lo[m];
+                const float* mv = mel_val + mel_off[m];
+                const int len = mel_len[m];
+                for (int i = 0; i < len; ++i) {
+                  const float2 p = Pm[i];
+                  const float w = 0.25f * __ldg(mv + i);
+                  ya = fmaf(p.x, w, ya);
+                  yb = fmaf(p.y, w, yb);
+                }
               }
-              for (int j = NP_UNROLL; j < np; ++j) {
-                const float2 s = pm[j];
-                ya += s.x;
-                yb += s.y;
+              if (is_log) {  // stft.py:726-727
+                ya = power_to_db(ya, amin, db_offset, db_floor);
+                yb = power_to_db(yb, amin, db_offset, db_floor);
               }
-            } else {
-              const float2* Pm = buf + C2::p2_base(t) + mel_lo[m];
-              const float* mv = mel_val + mel_off[m];
-              const int len = mel_len[m];
-              for (int i = 0; i < len; ++i) {
-                const float2 p = Pm[i];
-                const float w = 0.25f * __ldg(mv + i);
-                ya = fmaf(p.x, w, ya);
-                yb = fmaf(p.y, w, yb);
-              }
+              ya = fmaf(ya, sc.x, sc.y);
+              yb = fmaf(yb, sc.x, sc.y);
+              const unsigned rt = (redo >> (2 * t)) & 3u;
+              float* o = out + (static_cast<size_t>(b) * T + fa) * n_mels;
+              if (rep == 0 || rt == 1) o[m] = ya;
+              if (fa + 1 < T && (rep == 0 || rt == 2)) o[n_mels + m] = yb;
             }
-            if (is_log) {  // stft.py:726-727
-              ya = power_to_db(ya, amin, db_offset, db_floor);
-              yb = power_to_db(yb, amin, db_offset, db_floor);
-            }
-            ya = fmaf(ya, sc.x, sc.y);
-            yb = fmaf(yb, sc.x, sc.y);
-            float* o = out + (static_cast<size_t>(b) * T + fa) * n_mels;
-            o[m] = ya;
-            if (fa + 1 < T) o[n_mels + m] = yb;
           }
         }
+        __syncwarp();
+        if (rep == 1) break;
+        // after the epilogue: off the critical path; lanes t RA .. t RA + RA - 1 hold transform t
+        const unsigned r = static_cast<unsigned>(solo_frame<RA>(ea, eb));
+#pragma unroll
+        for (int t = 0; t < NT; ++t) redo |= __shfl_sync(0xffffffffu, r, t * RA) << (2 * t);
+        if (redo == 0) break;
       }
-      __syncwarp();
     }
   }
 }
@@ -1063,7 +1130,8 @@ __global__ void logmel_rows_kernel(const float* __restrict__ spec, long rows, in
   }
 }
 
-// claim counters of the launches in flight (one per launch, round robin; zeroed on the launch's stream)
+// claim counters of the launches in flight (one per launch, round robin; zeroed on the launch's stream).  More than 64
+// front-end launches in flight on one device at once would share a counter.
 __device__ int g_frontend_work_counters[64];
 static std::atomic<unsigned> g_frontend_launch_seq{0};
 
@@ -1075,8 +1143,12 @@ static std::atomic<unsigned> g_frontend_launch_seq{0};
 // At 512 the two-pass kernel executes 7 % fewer instructions and 19 % fewer shared-memory wavefronts than the
 // three-pass one (profiles/r02_ncu_full_frontend_two_pass_512.json) and only draws level with it: at 12 warps per SM it
 // has a quarter less latency hiding than the three-pass kernel's 16.
-// The two-pass kernel needs 8 KB of buffer per warp; where its shared memory does not fit (large hop) the three-pass
-// kernel takes over.  -DSED_FE_TWO_PASS(N)=1 builds a library that uses the two-pass kernel at every size.
+// The staging buffers grow with the hop, (FPB - 1) * hop + n_fft samples each, and bound the hop (frontend_max_hop);
+// beyond it the launch is refused with SED_ERR_UNSUPPORTED.  With 64 mel bands and float32 input: n_fft 1024 two-pass
+// up to hop 1805 (the three-pass kernel, twice the frames per item and 12 warps of buffers, only up to 552), n_fft 512
+// up to 1642, n_fft 256 up to 1793.  So in the shipped build the three-pass fallback below never fits where the
+// two-pass kernel does not; it serves -DSED_FE_TWO_PASS(N)=1, a library that uses the two-pass kernel at every size,
+// where at 256 / 512 the three-pass kernel's smaller buffers do reach larger hops.
 #ifndef SED_FE_TWO_PASS
 #define SED_FE_TWO_PASS(NFFT) ((NFFT) == 1024)
 #endif
@@ -1089,19 +1161,38 @@ struct FrontKernel<NFFT, TIn, MODE, true> {
   static auto get() { return frontend2_kernel<NFFT, TIn, MODE>; }
 };
 
+// Dynamic shared memory of one kernel variant: 128 bytes of alignment slack, the fixed tables, two staging buffers and
+// n_fft zero samples (s_zero).
+template <int NFFT, typename TIn, bool TWO_PASS>
+struct FrontSmem {
+  static constexpr int WARPS = TWO_PASS ? Front2Cfg<NFFT>::WARPS : FrontCfg<NFFT>::WARPS;
+  static constexpr int FPB = TWO_PASS ? Front2Cfg<NFFT>::template fpb<TIn>() : FrontCfg<NFFT>::template fpb<TIn>();
+  static constexpr int BUF_ELEMS = TWO_PASS ? Front2Cfg<NFFT>::WARPS * Front2Cfg<NFFT>::BUF : FrontCfg<NFFT>::WARPS * NFFT;
+  static constexpr int TW_ELEMS = (TWO_PASS && !Front2Cfg<NFFT>::TW_SMEM) ? 0 : NFFT;
+  // 227 KB per block hold the dynamic AND the static shared memory (claim slots and mbarriers, 32 bytes; 64 set aside)
+  static constexpr long LIMIT = 227 * 1024 - 64;
+  static long fixed(int n_mels) {
+    return 128 + static_cast<long>(frontend_fixed_smem<NFFT>(n_mels > 0 ? n_mels : 0, BUF_ELEMS, TW_ELEMS)) +
+           NFFT * static_cast<long>(sizeof(TIn));
+  }
+  static long bytes(int hop, int n_mels) {
+    const long seg_len = static_cast<long>(FPB - 1) * hop + NFFT;
+    return fixed(n_mels) + 2 * ((seg_len * static_cast<long>(sizeof(TIn)) + 15) & ~15L);
+  }
+  static int max_hop(int n_mels) {  // largest hop with bytes(hop) <= LIMIT
+    const long seg_len = (((LIMIT - fixed(n_mels)) / 2) & ~15L) / static_cast<long>(sizeof(TIn));
+    return seg_len < NFFT ? 0 : static_cast<int>((seg_len - NFFT) / (FPB - 1));
+  }
+};
+
 template <int NFFT, typename TIn, int MODE, bool TWO_PASS>
 static int launch_frontend_v(const FrontendArgs& a, cudaStream_t stream) {
-  constexpr int WARPS = TWO_PASS ? Front2Cfg<NFFT>::WARPS : FrontCfg<NFFT>::WARPS;
-  constexpr int FPB = TWO_PASS ? Front2Cfg<NFFT>::template fpb<TIn>() : FrontCfg<NFFT>::template fpb<TIn>();
-  constexpr int BUF_ELEMS = TWO_PASS ? Front2Cfg<NFFT>::WARPS * Front2Cfg<NFFT>::BUF : FrontCfg<NFFT>::WARPS * NFFT;
+  using S = FrontSmem<NFFT, TIn, TWO_PASS>;
+  constexpr int WARPS = S::WARPS, FPB = S::FPB;
   auto kernel = FrontKernel<NFFT, TIn, MODE, TWO_PASS>::get();
   const int seg_len = (FPB - 1) * a.hop + NFFT;
-  const int seg_bytes = (seg_len * static_cast<int>(sizeof(TIn)) + 15) & ~15;
-  constexpr int TW_ELEMS = (TWO_PASS && !Front2Cfg<NFFT>::TW_SMEM) ? 0 : NFFT;
-  const size_t smem = 128 +
-                      static_cast<size_t>(frontend_fixed_smem<NFFT>(a.n_mels > 0 ? a.n_mels : 0, BUF_ELEMS, TW_ELEMS)) +
-                      2 * static_cast<size_t>(seg_bytes);
-  if (smem > 227 * 1024) return SED_ERR_UNSUPPORTED;
+  if (S::bytes(a.hop, a.n_mels) > S::LIMIT) return SED_ERR_UNSUPPORTED;
+  const size_t smem = static_cast<size_t>(S::bytes(a.hop, a.n_mels));
   static int sm_count = 0;
   if (sm_count == 0) {
     int dev = 0;
@@ -1142,6 +1233,24 @@ static int launch_frontend_t(const FrontendArgs& a, cudaStream_t stream) {
     if (rc != SED_ERR_UNSUPPORTED) return rc;
   }
   return launch_frontend_v<NFFT, TIn, MODE, false>(a, stream);
+}
+
+template <int NFFT, typename TIn>
+static int max_hop_t(int n_mels) {
+  const int three = FrontSmem<NFFT, TIn, false>::max_hop(n_mels);
+  const int two = FrontSmem<NFFT, TIn, true>::max_hop(n_mels);
+  return SED_FE_TWO_PASS(NFFT) ? (two > three ? two : three) : three;
+}
+
+int frontend_max_hop(int n_fft, int wave_dtype, int n_mels) {
+  const bool i16 = wave_dtype == 1;
+  if (wave_dtype != 0 && wave_dtype != 1) return 0;
+  switch (n_fft) {
+    case 256: return i16 ? max_hop_t<256, short>(n_mels) : max_hop_t<256, float>(n_mels);
+    case 512: return i16 ? max_hop_t<512, short>(n_mels) : max_hop_t<512, float>(n_mels);
+    case 1024: return i16 ? max_hop_t<1024, short>(n_mels) : max_hop_t<1024, float>(n_mels);
+    default: return 0;
+  }
 }
 
 template <int NFFT>

@@ -28,6 +28,8 @@ struct FrontendArgs {
   int mode;  // 0 = log-mel [B,T,n_mels], 1 = power spectrogram [B,T,F]
 };
 int frontend_launch(const FrontendArgs& a, cudaStream_t stream);
+// largest hop whose staging buffers fit in shared memory (0: n_fft or wave_dtype not built); n_mels 0 = power mode
+int frontend_max_hop(int n_fft, int wave_dtype, int n_mels);
 int logmel_rows_launch(const float* spec, long rows, int F, const int* mel_lo, const int* mel_len, const int* mel_off,
                        const float* mel_val, int n_mels, float amin, float db_offset, int is_log, float* out,
                        cudaStream_t stream);
