@@ -150,8 +150,8 @@ int main(int argc, char** argv) {
   const int n_fft = argc > 4 ? atoi(argv[4]) : 512;
   const int hop = argc > 5 ? atoi(argv[5]) : 160;
   const int F = n_fft / 2 + 1, M = 64, DT = SED_DTYPE_F16;
-  if (sed_abi_version() != 12) {
-    fprintf(stderr, "libsed_b200 ABI %d, this driver was written against 12\n", sed_abi_version());
+  if (sed_abi_version() != 13) {
+    fprintf(stderr, "libsed_b200 ABI %d, this driver was written against 13\n", sed_abi_version());
     return 1;
   }
   load_weights(argv[1]);
@@ -265,13 +265,13 @@ int main(int argc, char** argv) {
   /* ---- the forward pass: every call is asynchronous on the (default) stream ---- */
   CHECK_SED(sed_frontend_logmel(wave, 0, B, L, L, NULL, (long)B * L, n_fft, hop, window, twiddle, mel_lo, mel_len, mel_off,
                                 mel_val, M, amin, db_offset, 1, bn0_s, bn0_b, logmel, NULL));
-  CHECK_SED(sed_conv_block1(logmel, B, T, 64, w1_scaled, c11_b, wp[0], cs[0], cb[0], p1, 1, DT, NULL));
-  CHECK_SED(sed_conv3x3_bn_relu(p1, B, H1, 32, 64, wp[1], cs[1], cb[1], 128, SED_CONV_STORE, a2, NULL, 0, 0, DT, 2, NULL));
-  CHECK_SED(sed_conv3x3_bn_relu(a2, B, H1, 32, 128, wp[2], cs[2], cb[2], 128, SED_CONV_POOL, p2, NULL, 0, 0, DT, 2, NULL));
-  CHECK_SED(sed_conv3x3_bn_relu(p2, B, H2, 16, 128, wp[3], cs[3], cb[3], 256, SED_CONV_STORE, a3, NULL, 0, 0, DT, 2, NULL));
-  CHECK_SED(sed_conv3x3_bn_relu(a3, B, H2, 16, 256, wp[4], cs[4], cb[4], 256, SED_CONV_POOL, p3, NULL, 0, 0, DT, 2, NULL));
-  CHECK_SED(sed_conv3x3_bn_relu(p3, B, Tp, 8, 256, wp[5], cs[5], cb[5], 512, SED_CONV_STORE, a4, NULL, 0, 0, DT, 2, NULL));
-  CHECK_SED(sed_conv3x3_bn_relu(a4, B, Tp, 8, 512, wp[6], cs[6], cb[6], 512, SED_CONV_FREQMEAN, feat, NULL, 1, Bp, DT, 2,
+  CHECK_SED(sed_conv_block1(logmel, B, T, 64, w1_scaled, c11_b, wp[0], cs[0], cb[0], p1, DT, NULL));
+  CHECK_SED(sed_conv3x3_bn_relu(p1, B, H1, 32, 64, wp[1], cs[1], cb[1], 128, SED_CONV_STORE, a2, NULL, 0, 0, DT, NULL));
+  CHECK_SED(sed_conv3x3_bn_relu(a2, B, H1, 32, 128, wp[2], cs[2], cb[2], 128, SED_CONV_POOL, p2, NULL, 0, 0, DT, NULL));
+  CHECK_SED(sed_conv3x3_bn_relu(p2, B, H2, 16, 128, wp[3], cs[3], cb[3], 256, SED_CONV_STORE, a3, NULL, 0, 0, DT, NULL));
+  CHECK_SED(sed_conv3x3_bn_relu(a3, B, H2, 16, 256, wp[4], cs[4], cb[4], 256, SED_CONV_POOL, p3, NULL, 0, 0, DT, NULL));
+  CHECK_SED(sed_conv3x3_bn_relu(p3, B, Tp, 8, 256, wp[5], cs[5], cb[5], 512, SED_CONV_STORE, a4, NULL, 0, 0, DT, NULL));
+  CHECK_SED(sed_conv3x3_bn_relu(a4, B, Tp, 8, 512, wp[6], cs[6], cb[6], 512, SED_CONV_FREQMEAN, feat, NULL, 1, Bp, DT,
                                 NULL));
   CHECK_SED(sed_linear(feat, (long)Tp * Bp, 512, wih16, bih, 1536, 0, gi, NULL, 1, DT, NULL));
   CHECK_SED(sed_bigru(gi, whh16, bhh, B, Tp, gru_out, gru_ws, DT, NULL));

@@ -76,7 +76,7 @@ int sed_conv_first_f32(const float* x, int NB, int H, int W, const float* w9, co
                        const float* shift, void* out, int dtype, void* stream);
 
 /* 3x3 stride-1 pad-1 convolution (no bias) + folded BatchNorm + ReLU [+ 2x2 avg-pool | + mean over W]
- * on the tcgen05 tensor cores.  Replaces ConvBlock.forward pytorch/models.py:125-141 (one conv each
+ * on the tcgen05 tensor cores, one kernel per layer on CTA pairs (cta_group::2).  Replaces ConvBlock.forward pytorch/models.py:125-141 (one conv each
  * call) and torch.mean(x, dim=3) models.py:668.
  *   x [NB, H, W, cin] NHWC 16-bit; wpacked [cout][9][cin] 16-bit (tap = 3*kh + kw);
  *   scale/shift [cout] f32; out NHWC 16-bit: [NB,H,W,cout] | [NB,H/2,W/2,cout] | [NB,H,cout];
@@ -84,22 +84,20 @@ int sed_conv_first_f32(const float* x, int NB, int H, int W, const float* w9, co
  *   out_stride_n / out_stride_h (FREQMEAN only; 0, 0 = default H, 1): output row of (image n, row h) is
  *   n*out_stride_n + h*out_stride_h -- (1, batch) writes the features time-major for the GRU.
  *   Supported (cin,cout,mode): (64,64,POOL) (64,128,STORE) (128,128,POOL) (128,256,STORE)
- *   (256,256,POOL) (256,512,STORE) (512,512,FREQMEAN).
- *   variant 0 = single-CTA haloed-patch operand reuse, 1 = one TMA box per tap, 2 = CTA pairs (cta_group::2). */
+ *   (256,256,POOL) (256,512,STORE) (512,512,FREQMEAN). */
 int sed_conv3x3_bn_relu(const void* x, int NB, int H, int W, int cin, const void* wpacked, const float* scale,
                         const float* shift, int cout, int mode, void* out, void* out_f32, long out_stride_n,
-                        long out_stride_h, int dtype, int variant, void* stream);
+                        long out_stride_h, int dtype, void* stream);
 
 /* conv_block1 in one kernel: conv1 (1 -> 64) + bn1 + ReLU computed on the fly as the tensor-core operand of
  * conv2 (64 -> 64) + bn2 + ReLU + 2x2 avg-pool.  Replaces ConvBlock.forward pytorch/models.py:125-141 for
- * conv_block1 (models.py:663); the [NB, H, W, 64] intermediate never reaches HBM.
- *   producer 0: conv1 on the CUDA cores (packed f32x2 FMAs) -- measured slower (1.07 ms per 148 clips) than
- *   sed_conv_first_f32 + sed_conv3x3_bn_relu (0.28 + 0.53 ms); producer 1: conv1 as a split-fp16 tensor-core GEMM
- *   whose accumulators are drained from TMEM into conv2's shared-memory operand.
+ * conv_block1 (models.py:663); the [NB, H, W, 64] intermediate never reaches HBM.  conv1 runs as a split-fp16
+ *   tensor-core GEMM (float32-grade, as sed_conv_first_f32) whose accumulators are drained from TMEM into conv2's
+ *   shared-memory operand.
  *   x [NB, H, W] f32 (log-mel after bn0, W % 16 == 0); w1_scaled [64][9] f32 = conv1 weights x folded bn1 scale;
  *   shift1 [64] folded bn1 shift; w2packed [64][9][64] 16-bit; scale2/shift2 [64]; out [NB, H/2, W/2, 64] 16-bit. */
 int sed_conv_block1(const float* x, int NB, int H, int W, const float* w1_scaled, const float* shift1,
-                    const void* w2packed, const float* scale2, const float* shift2, void* out, int producer, int dtype,
+                    const void* w2packed, const float* scale2, const float* shift2, void* out, int dtype,
                     void* stream);
 
 /* out[M, N] = a[M, K] * w[N, K]^T + bias (optional ReLU) on the tensor cores; K in {256, 512},

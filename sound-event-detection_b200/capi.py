@@ -40,8 +40,8 @@ SIGNATURES = {
     "sed_spectrogram_f32": ([_p, _i, _i, _i, _i, _p, _p, _p, _p], _i),
     "sed_logmel_rows_f32": ([_p, _l, _i, _p, _p, _p, _p, _i, _f, _f, _i, _p, _p], _i),
     "sed_conv_first_f32": ([_p, _i, _i, _i, _p, _p, _p, _p, _i, _p], _i),
-    "sed_conv3x3_bn_relu": ([_p, _i, _i, _i, _i, _p, _p, _p, _i, _i, _p, _p, _l, _l, _i, _i, _p], _i),
-    "sed_conv_block1": ([_p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _i, _i, _p], _i),
+    "sed_conv3x3_bn_relu": ([_p, _i, _i, _i, _i, _p, _p, _p, _i, _i, _p, _p, _l, _l, _i, _p], _i),
+    "sed_conv_block1": ([_p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _i, _p], _i),
     "sed_fold_bn": ([_p, _p, _p, _p, _i, _d, _p, _p, _p], _i),
     "sed_pack_conv3x3": ([_p, _i, _i, _p, _i, _p], _i),
     "sed_pack_conv_first": ([_p, _p, _p, _p], _i),

@@ -7,7 +7,7 @@
 
 #include "sed_kernels.h"
 
-#define SED_ABI_VERSION 12
+#define SED_ABI_VERSION 13
 
 static inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
@@ -168,22 +168,18 @@ int sed_conv_first_f32(const float* x, int NB, int H, int W, const float* w9, co
 
 int sed_conv3x3_bn_relu(const void* x, int NB, int H, int W, int cin, const void* wpacked, const float* scale,
                         const float* shift, int cout, int mode, void* out, void* out_f32, long out_stride_n,
-                        long out_stride_h, int dtype, int variant, void* stream) {
+                        long out_stride_h, int dtype, void* stream) {
   SED_REQUIRE(x); SED_REQUIRE(wpacked); SED_REQUIRE(scale); SED_REQUIRE(shift); SED_REQUIRE(out);
-  if (variant < 0 || variant > 2) {
-    sed::set_error("sed_conv3x3_bn_relu: variant must be 0 (patch), 1 (per-tap) or 2 (CTA pairs)");
-    return SED_ERR_UNSUPPORTED;
-  }
   return sed::conv3x3_launch(x, NB, H, W, cin, wpacked, scale, shift, cout, mode, out, out_f32, out_stride_n,
-                             out_stride_h, dtype, variant, as_stream(stream));
+                             out_stride_h, dtype, as_stream(stream));
 }
 
 int sed_conv_block1(const float* x, int NB, int H, int W, const float* w1_scaled, const float* shift1,
-                    const void* w2packed, const float* scale2, const float* shift2, void* out, int producer, int dtype,
+                    const void* w2packed, const float* scale2, const float* shift2, void* out, int dtype,
                     void* stream) {
   SED_REQUIRE(x); SED_REQUIRE(w1_scaled); SED_REQUIRE(shift1); SED_REQUIRE(w2packed); SED_REQUIRE(scale2);
   SED_REQUIRE(shift2); SED_REQUIRE(out);
-  return sed::conv_block1_launch(x, NB, H, W, w1_scaled, shift1, w2packed, scale2, shift2, out, producer, dtype,
+  return sed::conv_block1_launch(x, NB, H, W, w1_scaled, shift1, w2packed, scale2, shift2, out, dtype,
                                  as_stream(stream));
 }
 

@@ -104,15 +104,6 @@ SED_DEVICE_INLINE void tma_load_2d(void* dst, const CUtensorMap* m, uint64_t* ba
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-SED_DEVICE_INLINE void tma_load_4d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2,
-                                   int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
-      "[%2];" ::"r"(smem_u32(dst)),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-
 SED_DEVICE_INLINE void tma_store_4d(const CUtensorMap* m, const void* src, int c0, int c1, int c2, int c3) {
   asm volatile(
       "cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
@@ -232,20 +223,6 @@ SED_DEVICE_INLINE void mbar_arrive_remote_light(uint64_t* bar, uint32_t cta_rank
       "}\n" ::"r"(smem_u32(bar)),
       "r"(cta_rank)
       : "memory");
-}
-// packed f32x2 arithmetic (sm_100): two float32 FMAs per instruction on a 64-bit register pair
-SED_DEVICE_INLINE unsigned long long pack_f32x2(float lo, float hi) {
-  unsigned long long r;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-  return r;
-}
-SED_DEVICE_INLINE void unpack_f32x2(unsigned long long v, float& lo, float& hi) {
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-SED_DEVICE_INLINE unsigned long long ffma2(unsigned long long a, unsigned long long b, unsigned long long c) {
-  unsigned long long d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  return d;
 }
 SED_DEVICE_INLINE uint32_t cluster_ctarank() {
   uint32_t r;

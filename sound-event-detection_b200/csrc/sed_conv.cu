@@ -260,9 +260,6 @@ int conv_first_launch(const float* x, int NB, int H, int W, const float* w9, con
 }
 
 // ---------------------------------------------------------------------------------------------
-// tcgen05 conv / linear launch
-// ---------------------------------------------------------------------------------------------
-// ---------------------------------------------------------------------------------------------
 // conv_block1 as ONE tensor-core kernel (engine variant 4): conv1 (1 -> 64 channels) runs as a split-fp16 tcgen05 GEMM
 // (K = 9 taps padded to 16, hi*hi + lo*hi + hi*lo, float32-grade like conv_first_umma_kernel) on the 18 x 10 pixel halo
 // patch of every conv2 tile; its accumulators are drained from TMEM through bn1 + ReLU straight into the swizzled
@@ -647,28 +644,21 @@ conv_block1_tc_kernel(const __grid_constant__ CUtensorMap tmB, const ConvParams 
 }
 
 
-template <typename T, int CIN, int BN, int NT, bool BRES, bool PATCH, int EPI, int SA, int SB>
-static int launch_cfg(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmO, const ConvParams& p,
-                      cudaStream_t stream) {
-  using Cfg = ConvCfg<CIN, BN, NT, BRES, PATCH, EPI, SA, SB>;
-  auto kern = conv_umma_kernel<T, CIN, BN, NT, BRES, PATCH, EPI, SA, SB>;
+// ---------------------------------------------------------------------------------------------
+// tcgen05 conv / linear launch
+// ---------------------------------------------------------------------------------------------
+template <typename T, int CIN, int BN, int NT, int SA, int SB>
+static int launch_cfg(const CUtensorMap& tmA, const CUtensorMap& tmB, const ConvParams& p, cudaStream_t stream) {
+  using Cfg = ConvCfg<CIN, BN, NT, SA, SB>;
+  auto kern = conv_umma_kernel<T, CIN, BN, NT, SA, SB>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
   if (e != cudaSuccess) {
     set_error("cudaFuncSetAttribute(smem=%d): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e));
     return SED_ERR_CUDA;
   }
-  const int groups = (p.num_tiles + NT - 1) / NT;
-  int grid;
-  if (BRES) {
-    int per_slice = num_sms() / p.nslices;
-    if (per_slice > groups) per_slice = groups;
-    if (per_slice < 1) per_slice = 1;
-    grid = per_slice * p.nslices;
-  } else {
-    const long items = static_cast<long>(groups) * p.nslices;
-    grid = items < num_sms() ? static_cast<int>(items) : num_sms();
-  }
-  kern<<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, stream>>>(tmA, tmB, tmO, p);
+  const long items = static_cast<long>((p.num_tiles + NT - 1) / NT) * p.nslices;
+  const int grid = items < num_sms() ? static_cast<int>(items) : num_sms();
+  kern<<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, stream>>>(tmA, tmB, tmA, p);  // the third map is not read
   e = cudaGetLastError();
   if (e != cudaSuccess) {
     set_error("conv_umma launch: %s", cudaGetErrorString(e));
@@ -677,12 +667,11 @@ static int launch_cfg(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUte
   return SED_OK;
 }
 
-template <typename T, int CIN, int BN, int EPI, int SA, int ACC, bool BRES, int NT, int SB, int EG = 1,
-          bool FUSE1 = false>
+template <typename T, int CIN, int BN, int EPI, int SA, int ACC, bool BRES, int NT, int SB>
 static int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmO, const ConvParams& p,
                        cudaStream_t stream) {
-  using Cfg = Conv2Cfg<CIN, BN, EPI, SA, ACC, BRES, NT, SB, EG, FUSE1>;
-  auto kern = conv_umma2_kernel<T, CIN, BN, EPI, SA, ACC, BRES, NT, SB, EG, FUSE1>;
+  using Cfg = Conv2Cfg<CIN, BN, EPI, SA, ACC, BRES, NT, SB>;
+  auto kern = conv_umma2_kernel<T, CIN, BN, EPI, SA, ACC, BRES, NT, SB>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
   if (e != cudaSuccess) {
     set_error("cudaFuncSetAttribute(pair, smem=%d): %s", Cfg::SMEM_BYTES, cudaGetErrorString(e));
@@ -711,43 +700,24 @@ static int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUt
 
 template <typename T>
 static int conv3x3_dispatch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmO, ConvParams& p,
-                            int cin, int cout, int mode, int variant, cudaStream_t stream) {
-  // (cin, cout, mode) are the seven tensor-core layers of Cnn_9layers (SURVEY.md 8a, row a7).
-  // variant 2: CTA-pair (cta_group::2) kernels for the weight-stationary layers
-  if (variant == 2) {
-    if (cin == 64 && cout == 64 && mode == EPI_POOL) { p.nslices = 1; return launch_pair<T, 64, 64, EPI_POOL, 6, 4, true, 1, 1>(tmA, tmB, tmO, p, stream); }
-    if (cin == 64 && cout == 128 && mode == EPI_STORE) { p.nslices = 1; return launch_pair<T, 64, 128, EPI_STORE, 4, 4, true, 1, 1>(tmA, tmB, tmO, p, stream); }
-    if (cin == 128 && cout == 128 && mode == EPI_POOL) { p.nslices = 1; return launch_pair<T, 128, 128, EPI_POOL, 3, 2, true, 1, 1>(tmA, tmB, tmO, p, stream); }
-    if (cin == 128 && cout == 256 && mode == EPI_STORE) { p.nslices = 2; return launch_pair<T, 128, 128, EPI_STORE, 2, 2, true, 1, 1>(tmA, tmB, tmO, p, stream); }
-    // streamed weights: each CTA loads half of every 256-row weight block, two pixel tiles per CTA share it
-    if (cin == 256 && cout == 256 && mode == EPI_POOL) { p.nslices = 2; return launch_pair<T, 256, 128, EPI_POOL, 2, 2, false, 2, 6>(tmA, tmB, tmO, p, stream); }
-    if (cin == 256 && cout == 512 && mode == EPI_STORE) { p.nslices = 4; return launch_pair<T, 256, 128, EPI_STORE, 2, 2, false, 2, 6>(tmA, tmB, tmO, p, stream); }
-    if (cin == 512 && cout == 512 && mode == EPI_FREQMEAN) { p.nslices = 4; return launch_pair<T, 512, 128, EPI_FREQMEAN, 2, 2, false, 2, 6>(tmA, tmB, tmO, p, stream); }
-    variant = 0;
-  }
-#define SED_CASE(CIN_, COUT_, MODE_, BN_, NT_, BRES_, SA_P, SB_P, SA_T, SB_T)                                     \
-  if (cin == CIN_ && cout == COUT_ && mode == MODE_) {                                                             \
-    p.nslices = COUT_ / BN_;                                                                                       \
-    if (variant == 0)                                                                                              \
-      return launch_cfg<T, CIN_, BN_, NT_, BRES_, true, MODE_, SA_P, SB_P>(tmA, tmB, tmO, p, stream);              \
-    return launch_cfg<T, CIN_, BN_, NT_, BRES_, false, MODE_, SA_T, SB_T>(tmA, tmB, tmO, p, stream);               \
-  }
-  //        cin cout mode           BN  NT bres  SA/SB patch  SA/SB tap
-  SED_CASE(64, 64, EPI_POOL, 64, 1, true, 4, 1, 6, 1)       // conv_block1.conv2 : weights resident (72 KB)
-  SED_CASE(64, 128, EPI_STORE, 128, 1, true, 2, 1, 2, 1)    // conv_block2.conv1 : weights resident (144 KB)
-  SED_CASE(128, 128, EPI_POOL, 64, 1, true, 3, 1, 4, 1)     // conv_block2.conv2 : 2 Cout slices resident
-  SED_CASE(128, 256, EPI_STORE, 64, 1, true, 2, 1, 3, 1)    // conv_block3.conv1 : 4 Cout slices resident
-  SED_CASE(256, 256, EPI_POOL, 256, 2, false, 2, 3, 3, 3)   // conv_block3.conv2 : weights streamed, 2 tiles/CTA
-  SED_CASE(256, 512, EPI_STORE, 256, 2, false, 2, 3, 2, 3)  // conv_block4.conv1
-  SED_CASE(512, 512, EPI_FREQMEAN, 256, 2, false, 2, 3, 3, 3)  // conv_block4.conv2 (+ freq mean, models.py:668)
-#undef SED_CASE
+                            int cin, int cout, int mode, cudaStream_t stream) {
+  // (cin, cout, mode) are the seven tensor-core layers of Cnn_9layers (SURVEY.md 8a, row a7), all on CTA pairs.
+  // weights resident: each CTA of a pair holds half of the BN rows of its Cout slice
+  if (cin == 64 && cout == 64 && mode == EPI_POOL) { p.nslices = 1; return launch_pair<T, 64, 64, EPI_POOL, 6, 4, true, 1, 1>(tmA, tmB, tmO, p, stream); }
+  if (cin == 64 && cout == 128 && mode == EPI_STORE) { p.nslices = 1; return launch_pair<T, 64, 128, EPI_STORE, 4, 4, true, 1, 1>(tmA, tmB, tmO, p, stream); }
+  if (cin == 128 && cout == 128 && mode == EPI_POOL) { p.nslices = 1; return launch_pair<T, 128, 128, EPI_POOL, 3, 2, true, 1, 1>(tmA, tmB, tmO, p, stream); }
+  if (cin == 128 && cout == 256 && mode == EPI_STORE) { p.nslices = 2; return launch_pair<T, 128, 128, EPI_STORE, 2, 2, true, 1, 1>(tmA, tmB, tmO, p, stream); }
+  // streamed weights: each CTA loads half of every 256-row weight block, two pixel tiles per CTA share it
+  if (cin == 256 && cout == 256 && mode == EPI_POOL) { p.nslices = 2; return launch_pair<T, 256, 128, EPI_POOL, 2, 2, false, 2, 6>(tmA, tmB, tmO, p, stream); }
+  if (cin == 256 && cout == 512 && mode == EPI_STORE) { p.nslices = 4; return launch_pair<T, 256, 128, EPI_STORE, 2, 2, false, 2, 6>(tmA, tmB, tmO, p, stream); }
+  if (cin == 512 && cout == 512 && mode == EPI_FREQMEAN) { p.nslices = 4; return launch_pair<T, 512, 128, EPI_FREQMEAN, 2, 2, false, 2, 6>(tmA, tmB, tmO, p, stream); }  // + freq mean, models.py:668
   set_error("conv3x3: unsupported layer (cin=%d, cout=%d, mode=%d)", cin, cout, mode);
   return SED_ERR_UNSUPPORTED;
 }
 
 int conv3x3_launch(const void* x, int NB, int H, int W, int cin, const void* wpacked, const float* scale,
                    const float* shift, int cout, int mode, void* out, void* out_f32, long out_sn, long out_sh,
-                   int dtype, int variant, cudaStream_t stream) {
+                   int dtype, cudaStream_t stream) {
   if (NB <= 0 || H <= 0 || W <= 0 || (W % 8) != 0 || (cin % 64) != 0) {
     set_error("conv3x3: bad shape NB=%d H=%d W=%d cin=%d", NB, H, W, cin);
     return SED_ERR_BAD_SHAPE;
@@ -764,21 +734,14 @@ int conv3x3_launch(const void* x, int NB, int H, int W, int cin, const void* wpa
   {
     const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)W, (uint64_t)H, (uint64_t)NB};
     const uint64_t str[3] = {(uint64_t)cin * 2, (uint64_t)W * cin * 2, (uint64_t)H * W * cin * 2};
-    const uint32_t box_patch[4] = {64, 10, 18, 1};
-    const uint32_t box_tap[4] = {64, 8, 16, 1};
-    int rc = make_map(&tmA, dtype, 4, const_cast<void*>(x), dims, str, variant != 1 ? box_patch : box_tap);
+    const uint32_t box[4] = {64, 10, 18, 1};  // one haloed 16 x 8 pixel tile
+    int rc = make_map(&tmA, dtype, 4, const_cast<void*>(x), dims, str, box);
     if (rc) return rc;
   }
-  int bn = 0;
-  if (cin == 64 && cout == 64) bn = 64;
-  else if (cin == 64 && cout == 128) bn = 128;
-  else if (cin == 128) bn = 64;
-  else bn = 256;
-  if (variant == 2) bn = (cout == 64) ? 32 : 64;  // each CTA of a pair loads half of the N rows
   {
     const uint64_t dims[2] = {(uint64_t)9 * cin, (uint64_t)cout};
     const uint64_t str[1] = {(uint64_t)9 * cin * 2};
-    const uint32_t box[2] = {64, (uint32_t)bn};
+    const uint32_t box[2] = {64, cout == 64 ? 32u : 64u};  // each CTA of a pair loads half of the BN = 64 | 128 rows
     int rc = make_map(&tmB, dtype, 2, const_cast<void*>(wpacked), dims, str, box);
     if (rc) return rc;
   }
@@ -816,21 +779,16 @@ int conv3x3_launch(const void* x, int NB, int H, int W, int cin, const void* wpa
     p.dbg = e ? atoi(e) : 0;
   }
 #endif
-  if (dtype == 0) return conv3x3_dispatch<__half>(tmA, tmB, tmO, p, cin, cout, mode, variant, stream);
-  if (dtype == 1) return conv3x3_dispatch<__nv_bfloat16>(tmA, tmB, tmO, p, cin, cout, mode, variant, stream);
+  if (dtype == 0) return conv3x3_dispatch<__half>(tmA, tmB, tmO, p, cin, cout, mode, stream);
+  if (dtype == 1) return conv3x3_dispatch<__nv_bfloat16>(tmA, tmB, tmO, p, cin, cout, mode, stream);
   set_error("conv3x3: dtype must be 0 (fp16) or 1 (bf16)");
   return SED_ERR_UNSUPPORTED;
 }
 
-// conv_block1 as one kernel: conv1 (1 -> 64, CUDA cores, float32) feeds conv2's tensor-core operand through shared
-// memory; the [NB, H, 64, 64] intermediate never exists in HBM.
+// conv_block1 as one kernel: conv1 (1 -> 64, split-fp16 tensor-core GEMM) feeds conv2's tensor-core operand through
+// shared memory; the [NB, H, 64, 64] intermediate never exists in HBM.
 int conv_block1_launch(const float* x, int NB, int H, int W, const float* w1s, const float* shift1, const void* w2packed,
-                       const float* scale2, const float* shift2, void* out, int producer, int dtype,
-                       cudaStream_t stream) {
-  if (producer != 0 && producer != 1) {
-    set_error("conv_block1: producer must be 0 (CUDA-core FMAs) or 1 (split-fp16 tensor cores)");
-    return SED_ERR_UNSUPPORTED;
-  }
+                       const float* scale2, const float* shift2, void* out, int dtype, cudaStream_t stream) {
   if (NB <= 0 || H <= 0 || W <= 0 || (W % 16) != 0) {
     set_error("conv_block1: bad shape NB=%d H=%d W=%d (W %% 16 == 0)", NB, H, W);
     return SED_ERR_BAD_SHAPE;
@@ -869,38 +827,31 @@ int conv_block1_launch(const float* x, int NB, int H, int W, const float* w1s, c
     p.dbg = e ? atoi(e) : 0;
   }
 #endif
-  if (producer == 1) {
-    if (dtype != 0 && dtype != 1) {
-      set_error("conv_block1: dtype must be 0 (fp16) or 1 (bf16)");
-      return SED_ERR_UNSUPPORTED;
-    }
-    int pairs = num_sms() / 2;
-    const int items = (p.num_tiles + 1) / 2;
-    if (pairs > items) pairs = items;
-    cudaError_t e;
-    if (dtype == 0) {
-      e = cudaFuncSetAttribute(conv_block1_tc_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               c1tc::SMEM_BYTES);
-      if (e == cudaSuccess)
-        conv_block1_tc_kernel<__half><<<2 * pairs, c1tc::THREADS, c1tc::SMEM_BYTES, stream>>>(tmB, p);
-    } else {
-      e = cudaFuncSetAttribute(conv_block1_tc_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               c1tc::SMEM_BYTES);
-      if (e == cudaSuccess)
-        conv_block1_tc_kernel<__nv_bfloat16><<<2 * pairs, c1tc::THREADS, c1tc::SMEM_BYTES, stream>>>(tmB, p);
-    }
-    if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) {
-      set_error("conv_block1 (tensor-core producer) launch: %s", cudaGetErrorString(e));
-      return SED_ERR_CUDA;
-    }
-    return SED_OK;
+  if (dtype != 0 && dtype != 1) {
+    set_error("conv_block1: dtype must be 0 (fp16) or 1 (bf16)");
+    return SED_ERR_UNSUPPORTED;
   }
-  if (dtype == 0) return launch_pair<__half, 64, 64, EPI_POOL, 6, 4, true, 1, 1, 1, true>(tmB, tmB, tmB, p, stream);
-  if (dtype == 1)
-    return launch_pair<__nv_bfloat16, 64, 64, EPI_POOL, 6, 4, true, 1, 1, 1, true>(tmB, tmB, tmB, p, stream);
-  set_error("conv_block1: dtype must be 0 (fp16) or 1 (bf16)");
-  return SED_ERR_UNSUPPORTED;
+  int pairs = num_sms() / 2;
+  const int items = (p.num_tiles + 1) / 2;
+  if (pairs > items) pairs = items;
+  cudaError_t e;
+  if (dtype == 0) {
+    e = cudaFuncSetAttribute(conv_block1_tc_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             c1tc::SMEM_BYTES);
+    if (e == cudaSuccess)
+      conv_block1_tc_kernel<__half><<<2 * pairs, c1tc::THREADS, c1tc::SMEM_BYTES, stream>>>(tmB, p);
+  } else {
+    e = cudaFuncSetAttribute(conv_block1_tc_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             c1tc::SMEM_BYTES);
+    if (e == cudaSuccess)
+      conv_block1_tc_kernel<__nv_bfloat16><<<2 * pairs, c1tc::THREADS, c1tc::SMEM_BYTES, stream>>>(tmB, p);
+  }
+  if (e == cudaSuccess) e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    set_error("conv_block1 launch: %s", cudaGetErrorString(e));
+    return SED_ERR_CUDA;
+  }
+  return SED_OK;
 }
 
 #ifdef SED_C1_STAMPS
@@ -976,14 +927,14 @@ int linear_launch(const void* a16, long M, int K, const void* w16, const float* 
       // large M (the GRU input projection / QKV projection of a whole batch): the kernel is bound by L2 -> shared
       // memory operand traffic (A 128 KB + B 128 KB per 128 x 128 tile = 125 B/clk/SM); two row tiles per work item
       // share every B block (94 B/clk/SM)
-      rc = dtype == 0 ? launch_cfg<__half, 512, 128, 2, false, false, EPI_LINEAR, 4, 4>(tmA, tmBp, tmA, p, stream)
-                      : launch_cfg<__nv_bfloat16, 512, 128, 2, false, false, EPI_LINEAR, 4, 4>(tmA, tmBp, tmA, p, stream);
+      rc = dtype == 0 ? launch_cfg<__half, 512, 128, 2, 4, 4>(tmA, tmBp, p, stream)
+                      : launch_cfg<__nv_bfloat16, 512, 128, 2, 4, 4>(tmA, tmBp, p, stream);
     } else if (K == 512) {
-      rc = dtype == 0 ? launch_cfg<__half, 512, 128, 1, false, false, EPI_LINEAR, 4, 4>(tmA, tmBp, tmA, p, stream)
-                      : launch_cfg<__nv_bfloat16, 512, 128, 1, false, false, EPI_LINEAR, 4, 4>(tmA, tmBp, tmA, p, stream);
+      rc = dtype == 0 ? launch_cfg<__half, 512, 128, 1, 4, 4>(tmA, tmBp, p, stream)
+                      : launch_cfg<__nv_bfloat16, 512, 128, 1, 4, 4>(tmA, tmBp, p, stream);
     } else {
-      rc = dtype == 0 ? launch_cfg<__half, 256, 128, 1, false, false, EPI_LINEAR, 4, 4>(tmA, tmBp, tmA, p, stream)
-                      : launch_cfg<__nv_bfloat16, 256, 128, 1, false, false, EPI_LINEAR, 4, 4>(tmA, tmBp, tmA, p, stream);
+      rc = dtype == 0 ? launch_cfg<__half, 256, 128, 1, 4, 4>(tmA, tmBp, p, stream)
+                      : launch_cfg<__nv_bfloat16, 256, 128, 1, 4, 4>(tmA, tmBp, p, stream);
     }
   }
   return rc;

@@ -4,18 +4,17 @@
 // Reference semantics: ConvBlock.forward  pytorch/models.py:125-141 (conv 3x3 s1 p1 no bias -> BN(eval)
 // -> ReLU, twice, then avg_pool2d), freq-mean models.py:668, nn.Linear inside nn.GRU / MultiHead.
 //
-// GEMM view: M = output pixels (one 16(H) x 8(W) spatial patch = 128 rows per tile), N = Cout slice,
+// Conv GEMM view: M = output pixels (one 16(H) x 8(W) spatial patch = 128 rows per tile), N = Cout slice,
 // K = 9 taps x Cin.  Activations are NHWC 16-bit, weights are [Cout][tap][Cin] 16-bit (K-major).
 //
-//  * A operand, PATCH mode: per 64-channel chunk ONE TMA box (64ch x 10w x 18h) brings the haloed
-//    patch into a SWIZZLE_128B buffer (180 pixel rows of 128 B, zero-filled outside the image = conv
-//    padding).  The nine taps are nine UMMA descriptors into that single buffer: start address
+//  * conv_umma2_kernel (the conv layers, CTA pairs): per 64-channel chunk ONE TMA box (64ch x 10w x 18h)
+//    brings the haloed patch into a SWIZZLE_128B buffer (180 pixel rows of 128 B, zero-filled outside the
+//    image = conv padding).  The nine taps are nine UMMA descriptors into that single buffer: start address
 //    + (r*10+s)*128 B, 8-row group stride 1280 B.  A is therefore read from L2 once, not nine times.
-//  * A operand, TAP mode: one (64ch x 8w x 16h) box per tap (used for the GEMM and as fallback).
-//  * B operand: either streamed per (chunk, tap) through a ring, or RESIDENT in shared memory for the
-//    whole persistent CTA when the Cout-slice of the weights fits (weight-stationary).
-//  * NT (1|2) pixel tiles share every B block, accumulators live in TMEM (NT*BN columns per stage).
-//  * Warp roles: warp0 = TMA producer, warp1 = MMA issuer (+TMEM alloc), warps2-5 = epilogue.
+//    B is either streamed per (chunk, tap) through a ring, or RESIDENT in shared memory for the whole
+//    persistent CTA pair when the Cout slice of the weights fits (weight-stationary).
+//  * conv_umma_kernel (the GEMM, single CTA): one (64ch x 128 rows) box of A and one of B per K chunk.
+//  * NT (1|2) pixel / row tiles share every B block, accumulators live in TMEM (NT*BN columns per stage).
 #pragma once
 #include "sed_common.cuh"
 
@@ -39,7 +38,7 @@ struct ConvParams {
   void* out3;              // linear only, optional: 16-bit residual (value - its 16-bit rounding) of columns < lo_cols,
   int lo_cols;             //   [M, lo_cols]: hi + lo carry ~21 bits of the float32 result (split-precision operands)
   long out_sn, out_sh;     // EPI 2: output row of (image n, row h) = n*out_sn + h*out_sh (default H, 1)
-  // fused conv_block1 (FUSE1): the A operand is computed in the kernel from the 1-channel input
+  // conv_block1_tc_kernel: the A operand is computed in the kernel from the 1-channel input
   const float* x1;         // [NB, H, W] f32 (log-mel after bn0)
   const float* w1;         // [64][9] f32 conv_block1.conv1 weights with the bn1 scale folded in
   const float* shift1;     // [64] f32 folded bn1 shift
@@ -59,27 +58,24 @@ constexpr int kPatchBytes = 180 * 128;       // 18 x 10 pixels x 64 ch x 2 B
 constexpr int kPatchStride = 23 * 1024;      // padded so every patch starts 1024-aligned
 constexpr int kTileBytes = 128 * 128;        // 128 pixels x 64 ch x 2 B
 
-template <int CIN, int BN, int NT, bool BRES, bool PATCH, int EPI, int SA, int SB>
+template <int CIN, int BN, int NT, int SA, int SB>
 struct ConvCfg {
   // 8 epilogue warps: two per TMEM lane quarter, each draining half of the BN accumulator columns
   static constexpr int EW = 8;
   static constexpr int THREADS = 64 + 32 * EW;
   static constexpr int CPW = BN / 2;                                  // accumulator columns per epilogue warp
-  static constexpr int NSTG = (EPI == EPI_STORE) ? (CPW >= 64 ? 2 : 1) : 0;  // 16 KB TMA-store staging tiles
-  static constexpr int SS = BRES ? BN : (EPI == EPI_LINEAR ? 1536 : 512);  // cached scale/shift entries
-  static constexpr int TAPS = (EPI == EPI_LINEAR) ? 1 : 9;
+  static constexpr int SS = 1536;                                     // cached bias entries (one column panel)
   static constexpr int NCHUNK = CIN / 64;
-  static constexpr int A_STAGE = NT * (PATCH ? kPatchStride : kTileBytes);
+  static constexpr int A_STAGE = NT * kTileBytes;
   static constexpr int B_BLOCK = BN * 128;
-  static constexpr int B_BYTES = BRES ? NCHUNK * TAPS * B_BLOCK : SB * B_BLOCK;
+  static constexpr int B_BYTES = SB * B_BLOCK;
   static constexpr int ACC_COLS = NT * BN;
   static constexpr int ACC_STAGES = (2 * ACC_COLS <= 512) ? 2 : 1;
   static constexpr int TMEM_COLS = (ACC_COLS * ACC_STAGES <= 32) ? 32 : (ACC_COLS * ACC_STAGES <= 64) ? 64
                                    : (ACC_COLS * ACC_STAGES <= 128) ? 128 : (ACC_COLS * ACC_STAGES <= 256) ? 256 : 512;
   static constexpr int SMEM_A = SA * A_STAGE;
-  static constexpr int SMEM_STG = NSTG * kTileBytes;
   static constexpr int SMEM_MISC = 2 * SS * 4 + 256;
-  static constexpr int SMEM_BYTES = 1024 /*align slack*/ + SMEM_A + B_BYTES + SMEM_STG + SMEM_MISC;
+  static constexpr int SMEM_BYTES = 1024 /*align slack*/ + SMEM_A + B_BYTES + SMEM_MISC;
   static_assert(CIN % 64 == 0, "CIN must be a multiple of 64");
   static_assert(BN % 16 == 0 && BN >= 16 && BN <= 256, "UMMA N");
   static_assert(ACC_COLS <= 512, "TMEM columns");
@@ -272,12 +268,15 @@ SED_DEVICE_INLINE uint64_t desc_join(uint32_t lo, uint32_t hi) {
   return d;
 }
 
-template <typename T, int CIN, int BN, int NT, bool BRES, bool PATCH, int EPI, int SA, int SB>
-__global__ void __launch_bounds__(ConvCfg<CIN, BN, NT, BRES, PATCH, EPI, SA, SB>::THREADS, 1)
+// The plain GEMM out[M, N] = A[M, K] * B[N, K]^T (+ bias, ReLU) of the temporal blocks: one work item is NT row tiles
+// of 128 rows against one BN-column slice, the slices of a row-tile group are consecutive items.  Warp roles:
+// warp0 = TMA producer, warp1 = MMA issuer (+TMEM alloc), warps2-9 = epilogue.  tmO is not read (the epilogue stores
+// from registers); it keeps the parameter block laid out as in conv_umma2_kernel.
+template <typename T, int CIN, int BN, int NT, int SA, int SB>
+__global__ void __launch_bounds__(ConvCfg<CIN, BN, NT, SA, SB>::THREADS, 1)
 conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmO, const ConvParams p) {
-  using Cfg = ConvCfg<CIN, BN, NT, BRES, PATCH, EPI, SA, SB>;
-  constexpr int TAPS = Cfg::TAPS;
+  using Cfg = ConvCfg<CIN, BN, NT, SA, SB>;
   constexpr int NCHUNK = Cfg::NCHUNK;
   constexpr int ACC_STAGES = Cfg::ACC_STAGES;
 
@@ -285,13 +284,12 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   uint8_t* smem = align_smem_1024(smem_raw);
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem + Cfg::SMEM_A;
-  uint8_t* smem_stg = smem_b + Cfg::B_BYTES;  // [NSTG][128 px][128 B] SWIZZLE_128B staging for TMA stores
-  float* s_scale = reinterpret_cast<float*>(smem_stg + Cfg::SMEM_STG);
+  float* s_scale = reinterpret_cast<float*>(smem_b + Cfg::B_BYTES);
   float* s_shift = s_scale + Cfg::SS;
   uint64_t* bars = reinterpret_cast<uint64_t*>(s_shift + Cfg::SS);
   uint64_t* a_full = bars;             // [SA]
   uint64_t* a_empty = a_full + SA;     // [SA]
-  uint64_t* b_full = a_empty + SA;     // [SB] (index 0 doubles as "resident weights landed")
+  uint64_t* b_full = a_empty + SA;     // [SB]
   uint64_t* b_empty = b_full + SB;     // [SB]
   uint64_t* t_full = b_empty + SB;     // [2]
   uint64_t* t_empty = t_full + 2;      // [2]
@@ -302,33 +300,17 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 
   // ---- work decomposition -------------------------------------------------------------
   const int groups = (p.num_tiles + NT - 1) / NT;
-  int item_begin, item_stride, item_end;
-  int fixed_slice = 0;
-  if (BRES) {
-    fixed_slice = blockIdx.x % p.nslices;
-    item_begin = blockIdx.x / p.nslices;
-    item_stride = gridDim.x / p.nslices;
-    item_end = groups;
-  } else {
-    item_begin = blockIdx.x;
-    item_stride = gridDim.x;
-    item_end = groups * p.nslices;
-  }
+  const int item_begin = blockIdx.x, item_stride = gridDim.x, item_end = groups * p.nslices;
 
   // ---- one-time setup -------------------------------------------------------------------
-  // folded BatchNorm scale / shift (linear: 1 / bias); resident-weight CTAs only cache their own slice
-  const int ss_base = BRES ? fixed_slice * BN : 0;
-  for (int i = threadIdx.x; i < Cfg::SS && ss_base + i < p.cout; i += blockDim.x) {
-    // the averaging factor of the pooling epilogues rides the BN affine: relu(k x) = k relu(x) for k > 0, and scaling
-    // by a power of two is exact, so the result is bit-identical to averaging afterwards
-    constexpr float kAvg = (EPI == EPI_POOL) ? 0.25f : (EPI == EPI_FREQMEAN) ? 0.125f : 1.0f;
-    s_scale[i] = (EPI == EPI_LINEAR) ? 1.0f : kAvg * p.scale[ss_base + i];
-    s_shift[i] = p.shift ? kAvg * p.shift[ss_base + i] : 0.0f;
+  // the epilogue's affine is 1 x acc + bias
+  for (int i = threadIdx.x; i < Cfg::SS && i < p.cout; i += blockDim.x) {
+    s_scale[i] = 1.0f;
+    s_shift[i] = p.shift ? p.shift[i] : 0.0f;
   }
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if (EPI == EPI_STORE) tma_prefetch_desc(&tmO);
     for (int i = 0; i < SA; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 1); }
     for (int i = 0; i < SB; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&t_full[i], 1); mbar_init(&t_empty[i], Cfg::EW); }
@@ -343,66 +325,24 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  auto tile_coords = [&](int tile, int& n, int& h0, int& w0) {
-    const int per_img = p.tiles_h * p.tiles_w;
-    n = fast_div(tile, p.magic_img);
-    const int rem = tile - n * per_img;
-    const int th = fast_div(rem, p.magic_w);
-    h0 = th * 16;
-    w0 = (rem - th * p.tiles_w) * 8;
-  };
-
   if (warp == 0) {
     // =============================== TMA producer ===========================================
     if (elect_one()) {
       uint32_t sa = 0, pa = 0, sb = 0, pb = 0;
-      if (BRES) {
-        mbar_expect_tx(&b_full[0], NCHUNK * TAPS * Cfg::B_BLOCK);
-        for (int c = 0; c < NCHUNK; ++c)
-          for (int tap = 0; tap < TAPS; ++tap)
-            tma_load_2d(smem_b + (c * TAPS + tap) * Cfg::B_BLOCK, &tmB, &b_full[0], tap * CIN + c * 64,
-                        fixed_slice * BN);
-      }
       for (int item = item_begin; item < item_end; item += item_stride) {
-        const int g = BRES ? item : item / p.nslices;
-        const int slice = BRES ? fixed_slice : item - g * p.nslices;
+        const int g = item / p.nslices;
+        const int slice = item - g * p.nslices;
         for (int c = 0; c < NCHUNK; ++c) {
-          if (PATCH) {
-            mbar_wait(&a_empty[sa], pa ^ 1);
-            mbar_expect_tx(&a_full[sa], NT * kPatchBytes);
+          mbar_wait(&a_empty[sa], pa ^ 1);
+          mbar_expect_tx(&a_full[sa], NT * kTileBytes);
 #pragma unroll
-            for (int t = 0; t < NT; ++t) {
-              int n, h0, w0;
-              tile_coords(g * NT + t, n, h0, w0);  // tiles past the end have n >= NB: fully OOB -> zeros
-              tma_load_4d(smem_a + sa * Cfg::A_STAGE + t * kPatchStride, &tmA, &a_full[sa], c * 64, w0 - 1,
-                          h0 - 1, n);
-            }
-            if (++sa == SA) { sa = 0; pa ^= 1; }
-          }
-          for (int tap = 0; tap < TAPS; ++tap) {
-            if (!PATCH) {
-              mbar_wait(&a_empty[sa], pa ^ 1);
-              mbar_expect_tx(&a_full[sa], NT * kTileBytes);
-#pragma unroll
-              for (int t = 0; t < NT; ++t) {
-                uint8_t* dst = smem_a + sa * Cfg::A_STAGE + t * kTileBytes;
-                if (EPI == EPI_LINEAR) {
-                  tma_load_2d(dst, &tmA, &a_full[sa], c * 64, (g * NT + t) * 128);
-                } else {
-                  int n, h0, w0;
-                  tile_coords(g * NT + t, n, h0, w0);
-                  tma_load_4d(dst, &tmA, &a_full[sa], c * 64, w0 + (tap % 3) - 1, h0 + (tap / 3) - 1, n);
-                }
-              }
-              if (++sa == SA) { sa = 0; pa ^= 1; }
-            }
-            if (!BRES) {
-              mbar_wait(&b_empty[sb], pb ^ 1);
-              mbar_expect_tx(&b_full[sb], Cfg::B_BLOCK);
-              tma_load_2d(smem_b + sb * Cfg::B_BLOCK, &tmB, &b_full[sb], tap * CIN + c * 64, slice * BN);
-              if (++sb == SB) { sb = 0; pb ^= 1; }
-            }
-          }
+          for (int t = 0; t < NT; ++t)
+            tma_load_2d(smem_a + sa * Cfg::A_STAGE + t * kTileBytes, &tmA, &a_full[sa], c * 64, (g * NT + t) * 128);
+          if (++sa == SA) { sa = 0; pa ^= 1; }
+          mbar_wait(&b_empty[sb], pb ^ 1);
+          mbar_expect_tx(&b_full[sb], Cfg::B_BLOCK);
+          tma_load_2d(smem_b + sb * Cfg::B_BLOCK, &tmB, &b_full[sb], c * 64, slice * BN);
+          if (++sb == SB) { sb = 0; pb ^= 1; }
         }
       }
     }
@@ -410,66 +350,36 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     // =============================== MMA issuer =============================================
     if (elect_one()) {
       constexpr uint32_t idesc = umma_idesc_f16(Elem16<T>::kFmt, 128, BN);
-      constexpr uint32_t a_hi = desc_hi_sw128(PATCH ? 1280 : 1024);
+      constexpr uint32_t a_hi = desc_hi_sw128(1024);
       constexpr uint32_t b_hi = desc_hi_sw128(1024);
-      constexpr uint32_t a_tile_step = (PATCH ? kPatchStride : kTileBytes) >> 4;
+      constexpr uint32_t a_tile_step = kTileBytes >> 4;
       const uint32_t a_lo0 = desc_lo(smem_u32(smem_a));
       const uint32_t b_lo0 = desc_lo(smem_u32(smem_b));
       uint32_t sa = 0, pa = 0, sb = 0, pb = 0, acc = 0, pacc = 0;
-      if (BRES) {
-        mbar_wait(&b_full[0], 0);
-        tc_fence_after();
-      }
       for (int item = item_begin; item < item_end; item += item_stride) {
         mbar_wait(&t_empty[acc], pacc ^ 1);
         tc_fence_after();
         const uint32_t d_base = tmem_base + acc * Cfg::ACC_COLS;
         for (int c = 0; c < NCHUNK; ++c) {
-          uint32_t a_lo = 0;
-          if (PATCH) {
-            mbar_wait(&a_full[sa], pa);
-            tc_fence_after();
-            a_lo = a_lo0 + sa * (Cfg::A_STAGE >> 4);
-          }
+          mbar_wait(&a_full[sa], pa);
+          tc_fence_after();
+          const uint32_t a_lo = a_lo0 + sa * (Cfg::A_STAGE >> 4);
+          mbar_wait(&b_full[sb], pb);
+          tc_fence_after();
+          const uint32_t b_lo = b_lo0 + sb * (Cfg::B_BLOCK >> 4);
 #pragma unroll
-          for (int tap = 0; tap < TAPS; ++tap) {
-            if (!PATCH) {
-              mbar_wait(&a_full[sa], pa);
-              tc_fence_after();
-              a_lo = a_lo0 + sa * (Cfg::A_STAGE >> 4);
-            }
-            uint32_t b_lo;
-            if (BRES) {
-              b_lo = b_lo0 + (c * TAPS + tap) * (Cfg::B_BLOCK >> 4);
-            } else {
-              mbar_wait(&b_full[sb], pb);
-              tc_fence_after();
-              b_lo = b_lo0 + sb * (Cfg::B_BLOCK >> 4);
-            }
-            // PATCH: tap (r, s) is the same haloed buffer shifted by (r*10 + s) pixel rows of 128 B
-            const uint32_t tap_off = PATCH ? ((tap / 3) * 10 + (tap % 3)) * 8 : 0;
+          for (int t = 0; t < NT; ++t) {
 #pragma unroll
-            for (int t = 0; t < NT; ++t) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                if (!SED_CONV_DBG(p, 4))
-                  umma_f16(d_base + t * BN, desc_join(a_lo + t * a_tile_step + tap_off + k * 2, a_hi),
-                           desc_join(b_lo + k * 2, b_hi), idesc, (c | tap | k) ? 1u : 0u);
-              }
-            }
-            if (!PATCH) {
-              umma_commit(&a_empty[sa]);
-              if (++sa == SA) { sa = 0; pa ^= 1; }
-            }
-            if (!BRES) {
-              umma_commit(&b_empty[sb]);
-              if (++sb == SB) { sb = 0; pb ^= 1; }
+            for (int k = 0; k < 4; ++k) {
+              if (!SED_CONV_DBG(p, 4))
+                umma_f16(d_base + t * BN, desc_join(a_lo + t * a_tile_step + k * 2, a_hi),
+                         desc_join(b_lo + k * 2, b_hi), idesc, (c | k) ? 1u : 0u);
             }
           }
-          if (PATCH) {
-            umma_commit(&a_empty[sa]);
-            if (++sa == SA) { sa = 0; pa ^= 1; }
-          }
+          umma_commit(&a_empty[sa]);
+          if (++sa == SA) { sa = 0; pa ^= 1; }
+          umma_commit(&b_empty[sb]);
+          if (++sb == SB) { sb = 0; pb ^= 1; }
         }
         umma_commit(&t_full[acc]);
         if (++acc == ACC_STAGES) { acc = 0; pacc ^= 1; }
@@ -480,11 +390,10 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     const int quarter = warp & 3;            // TMEM lane quarter this warp may access
     const int chalf = (warp - 2) >> 2;       // which half of the BN columns this warp drains
     constexpr int CPW = Cfg::CPW;            // columns per warp
-    const bool stg_leader = (lane == 0) && (warp == ((CPW >= 64) ? 2 + 4 * chalf : 2));
     uint32_t acc = 0, pacc = 0;
     for (int item = item_begin; item < item_end; item += item_stride) {
-      const int g = BRES ? item : item / p.nslices;
-      const int slice = BRES ? fixed_slice : item - g * p.nslices;
+      const int g = item / p.nslices;
+      const int slice = item - g * p.nslices;
       const int ch0 = slice * BN;
       mbar_wait(&t_full[acc], pacc);
       tc_fence_after();
@@ -493,19 +402,16 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         if (SED_CONV_DBG(p, 2)) break;
         const int tile = g * NT + t;
         const bool tile_ok = (tile < p.num_tiles) && !SED_CONV_DBG(p, 1);
-        int n = 0, h0 = 0, w0 = 0;
-        if (EPI != EPI_LINEAR) tile_coords(tile, n, h0, w0);
         const uint32_t taddr = tmem_base + acc * Cfg::ACC_COLS + t * BN + chalf * CPW +
                                (static_cast<uint32_t>(quarter * 32) << 16);
-        conv_epilogue_tile<T, BN, BRES, EPI>(taddr, chalf, warp, lane, s_scale, s_shift, ch0, tile, tile_ok, n, h0, w0, p,
-                                             smem_stg, &tmO);
+        conv_epilogue_tile<T, BN, false, EPI_LINEAR>(taddr, chalf, warp, lane, s_scale, s_shift, ch0, tile, tile_ok, 0,
+                                                     0, 0, p, nullptr, nullptr);
       }
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&t_empty[acc]);
       if (++acc == ACC_STAGES) { acc = 0; pacc ^= 1; }
     }
-    if (EPI == EPI_STORE && stg_leader) bulk_wait_all0();  // staging tiles must outlive their stores
   }
 
   tc_fence_before();
@@ -517,11 +423,11 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 }
 
 // =================================================================================================
-// CTA-pair variant (tcgen05 cta_group::2) for the weight-stationary layers.
+// The conv layers on CTA pairs (tcgen05 cta_group::2).
 //
 // With the accumulator N of a single-CTA MMA limited to the layer's Cout slice (64 or 128), each
 // K=16 MMA step reads 4 KB of A plus N*32 B of B from shared memory in N/2 cycles -- more than the
-// 128 B/clk the shared-memory pipe delivers, so those layers ran at half the tensor rate.  A CTA pair
+// 128 B/clk the shared-memory pipe delivers, so a single CTA runs at half the tensor rate.  A CTA pair
 // computes M = 256 pixels (one 16x8 tile per CTA) against the SAME N columns; each CTA keeps only half of
 // the weight rows (N/2) resident and the hardware shares the halves, so the per-CTA shared-memory traffic
 // per MMA drops to 4 KB + N*16 B and the weight-resident footprint halves as well.
@@ -530,7 +436,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 // warp1 = TMEM allocation (+ MMA issue on the leader only, commits multicast to both CTAs),
 // warps2-9 = epilogue of the CTA's own 128 accumulator rows.
 // =================================================================================================
-template <int CIN, int BN, int EPI, int SA, int ACC, bool BRES, int NT, int SB, int EG = 1, bool FUSE1 = false>
+template <int CIN, int BN, int EPI, int SA, int ACC, bool BRES, int NT, int SB>
 struct Conv2Cfg {
   static constexpr int NCHUNK = CIN / 64;
   static constexpr int TAPS = 9;
@@ -542,30 +448,23 @@ struct Conv2Cfg {
   static constexpr int NSTG = (EPI == EPI_STORE) ? (CPW >= 64 ? 2 : 1) : 0;
   static constexpr int SMEM_STG = NSTG * kTileBytes;
   static constexpr int SS = BRES ? BN : 512;
-  static constexpr int PW = FUSE1 ? 6 : 0;                            // operand-producer warps (fused conv_block1)
-  static constexpr int SMEM_IN = PW * 5 * 12 * 4;                     // per producer warp: 5 x 12 input window (f32)
-  static constexpr int SMEM_MISC = 2 * SS * 4 + 256 + SMEM_IN;
+  static constexpr int SMEM_MISC = 2 * SS * 4 + 256;
   static constexpr int SMEM_BYTES = 1024 + SMEM_A + B_BYTES + SMEM_STG + SMEM_MISC;
   static constexpr int ACC_COLS = NT * BN;
   static constexpr int TMEM_COLS = (ACC * ACC_COLS <= 32) ? 32 : (ACC * ACC_COLS <= 64) ? 64
                                    : (ACC * ACC_COLS <= 128) ? 128 : (ACC * ACC_COLS <= 256) ? 256 : 512;
-  static_assert(!FUSE1 || (CIN == 64 && NT == 1 && BRES), "fused conv_block1: 64 input channels, one tile per CTA");
-  // EG epilogue groups of 8 warps drain alternate accumulator stages.  Measured on conv_block1.conv2 (N = 64): no
-  // gain from EG = 2 -- that layer is bound by the shared-memory pipe (operand reads + TMA writes), not the epilogue
-  static constexpr int THREADS = 64 + 32 * 8 * EG + 32 * PW;
-  static_assert(EG == 1 || EPI != EPI_STORE, "the TMA-store staging tiles belong to one epilogue group");
+  static constexpr int THREADS = 64 + 32 * 8;
   static_assert(ACC * ACC_COLS <= 512, "TMEM columns");
   static_assert(BN % 32 == 0 && BN <= 256, "pair MMA: N multiple of 16 per CTA half");
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
 
-template <typename T, int CIN, int BN, int EPI, int SA, int ACC, bool BRES, int NT, int SB, int EG = 1,
-          bool FUSE1 = false>
+template <typename T, int CIN, int BN, int EPI, int SA, int ACC, bool BRES, int NT, int SB>
 __global__ void __cluster_dims__(2, 1, 1)
-__launch_bounds__(Conv2Cfg<CIN, BN, EPI, SA, ACC, BRES, NT, SB, EG, FUSE1>::THREADS, 1)
+__launch_bounds__(Conv2Cfg<CIN, BN, EPI, SA, ACC, BRES, NT, SB>::THREADS, 1)
 conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                   const __grid_constant__ CUtensorMap tmO, const ConvParams p) {
-  using Cfg = Conv2Cfg<CIN, BN, EPI, SA, ACC, BRES, NT, SB, EG, FUSE1>;
+  using Cfg = Conv2Cfg<CIN, BN, EPI, SA, ACC, BRES, NT, SB>;
   constexpr int TAPS = Cfg::TAPS;
   constexpr int NCHUNK = Cfg::NCHUNK;
 
@@ -584,7 +483,6 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   uint64_t* t_full = b_empty + SB;    // [ACC] per CTA (multicast commit)
   uint64_t* t_empty = t_full + ACC;   // [ACC] leader's copy, 16 arrivals (8 warps x 2 CTAs)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + ACC);
-  float* s_in = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(s_shift + Cfg::SS) + 256);  // [PW][5][12] (FUSE1)
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -608,7 +506,9 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 
   const int ss_base = BRES ? fixed_slice * BN : 0;
   for (int i = threadIdx.x; i < Cfg::SS && ss_base + i < p.cout; i += blockDim.x) {
-    constexpr float kAvg = (EPI == EPI_POOL) ? 0.25f : (EPI == EPI_FREQMEAN) ? 0.125f : 1.0f;  // see conv_umma_kernel
+    // the averaging factor of the pooling epilogues rides the BN affine: relu(k x) = k relu(x) for k > 0, and scaling
+    // by a power of two is exact, so the result is bit-identical to averaging afterwards
+    constexpr float kAvg = (EPI == EPI_POOL) ? 0.25f : (EPI == EPI_FREQMEAN) ? 0.125f : 1.0f;
     s_scale[i] = kAvg * p.scale[ss_base + i];
     s_shift[i] = kAvg * p.shift[ss_base + i];
   }
@@ -616,8 +516,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
     if (EPI == EPI_STORE) tma_prefetch_desc(&tmO);
-    // a_full: one TMA transaction (armed by the leader) or, fused, one arrive per producer warp of both CTAs
-    for (int i = 0; i < SA; ++i) { mbar_init(&a_full[i], FUSE1 ? 2 * Cfg::PW : 1); mbar_init(&a_empty[i], 1); }
+    for (int i = 0; i < SA; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 1); }
     for (int i = 0; i < SB; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
     for (int i = 0; i < ACC; ++i) { mbar_init(&t_full[i], 1); mbar_init(&t_empty[i], 16); }
     fence_barrier_init();
@@ -653,7 +552,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
                             fixed_slice * BN + rank * (BN / 2));
       }
       uint32_t sa = 0, pa = 0, sb = 0, pb = 0;
-      for (int w = work_begin; w < work_end && !FUSE1; w += work_stride) {
+      for (int w = work_begin; w < work_end; w += work_stride) {
         const int item = BRES ? w : w / p.nslices;
         const int slice = BRES ? fixed_slice : w - item * p.nslices;
         for (int c = 0; c < NCHUNK; ++c) {
@@ -698,7 +597,7 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         tc_fence_after();
         const uint32_t d_base = tmem_base + acc * Cfg::ACC_COLS;
         for (int c = 0; c < NCHUNK; ++c) {
-          if (FUSE1) mbar_wait_cluster(&a_full[sa], pa); else mbar_wait(&a_full[sa], pa);
+          mbar_wait(&a_full[sa], pa);
           tc_fence_after();
           const uint32_t a_lo = a_lo0 + sa * (Cfg::A_STAGE >> 4);
 #pragma unroll
@@ -733,112 +632,15 @@ conv_umma2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         if (++acc == ACC) { acc = 0; pacc ^= 1; }
       }
     }
-  } else if (FUSE1 && warp >= 2 + 8 * EG) {
-    // =============================== fused conv_block1.conv1 operand producer ===============
-    // EXPERIMENTAL (engine variant 3, not the default).  Measured on B200: 1.07 ms per 148 clips against 0.28 + 0.53 ms
-    // for the split-fp16 tensor-core conv1 kernel + this kernel fed by TMA.  The 104 k float32 FMAs per tile occupy the
-    // FMA pipe for >= 810 clk and six producer warps execute them as latency-exposed serial streams (~4000 clk per
-    // tile); more producer warps would cap registers below what the epilogue needs.  Kept as the record of that
-    // experiment and as a second implementation the parity tests can cross-check.
-    // conv_block1.conv2's A operand -- the haloed 18 x 10 pixel x 64 channel patch of relu(bn1(conv1(x))) -- is computed
-    // here from the one-channel input instead of being read back from HBM (pytorch/models.py:128 feeding :129).
-    // Warp pw owns patch rows 3pw..3pw+2; lane l owns channels 2l, 2l+1 (packed f32x2 FMAs); pixels outside the image
-    // are the ZERO padding of conv2, inputs outside the image the zero padding of conv1.
-    const int pw = warp - (2 + 8 * EG);
-    float* win = s_in + pw * 60;  // 5 input rows x 12 columns
-    unsigned long long wreg[9];   // {w[2l][tap], w[2l+1][tap]}
-#pragma unroll
-    for (int t = 0; t < 9; ++t) wreg[t] = pack_f32x2(p.w1[(2 * lane) * 9 + t], p.w1[(2 * lane + 1) * 9 + t]);
-    const unsigned long long shreg = pack_f32x2(p.shift1[2 * lane], p.shift1[2 * lane + 1]);
-    // input element e (0..59) of a tile's window for this warp: row e / 12, column e % 12
-    auto load_inputs = [&](int tile, float& v0, float& v1) {
-      int n, h0, w0;
-      tile_coords(tile, n, h0, w0);
-      const bool tv = tile < p.num_tiles;
-#pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        const int e = lane + 32 * k;
-        const int hh = h0 - 2 + 3 * pw + e / 12, ww = w0 - 2 + e % 12;
-        float v = 0.0f;
-        if (tv && e < 60 && hh >= 0 && hh < p.H && ww >= 0 && ww < p.W)
-          v = __ldg(p.x1 + (static_cast<size_t>(n) * p.H + hh) * p.W + ww);
-        if (k == 0) v0 = v; else v1 = v;
-      }
-    };
-    uint32_t sa = 0, pa = 0;
-    // two tiles of input prefetch in registers; the loads are issued right AFTER a tile's release-arrive (which waits
-    // for every outstanding memory operation of the thread) and consumed two tiles later
-    float c0 = 0.0f, c1 = 0.0f, d0 = 0.0f, d1 = 0.0f;
-    if (work_begin < work_end) load_inputs((work_begin * 2 + static_cast<int>(rank)) * NT, c0, c1);
-    if (work_begin + work_stride < work_end)
-      load_inputs(((work_begin + work_stride) * 2 + static_cast<int>(rank)) * NT, d0, d1);
-    for (int w = work_begin; w < work_end; w += work_stride) {
-      const int tile = (w * 2 + static_cast<int>(rank)) * NT;
-      int n, h0, w0;
-      tile_coords(tile, n, h0, w0);
-      const bool tv = tile < p.num_tiles;
-      win[lane] = c0;
-      if (lane < 28) win[32 + lane] = c1;
-      __syncwarp();
-      mbar_wait(&a_empty[sa], pa ^ 1);
-      uint8_t* patch = smem_a + sa * Cfg::A_STAGE;
-#pragma unroll
-      for (int rr = 0; rr < 3; ++rr) {
-        const int r = 3 * pw + rr;       // patch row; image row h0 - 1 + r
-        const int hh = h0 - 1 + r;
-        const bool rv = tv && hh >= 0 && hh < p.H;
-        float x[3][12];
-#pragma unroll
-        for (int dr = 0; dr < 3; ++dr)
-#pragma unroll
-          for (int q4 = 0; q4 < 3; ++q4) {
-            const float4 v = *reinterpret_cast<const float4*>(win + (rr + dr) * 12 + q4 * 4);
-            x[dr][q4 * 4] = v.x; x[dr][q4 * 4 + 1] = v.y; x[dr][q4 * 4 + 2] = v.z; x[dr][q4 * 4 + 3] = v.w;
-          }
-        // ten independent accumulator chains (one per pixel of the row), taps outermost: full FMA-pipe ILP
-        unsigned long long acc[10];
-#pragma unroll
-        for (int c = 0; c < 10; ++c) acc[c] = shreg;
-#pragma unroll
-        for (int dr = 0; dr < 3; ++dr)
-#pragma unroll
-          for (int dc = 0; dc < 3; ++dc)
-#pragma unroll
-            for (int c = 0; c < 10; ++c)
-              acc[c] = ffma2(pack_f32x2(x[dr][c + dc], x[dr][c + dc]), wreg[dr * 3 + dc], acc[c]);
-#pragma unroll
-        for (int c = 0; c < 10; ++c) {
-          const int ww = w0 - 1 + c;
-          float y0, y1;
-          unpack_f32x2(acc[c], y0, y1);
-          const bool valid = rv && ww >= 0 && ww < p.W;
-          const uint32_t packed = valid ? Elem16<T>::pack2(fmaxf(y0, 0.0f), fmaxf(y1, 0.0f)) : 0u;
-          const int pr = r * 10 + c;
-          *reinterpret_cast<uint32_t*>(patch + pr * 128 + (((lane >> 2) ^ (pr & 7)) << 4) + (lane & 3) * 4) = packed;
-        }
-      }
-      fence_proxy_async_smem();  // generic stores -> the tensor core's (async proxy) operand reads
-      __syncwarp();
-      // the patch lives in THIS SM's shared memory and is read by THIS SM's tensor-core datapath: after the proxy fence
-      // a default (.release.cta) arrive on the leader's barrier is enough; a cluster-scope release costs ~1.5 us
-      if (lane == 0) mbar_arrive_remote_light(&a_full[sa], 0);
-      if (++sa == SA) { sa = 0; pa ^= 1; }
-      c0 = d0;
-      c1 = d1;
-      if (w + 2 * work_stride < work_end)
-        load_inputs(((w + 2 * work_stride) * 2 + static_cast<int>(rank)) * NT, d0, d1);
-    }
-  } else if (warp >= 2 && warp < 2 + 8 * EG) {
-    // =============================== epilogue (EG groups of 8 warps, both CTAs) =============
+  } else if (warp >= 2 && warp < 10) {
+    // =============================== epilogue (8 warps, both CTAs) ==========================
     const int ew = warp - 2;
-    const int grp = ew >> 3;            // epilogue group: drains the work items with (index % EG) == grp
     const int quarter = warp & 3;
     const int chalf = (ew & 7) >> 2;
     constexpr int CPW = Cfg::CPW;
     const bool stg_leader = (lane == 0) && (warp == ((CPW >= 64) ? 2 + 4 * chalf : 2));
     uint32_t it = 0;
     for (int w = work_begin; w < work_end; w += work_stride, ++it) {
-      if (EG > 1 && static_cast<int>(it % EG) != grp) continue;
       const uint32_t acc = it % ACC, pacc = (it / ACC) & 1;
       const int item = BRES ? w : w / p.nslices;
       const int slice = BRES ? fixed_slice : w - item * p.nslices;

@@ -38,14 +38,13 @@ int logmel_rows_launch(const float* spec, long rows, int F, const int* mel_lo, c
 int conv_first_launch(const float* x, int NB, int H, int W, const float* w9, const float* scale, const float* shift,
                       void* out, int dtype, cudaStream_t stream);
 
-// mode: 0 = store NHWC, 1 = 2x2 avg-pool, 2 = freq-mean (W must be 8) ; variant: 0 = patch (halo reuse), 1 = per-tap
+// mode: 0 = store NHWC, 1 = 2x2 avg-pool, 2 = freq-mean (W must be 8); every layer runs on CTA pairs
 int conv3x3_launch(const void* x, int NB, int H, int W, int cin, const void* wpacked, const float* scale,
                    const float* shift, int cout, int mode, void* out, void* out_f32, long out_sn, long out_sh,
-                   int dtype, int variant, cudaStream_t stream);
+                   int dtype, cudaStream_t stream);
 
 int conv_block1_launch(const float* x, int NB, int H, int W, const float* w1s, const float* shift1, const void* w2packed,
-                       const float* scale2, const float* shift2, void* out, int producer, int dtype,
-                       cudaStream_t stream);
+                       const float* scale2, const float* shift2, void* out, int dtype, cudaStream_t stream);
 
 int linear_launch(const void* a16, long M, int K, const void* w16, const float* bias, int N, int relu, float* out,
                   void* out16, int out_layout, int dtype, cudaStream_t stream, void* out_lo = nullptr, int lo_cols = 0);

@@ -593,7 +593,7 @@ class PackedModel:
         length T, sized for the largest micro-batch seen (micro-batch sizes vary inside forward_host).  A small LRU of
         clip lengths is kept, so that callers alternating between lengths (10 s evaluation clips and 5 s streaming
         windows) do not re-allocate ~14.5 GB per switch.  a1, the 8.2 MB/clip output of conv_block1.conv1, only exists
-        for the two-kernel variants of block 1."""
+        for the two-kernel block 1 (variant 2)."""
         ent = self._ws.get(T)
         if ent is None or ent["cap"] < mb or (need_a1 and "a1" not in ent["buf"]):
             cap = mb if ent is None else max(mb, ent["cap"])
@@ -636,7 +636,11 @@ class PackedModel:
         windows=(mb, L, stride): wave_mb is a 1-D recording read as overlapping windows.
         feat32: optional [mb, T', 512] f32 copy of the features (models without a temporal block).
         feat_strides=(sn, sh): feature row of (clip n, step h) is n*sn + h*sh rows after feat_out's first element
-        ((0, 0) = clip-major [mb, T', 512]; (1, Bp) = time-major [T', Bp, 512] as the GRU wants it)."""
+        ((0, 0) = clip-major [mb, T', 512]; (1, Bp) = time-major [T', Bp, 512] as the GRU wants it).
+        variant 4: conv_block1 as one kernel (its 64-channel intermediate stays on chip); 2: conv_block1.conv1 as its
+        own kernel writing a1 (the reference the fused kernel is tested against).  Every other layer runs on CTA pairs."""
+        if variant not in (2, 4):
+            raise ValueError("conv variant must be 2 or 4 (got %r)" % (variant,))
         lib = capi.load()
         if windows is None:
             mb, L = wave_mb.shape
@@ -645,14 +649,11 @@ class PackedModel:
         T = L // self.front.hop + 1
         if T // 8 < 1:
             raise ValueError("clip too short: %d frames" % T)
-        fused1 = variant in (3, 4)  # conv_block1 as one kernel (its 64-channel intermediate stays on chip)
+        fused1 = variant == 4
         ws = self._workspace(mb, T, need_a1=not fused1)
         stream = capi.current_stream(self.device)
         logmel_forward(self.front, wave_mb, self.bn0_scale, self.bn0_shift, out=ws["logmel"], windows=windows)
-        producer = 1 if variant == 4 else 0  # conv1 on the tensor cores (split fp16) / on the CUDA cores
-        if fused1:
-            variant = 2
-        else:
+        if not fused1:
             rc = lib.sed_conv_first_f32(capi.ptr(ws["logmel"]), mb, T, 64, capi.ptr(self.c11_w),
                                         capi.ptr(self.c11_scale), capi.ptr(self.c11_shift), capi.ptr(ws["a1"]),
                                         self.dtype_code, stream)
@@ -666,7 +667,7 @@ class PackedModel:
             if fused1 and li == 0:
                 rc = lib.sed_conv_block1(capi.ptr(ws["logmel"]), mb, T, 64, capi.ptr(self.c11_ws),
                                          capi.ptr(self.c11_shift), capi.ptr(wp), capi.ptr(s), capi.ptr(b),
-                                         capi.ptr(ws["p1"]), producer, self.dtype_code, stream)
+                                         capi.ptr(ws["p1"]), self.dtype_code, stream)
                 capi.check(rc, "sed_conv_block1")
                 capi._count()
                 continue
@@ -676,7 +677,7 @@ class PackedModel:
                                          capi.ptr(b), cout, mode, capi.ptr(out),
                                          capi.ptr(feat32) if dst is None else None,
                                          feat_strides[0] if dst is None else 0, feat_strides[1] if dst is None else 0,
-                                         self.dtype_code, variant, stream)
+                                         self.dtype_code, stream)
             capi.check(rc, "sed_conv3x3_bn_relu(%d->%d)" % (cin, cout))
             capi._count()
         if self.conv_events is not None:

@@ -100,8 +100,8 @@ class _Cnn9Base(nn.Module):
         self._master_ref = [weakref.ref(self)]  # DataParallel replicas copy __dict__: they find the master through it
         self.precision = "fp16"   # 16-bit operand type of the tensor-core layers: 'fp16' or 'bf16'
         self.micro_batch = engine.DEFAULT_MICRO_BATCH   # clips per conv-stack launch group (whole waves of the 148 SMs)
-        self.conv_variant = 4   # 4 = CTA-pair kernels + conv_block1 fused on the tensor cores (default); 2 = CTA-pair kernels with
-        # conv_block1 as two kernels; 0 = single-CTA patch; 1 = per-tap; 3 = 2 + conv_block1 fused on the CUDA cores (slower)
+        self.conv_variant = 4   # 4 = conv_block1 as one tensor-core kernel (default); 2 = conv_block1 as two kernels
+        # (conv1 writes its 64-channel output to memory); every other conv layer runs on CTA pairs either way
 
     # any parameter movement / reload invalidates the packed copies
     def _invalidate(self):

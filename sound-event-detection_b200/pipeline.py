@@ -143,7 +143,7 @@ class HostPipeline:
             events = iter(events)
             # ---- compute stream
             with torch.cuda.stream(compute):
-                pm._workspace(max(b1 - b0 for spans in plan for b0, b1 in spans), T, need_a1=self.variant not in (3, 4))
+                pm._workspace(max(b1 - b0 for spans in plan for b0, b1 in spans), T, need_a1=self.variant == 2)
                 for (p0, p1), spans in zip(parts, plan):
                     n = p1 - p0
                     feat16, feat32, slot_kw = pm._alloc_features(n, Tp)

@@ -1,7 +1,7 @@
 """Per-kernel GPU diagnostics against the CPU oracle (developer tool beside the graded checks; like them it may use the oracle).
 
 Usage on a GPU box:  python tests/gpu_diag.py            # every stage, each in its own subprocess
-                     python tests/gpu_diag.py --stage conv_tap
+                     python tests/gpu_diag.py --stage conv
 """
 import argparse
 import os
@@ -13,7 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
-STAGES = ["frontend", "conv_first", "conv_tap", "conv_patch", "linear", "gru", "mha", "attpool",
+STAGES = ["frontend", "conv_first", "conv", "linear", "gru", "mha", "attpool",
           "model_gru", "model_tr"]
 
 
@@ -92,8 +92,7 @@ def run_stage(stage):
         print("conv_first rel/abs err", rel_err(out.float(), ref))
         return
 
-    if stage in ("conv_tap", "conv_patch"):
-        variant = 1 if stage == "conv_tap" else 0
+    if stage == "conv":
         for (name, cin, cout, mode) in engine.CONV_LAYERS:
             W = {64: 64 if cout == 64 else 32, 128: 32 if cout == 128 else 16, 256: 16 if cout == 256 else 8, 512: 8}[cin]
             for (NB, H) in ((1, 16), (3, 37)):
@@ -107,7 +106,7 @@ def run_stage(stage):
                 t0 = time.time()
                 xd, sc, sh = x.to(dev), scale.to(dev), shift.to(dev)
                 rc = lib.sed_conv3x3_bn_relu(capi.ptr(xd), NB, H, W, cin, capi.ptr(wp), capi.ptr(sc),
-                                             capi.ptr(sh), cout, mode, capi.ptr(out), None, 0, 0, code, variant, stream)
+                                             capi.ptr(sh), cout, mode, capi.ptr(out), None, 0, 0, code, stream)
                 capi.check(rc, name)
                 torch.cuda.synchronize()
                 ref = conv_ref(x.float(), w.float(), scale, shift, mode)
@@ -179,7 +178,7 @@ def run_stage(stage):
         sd = synth.synthetic_state_dict(mt)
         wave = torch.cat([synth.synthetic_waveform(2, 160000, kind="events"), synth.synthetic_waveform(1, 160000)])
         ref, rst = so.model_forward(sd, wave, mt, 512, 160, return_stages=True)
-        for variant in (1, 0):
+        for variant in (4, 2):
             pm = engine.PackedModel(sd, mt, 512, 160, dev)
             t0 = time.time()
             got, st = pm.forward(wave.to(dev), variant=variant, return_stages=True)

@@ -60,7 +60,7 @@ def test_binding_matches_header():
     for name, nargs in decl.items():
         assert len(capi.SIGNATURES[name][0]) == nargs, name
     lib = capi.load()
-    assert lib.sed_abi_version() == 12
+    assert lib.sed_abi_version() == 13
     assert isinstance(lib.sed_last_error_string(), bytes)
 
 

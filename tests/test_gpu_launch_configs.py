@@ -1,8 +1,8 @@
 """The launch configurations a default forward runs, each against a float64 reference of the same operation computed
 from the same 16-bit-rounded operands:
 
-  * sed_conv_block1 (conv_block1 as one kernel), producers 0 and 1, fp16 and bf16, including the 32-bit tile index
-    limit that engine.clamp_micro_batch mirrors;
+  * conv_block1 as one kernel (sed_conv_block1, engine variant 4) and as two (sed_conv_first_f32 + the conv1_2 pair
+    kernel, variant 2), fp16 and bf16, including the 32-bit tile index limit that engine.clamp_micro_batch mirrors;
   * sed_conv3x3_bn_relu 512 -> 512 with the freq-mean epilogue writing time-major feature rows (and its float32 copy);
   * sed_linear / sed_linear_split16 at production row counts (two row tiles per work item, column panels), and the
     temporal blocks that run them at B = 300, T' = 125;
@@ -158,21 +158,34 @@ def test_clamp_micro_batch_keeps_conv_block1_tile_indices_in_32_bits():
     assert accepted(3, 65536) and not accepted(4, 65536)
 
 
-def run_block1(x, w1s, shift1, w2_16, scale2, shift2, producer, code, td, out=None):
+BLOCK1_PATHS = ["fused", "two_kernel"]
+
+
+def run_block1(x, w1s, shift1, w2_16, scale2, shift2, path, code, td, out=None):
+    """conv_block1 through `path`: "fused" = sed_conv_block1, "two_kernel" = sed_conv_first_f32 (bn1 scale 1, as w1s
+    carries it) writing a1, then sed_conv3x3_bn_relu 64 -> 64 with the pooling epilogue."""
     NB, H, W = x.shape
     n = NB * (H // 2) * (W // 2) * 64
     if out is None:
         out = torch.full((n + GUARD,), float("nan"), dtype=td, device=DEV)
     wp = w2_16.permute(0, 2, 3, 1).reshape(64, 576).contiguous()
-    call("sed_conv_block1", capi.ptr(x), NB, H, W, capi.ptr(w1s), capi.ptr(shift1), capi.ptr(wp), capi.ptr(scale2),
-         capi.ptr(shift2), capi.ptr(out), producer, code, stream())
+    if path == "fused":
+        call("sed_conv_block1", capi.ptr(x), NB, H, W, capi.ptr(w1s), capi.ptr(shift1), capi.ptr(wp), capi.ptr(scale2),
+             capi.ptr(shift2), capi.ptr(out), code, stream())
+    else:
+        a1 = torch.empty((NB, H, W, 64), dtype=td, device=DEV)
+        ones = torch.ones(64, device=DEV)
+        call("sed_conv_first_f32", capi.ptr(x), NB, H, W, capi.ptr(w1s), capi.ptr(ones), capi.ptr(shift1), capi.ptr(a1),
+             code, stream())
+        call("sed_conv3x3_bn_relu", capi.ptr(a1), NB, H, W, 64, capi.ptr(wp), capi.ptr(scale2), capi.ptr(shift2), 64,
+             capi.CONV_POOL, capi.ptr(out), None, 0, 0, code, stream())
     torch.cuda.synchronize()
     assert torch.isnan(out[n:n + GUARD].float()).all(), "conv_block1 wrote past its output"
     return out[:n].view(NB, H // 2, W // 2, 64)
 
 
 # Measured on a B200 at 1000 W: the pooled 16-bit a1 equals the float64 rounding on 99.98 % (fp16) / 100 % (bf16) of the
-# outputs for both producers, at most 2 ulps off; a conv1 from the fp16 hi parts alone misses 33 % (fp16) / 6.2 % (bf16),
+# outputs on both block-1 paths, at most 2 ulps off; a conv1 from the fp16 hi parts alone misses 33 % (fp16) / 6.2 % (bf16),
 # 1400-6900 times as often as the kernels.
 PROBE_MIN_EXACT = 0.999
 PROBE_PLAIN_RATIO = 100.0
@@ -180,23 +193,23 @@ PROBE_PLAIN_RATIO = 100.0
 
 @gpu
 @pytest.mark.parametrize("dt", ["fp16", "bf16"])
-@pytest.mark.parametrize("producer", [1, 0])
-def test_conv_block1_conv1_precision_probe(producer, dt):
-    """w2 = identity at the centre tap: p1 is the pooled, rounded a1.  conv1 runs as split 16-bit products (producer 1:
-    hi*hi + lo*hi + hi*lo on the tensor cores, the operands are fp16 whatever the output type) or as float32 FMAs
-    (producer 0), so a1 must round like the float64 value nearly everywhere.  Where one a1 of a window rounds the other
+@pytest.mark.parametrize("path", BLOCK1_PATHS)
+def test_conv_block1_conv1_precision_probe(path, dt):
+    """w2 = identity at the centre tap: p1 is the pooled, rounded a1.  conv1 runs as split 16-bit products
+    (hi*hi + lo*hi + hi*lo on the tensor cores, the operands are fp16 whatever the output type), so a1 must round like
+    the float64 value nearly everywhere.  Where one a1 of a window rounds the other
     way the window mean moves by a quarter of that a1's ulp: up to two output ulps when that pixel dominates the window.
     A conv1 computed from the fp16 hi parts alone (what a dropped lo term gives) misses far more often."""
     code, td = DTYPES[dt]
     x, w1s, shift1, w2, scale2, shift2 = block1_inputs(3, 37, 11, DEV, probe=True)
-    got = run_block1(x, w1s, shift1, w2.to(td), scale2, shift2, producer, code, td)
+    got = run_block1(x, w1s, shift1, w2.to(td), scale2, shift2, path, code, td)
     want = block1_ref(x, w1s, shift1, w2, scale2, shift2, td)[0].to(td)
     d = ulp_distance(got, want)
     exact = (d == 0).double().mean().item()
     h = torch.float16  # the kernel's split type
     plain = block1_ref(x.to(h).float(), w1s.to(h).float(), shift1.to(h).float(), w2, scale2, shift2, td)[0].to(td)
     plain_miss = (ulp_distance(plain, want) != 0).double().mean().item()
-    report("conv_block1 probe producer %d %s" % (producer, dt), exact=exact, max_ulp=int(d.max()),
+    report("conv_block1 probe %s %s" % (path, dt), exact=exact, max_ulp=int(d.max()),
            plain16_miss=plain_miss, miss_ratio=plain_miss / max(1.0 - exact, 1e-9))
     assert int(d.max()) <= 2
     assert exact >= PROBE_MIN_EXACT
@@ -209,22 +222,22 @@ def test_conv_block1_conv1_precision_probe(producer, dt):
 BLOCK1_REL = {"fp16": 2.0 ** -14, "bf16": 2.0 ** -12}
 # With W % 16 == 0 the tile count NB * ceil(H / 16) * W / 8 is always even: every work item of a CTA pair holds two
 # tiles.  What varies is the number of items per pair (one each for small NB, several waves for 37 x 37) and whether
-# the two producer groups, which take alternate items, get equally many.
+# the kernel's two conv1 producer groups, which take alternate items, get equally many.
 BLOCK1_SHAPES = [(1, 1), (1, 2), (2, 15), (3, 16), (1, 17), (37, 37), (2, 1001), (3, 501)]
 
 
 @gpu
 @pytest.mark.parametrize("dt", ["fp16", "bf16"])
-@pytest.mark.parametrize("producer", [1, 0])
+@pytest.mark.parametrize("path", BLOCK1_PATHS)
 @pytest.mark.parametrize("NB,H", BLOCK1_SHAPES, ids=["%dx%d" % s for s in BLOCK1_SHAPES])
-def test_conv_block1_matches_float64(NB, H, producer, dt):
+def test_conv_block1_matches_float64(NB, H, path, dt):
     """Random conv2 weights, ragged heights (1 row: no output; odd H floors; a partial last 16-row tile), 1-37 images
     (37 x 37 = 444 work items: six waves of the 74 CTA pairs).  A padding pixel computed as relu(shift1) shows at the
     first / last rows and columns."""
     code, td = DTYPES[dt]
     x, w1s, shift1, w2, scale2, shift2 = block1_inputs(NB, H, 100 * NB + H, DEV)
     w2 = w2.to(td)
-    got = run_block1(x, w1s, shift1, w2, scale2, shift2, producer, code, td).double()
+    got = run_block1(x, w1s, shift1, w2, scale2, shift2, path, code, td).double()
     want, m = block1_ref(x, w1s, shift1, w2, scale2, shift2, td)
     if got.numel() == 0:
         return
@@ -232,14 +245,14 @@ def test_conv_block1_matches_float64(NB, H, producer, dt):
     edge = torch.zeros_like(got, dtype=torch.bool)
     edge[:, 0] = edge[:, -1] = True
     edge[:, :, 0] = edge[:, :, -1] = True
-    report("conv_block1 %dx%d producer %d %s" % (NB, H, producer, dt), rel=excess.max().item(),
+    report("conv_block1 %dx%d %s %s" % (NB, H, path, dt), rel=excess.max().item(),
            rel_edge=excess[edge].max().item(), max_abs=(got - want).abs().max().item())
     assert excess.max().item() <= BLOCK1_REL[dt]
 
 
 @gpu
-@pytest.mark.parametrize("producer", [1, 0])
-def test_conv_block1_tile_index_limit(producer):
+@pytest.mark.parametrize("path", BLOCK1_PATHS)
+def test_conv_block1_tile_index_limit(path):
     """NB = 3, H = 65 536 (4096 tiles of 16 rows per image) is the largest launch the 32-bit index arithmetic takes:
     correct in row slices around the image and tile boundaries of every image; NB = 4 is refused before launching."""
     code, td = DTYPES["fp16"]
@@ -248,7 +261,7 @@ def test_conv_block1_tile_index_limit(producer):
     w2 = w2.to(td)
     out = torch.full((4 * (H // 2) * (W // 2) * 64 + GUARD,), float("nan"), dtype=td, device=DEV)
     x = x4[:3]
-    got = run_block1(x, w1s, shift1, w2, scale2, shift2, producer, code, td, out=out)
+    got = run_block1(x, w1s, shift1, w2, scale2, shift2, path, code, td, out=out)
     worst = 0.0
     for n in range(3):
         for r0 in (0, H // 4 - 6, H // 2 - 12):
@@ -256,11 +269,16 @@ def test_conv_block1_tile_index_limit(producer):
             g_ = got[n:n + 1, r0:r0 + 12].double()
             excess = ((g_ - want).abs() - 0.5 * ulp16(want, td)).clamp(min=0) / m.clamp(min=1e-30)
             worst = max(worst, excess.max().item())
-    report("conv_block1 3x65536 producer %d" % producer, rel=worst)
+    report("conv_block1 3x65536 %s" % path, rel=worst)
     assert worst <= BLOCK1_REL["fp16"]
     wp = w2.permute(0, 2, 3, 1).reshape(64, 576).contiguous()
-    rc = capi.load().sed_conv_block1(capi.ptr(x4), 4, H, W, capi.ptr(w1s), capi.ptr(shift1), capi.ptr(wp),
-                                     capi.ptr(scale2), capi.ptr(shift2), capi.ptr(out), producer, code, stream())
+    lib = capi.load()
+    if path == "fused":
+        rc = lib.sed_conv_block1(capi.ptr(x4), 4, H, W, capi.ptr(w1s), capi.ptr(shift1), capi.ptr(wp), capi.ptr(scale2),
+                                 capi.ptr(shift2), capi.ptr(out), code, stream())
+    else:  # conv1_2 is where the two-kernel path divides tile indices (its input is any 16-bit buffer: not read)
+        rc = lib.sed_conv3x3_bn_relu(capi.ptr(out), 4, H, W, 64, capi.ptr(wp), capi.ptr(scale2), capi.ptr(shift2), 64,
+                                     capi.CONV_POOL, capi.ptr(out), None, 0, 0, code, stream())
     assert capi.ERR_NAMES.get(rc) == "SED_ERR_BAD_SHAPE"
     assert engine.clamp_micro_batch(1 << 20, H) == 3
 
@@ -316,7 +334,7 @@ def test_freqmean_epilogue_writes_time_major_rows(b0, NB, H, dt):
         o32 = torch.full((H, Bp, 512), float("nan"), device=DEV) if with_f32 else None
         call("sed_conv3x3_bn_relu", capi.ptr(x), NB, H, 8, 512, capi.ptr(wp), capi.ptr(scale), capi.ptr(shift), 512,
              capi.CONV_FREQMEAN, capi.ptr(o16[0, b0:]), capi.ptr(None if o32 is None else o32[0, b0:]), 1, Bp, code,
-             2, stream())
+             stream())
         torch.cuda.synchronize()
         assert torch.isnan(o16[:, ~inside].float()).all(), "rows outside [b0, b0 + NB) were written"
         got16 = o16[:, inside]

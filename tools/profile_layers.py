@@ -53,13 +53,11 @@ def main():
     for (name, _, _, _), (cin, cout, mode, wp, s, b), (src, dst) in zip(engine.CONV_LAYERS, pm.convs, chain):
         x = ws[src]
         out = feat if dst is None else ws[dst]
-        for variant in (0, 2):
-            t = timeit(lambda: lib.sed_conv3x3_bn_relu(capi.ptr(x), mb, x.shape[1], x.shape[2], cin, capi.ptr(wp),
-                                                       capi.ptr(s), capi.ptr(b), cout, mode, capi.ptr(out), None, 0, 0,
-                                                       pm.dtype_code, variant, stream))
-            flops = 2.0 * mb * x.shape[1] * x.shape[2] * 9 * cin * cout
-            rows.append(("%s %d->%d %s" % (name, cin, cout, {0: "patch", 1: "tap", 2: "pair"}[variant]), t, flops,
-                         x.numel() * 2 + out.numel() * 2))
+        t = timeit(lambda: lib.sed_conv3x3_bn_relu(capi.ptr(x), mb, x.shape[1], x.shape[2], cin, capi.ptr(wp),
+                                                   capi.ptr(s), capi.ptr(b), cout, mode, capi.ptr(out), None, 0, 0,
+                                                   pm.dtype_code, stream))
+        flops = 2.0 * mb * x.shape[1] * x.shape[2] * 9 * cin * cout
+        rows.append(("%s %d->%d pair" % (name, cin, cout), t, flops, x.numel() * 2 + out.numel() * 2))
     B = args.batch
     featB = torch.randn(B, 125, 512, device=dev).to(pm.tdtype)
     if args.model.endswith("Gru_FrameAtt"):
@@ -81,12 +79,8 @@ def main():
     tot = 0.0
     print("per micro-batch of %d clips (temporal/head rows scaled from B=%d)" % (mb, B))
     for name, t, fl, by in rows:
-        if name.endswith("patch") and ("pair" in [r[0].split()[-1] for r in rows if r[0].split()[0] == name.split()[0]]):
-            tag = "   (alt)"
-        else:
-            tag = ""
-            tot += t
-        print("%-44s %8.3f ms  %8.1f TFLOP/s  %7.1f GB/s%s" % (name, t, fl / t / 1e9, by / t / 1e6, tag))
+        tot += t
+        print("%-44s %8.3f ms  %8.1f TFLOP/s  %7.1f GB/s" % (name, t, fl / t / 1e9, by / t / 1e6))
     print("sum %.3f ms per %d clips -> %.0f clips/s" % (tot, mb, mb / tot * 1e3))
     t = timeit(lambda: pm.forward(synth_wave_cache(B, dev), micro_batch=mb, variant=args.variant), n=5, warm=2)
     print("whole forward B=%d: %.3f ms -> %.0f clips/s" % (B, t, B / t * 1e3))
